@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the polar-code hot path on B200 (contract: see DESIGN.md "Measurement").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): SC decoder, k=512 n=1024 RM-rule code, AWGN/BPSK at Eb/N0 = 4 dB,
@@ -19,6 +19,8 @@ on the device by polar_awgn_frontend.  One step = one decode of the whole batch.
           the timed region, with the per-iteration split.
 --impl reference: the CPU restatement of the reference (oracle/libpolar_oracle.so, all host threads) on a
 bounded sample per step (the reference itself is pure Python and cannot travel to the GPU box).
+--dump-outputs DIR: after the timed steps, the decisions of the last step for a fixed, seeded sample of codewords
+(dump_outputs), so that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -51,6 +53,22 @@ def frozen_set(n, k):
             return d[key]
     from oracle import polar_oracle as po
     return po.rm_frozen_pos(n, n - k)
+
+
+DUMP_ROWS = 8192        # 8192 x n=1024 fp32 = 32 MiB
+
+
+def dump_rows(batch):
+    """Batch indices of the codewords --dump-outputs writes: a fixed, seeded sample, the same for every run and build."""
+    return np.sort(np.random.default_rng(0).choice(batch, size=min(batch, DUMP_ROWS), replace=False))
+
+
+def dump_outputs(out_dir, rows, u_hat_bits):
+    """DIR/u_hat.npy: the decisions u_hat[rows, 0:n] (frozen positions included) as fp32 0./1.;
+    DIR/u_hat_rows.npy: the batch index of each of those rows, as float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "u_hat.npy"), np.asarray(u_hat_bits, dtype=np.float32))
+    np.save(os.path.join(out_dir, "u_hat_rows.npy"), np.asarray(rows, dtype=np.float64))
 
 
 _FULL_AFFINITY = None
@@ -180,8 +198,11 @@ def run_reference(args):
         co.sc_decode_full(logits, fz)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        co.sc_decode_full(logits, fz)
+        u_hat = co.sc_decode_full(logits, fz)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        rows = dump_rows(sample)
+        dump_outputs(args.dump_outputs, rows, u_hat[rows])
     cws = sample * args.steps / dt
     val = cws * K_CODE / 1e9
     line = {"impl": "reference", "metric": "decoded_info_throughput_sc_n1024", "value": val, "unit": "Gbit/s",
@@ -291,7 +312,11 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-sweep", action="store_true")
     ap.add_argument("--skip-link", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the SC decisions of the last timed step (rank 0, seeded sample of %d codewords) to DIR" % DUMP_ROWS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -373,6 +398,10 @@ def main():
     ms_per_step = total_ms / args.steps
     cws = world * B / (ms_per_step * 1e-3)
     value = cws * k / 1e9
+    if args.dump_outputs and rank == 0:
+        rows = dump_rows(B)
+        words = u_hat[torch.from_numpy(rows).to(dev)].cpu().numpy()
+        dump_outputs(args.dump_outputs, rows, np.unpackbits(words.view(np.uint8), axis=-1, bitorder="little")[:, :n])
 
     # ---- same decode writing the reference's API tensor [B,k] fp32 as well (SURVEY 8d C2: "report both") -----
     u_api = torch.empty((B, k), dtype=torch.float32, device=dev)

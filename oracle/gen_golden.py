@@ -143,7 +143,8 @@ def gen_sc_boxplus(fz):
     """SURVEY 8f N2: the Sionna-style boxplus SC decoder (my_sn/fec/polar/dec.py:13-157).  Statistical fixture: the
     reference's decisions on AWGN words; the numpy restatement must agree on (almost) every codeword."""
     from my_sn.fec.polar.dec import SC_Dec as MySC
-    for (n, k, bs, ebno_db) in ((64, 32, 2000, 2.0), (256, 128, 1000, 2.5), (1024, 512, 400, 3.0)):
+    # keep: codewords stored (the first ones of the batch), so that every fixture stays under 1 MB
+    for (n, k, bs, ebno_db, keep) in ((64, 32, 2000, 2.0, 2000), (256, 128, 1000, 2.5, 1000), (1024, 512, 400, 3.0, 240)):
         fp = fz["rm_%d_%d" % (n, k)]
         G = tc.from_numpy(po.arikan_G(n))
         set_seed(900 + n)
@@ -157,8 +158,8 @@ def gen_sc_boxplus(fz):
               % (n, k, np.mean(np.any(u_ref != bits, axis=1)), np.mean(np.any(u_or != bits, axis=1)),
                  np.mean(np.any(u_ms != bits, axis=1)), agree))
         assert agree > 0.995
-        save("scbp_rm_%d_%d" % (n, k), logits=llr, frozen_pos=fp, u_hat=u_ref.astype(np.uint8), bits=bits.astype(np.uint8),
-             ebno_db=np.float32(ebno_db))
+        save("scbp_rm_%d_%d" % (n, k), logits=llr[:keep], frozen_pos=fp, u_hat=u_ref[:keep].astype(np.uint8),
+             bits=bits[:keep].astype(np.uint8), ebno_db=np.float32(ebno_db))
 
 
 def gen_scl_boxplus(fz):

@@ -2,8 +2,6 @@
 reference draws from torch's CPU mt19937, the kernel from Philox), error counters, CRC-aided list
 decoding, the link model + Monte-Carlo loop (BER/BLER inside confidence intervals of the oracle),
 and the host-buffer C-ABI entry points."""
-import os
-
 import numpy as np
 import pytest
 
@@ -395,8 +393,8 @@ def test_on_device_loop_with_process_group_of_one():
     ebnos = np.array([2.0, 4.0], dtype=np.float32)
     ref = sim_ber_device(System_AWGN_model(n, k, PolarEncoder(fp, n, None), SC_Dec(fp, n), seed=3), ebnos, bs, 3,
                          target_block_errs=100, verbose=False, return_counters=True)
-    os.environ.setdefault("MASTER_ADDR", "127.0.0.1"); os.environ.setdefault("MASTER_PORT", "29731")
-    dist.init_process_group("nccl", rank=0, world_size=1)
+    # an in-process store: a group of one needs no TCP rendezvous, so no port that another job on the host could hold
+    dist.init_process_group("nccl", store=dist.HashStore(), rank=0, world_size=1)
     try:
         got = sim_ber_device(System_AWGN_model(n, k, PolarEncoder(fp, n, None), SC_Dec(fp, n), seed=3), ebnos, bs, 3,
                              target_block_errs=100, verbose=False, return_counters=True)

@@ -168,11 +168,11 @@ def test_library_is_sm100a_only():
     assert "sm_100a" in out and "sm_90" not in out and "sm_80" not in out
 
 
-def test_register_subtree_decoder_on_host():
+def test_register_subtree_decoder_on_host(tmp_path):
     """polar_common.cuh's SubTree<T> (the per-thread 32-leaf SC decoder) compiled as plain C++ vs the C oracle."""
     from oracle import c_oracle as co
     co.build()
-    exe = "/tmp/polar_subtree_check"
+    exe = str(tmp_path / "polar_subtree_check")
     subprocess.check_call(["g++", "-O2", "-ffp-contract=off", "-I" + os.path.join(PKG, "csrc"),
                            os.path.join(ROOT, "tests", "host", "subtree_check.cpp"), "-o", exe,
                            "-L" + os.path.join(ROOT, "oracle"), "-lpolar_oracle",
