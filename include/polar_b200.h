@@ -125,7 +125,35 @@ int polar_scl_decode_boxplus_pruned(const float *d_logit, const uint32_t *d_froz
                                     const uint32_t *d_crc_rows, int crc_len,
                                     void *d_workspace, size_t workspace_bytes, void *stream);
 
-/* ---- encoder -----------------------------------------------------------------------------
+/* ---- hybrid SC -> SCL decoder (use_hybrid_sc=True of the Sionna-style SCL_Dec, my_sn/fec/polar/dec.py:437-470) --------
+ * For each row b:  s = SC(x[b]) (all n decisions, frozen = 0);  out[b] = s if the CRC over s holds, else the CRC-aided
+ * list decision of x[b] (L paths, selection as in polar_scl_decode).  An SC decision that passes the CRC by chance is kept,
+ * so the result is not the full list decoder's.  Four operations enqueued on `stream`, no synchronisation, no allocation:
+ *   1. the SC decoder of the chosen arithmetic over all B rows -> d_best_packed (the workspace when NULL) and d_u_info_f32
+ *   2. a memset of the failing-row count (d_n_list_out when given, else the workspace)
+ *   3. csrc/polar_hybrid.cu: syndrome of every SC row (XOR of d_crc_rows[i] over its set bits i), failing rows compacted
+ *   4. the generic list kernel (csrc/polar_scl.cu scl2, in every arithmetic) over the failing rows only, overwriting
+ *      their d_best_packed / d_u_info_f32 rows in place; its decisions equal polar_scl_decode*'s for the same row
+ *  cn_mode         0: min-sum (polar_sc_decode_f32 + the min-sum list kernel), 1: exact boxplus (polar_sc_decode_boxplus_f32
+ *                  + polar_scl_decode_boxplus's kernel), 2: boxplus with fast-SCL pruning (list stage as
+ *                  polar_scl_decode_boxplus_pruned)
+ *  d_logit etc.    as polar_sc_decode_f32 (16-byte aligned rows) and polar_scl_decode; n, L in the SCL range
+ *  d_crc_rows      required, crc_len in 1..32, k in 1..n (the number of information positions)
+ *  d_best_packed / d_u_info_f32   at least one of the two; there is no path-metric or list output
+ *  d_n_list_out    device int32, or NULL: number of list-decoded rows (stream ordered)
+ *  d_workspace     polar_scl_hybrid_workspace_bytes(n, L, B, cn_mode) bytes, 256-byte aligned (ENOMEM / EALIGN).  Layout:
+ *                  packed SC rows [B, POLAR_WORDS(n)] uint32 | count int32 | failing rows [B] int32 | list-kernel
+ *                  workspace for a persistent grid sized for B rows, each region 256-byte aligned.  The list workspace
+ *                  dominates: at n = 1024, L = 8 it is about 1.3 GB once B fills the grid (B >= 4 x the resident warps,
+ *                  18944 rows on a 148-SM B200); the other regions add 132 B per row.
+ *  B == 0 returns POLAR_OK and launches nothing. */
+size_t polar_scl_hybrid_workspace_bytes(int n, int L, int64_t B, int cn_mode);
+int polar_scl_decode_hybrid(const float *d_logit, const uint32_t *d_frozen_mask, int n, int L, int64_t B,
+                            uint32_t *d_best_packed, float *d_u_info_f32, const int32_t *d_info_pos, int k,
+                            const uint32_t *d_crc_rows, int crc_len, int cn_mode, int32_t *d_n_list_out,
+                            void *d_workspace, size_t workspace_bytes, void *stream);
+
+/* ---- encoder-----------------------------------------------------------------------------
  * polar_encode_packed: x = u.G over GF(2) on bit-packed rows (XOR butterfly; the transform of
  * my_sn/fec/polar/enc.py:85-96 == (c @ G) % 2 of x_run_sn_polar/polar/enc.py:42).
  * polar_encode_f32: the whole PolarEncoder.forward (x_run enc.py:30-43 / my_sn enc.py:97-113):

@@ -15,6 +15,7 @@
 // tree, counting rank); both return identical bits (tests/test_gpu_parity.py).
 #include <math.h>
 
+#include "polar_hybrid.h"
 #include "polar_internal.h"
 #include "polar_warp.cuh"
 
@@ -54,6 +55,9 @@ struct SclParams {
   size_t smem_per_warp;
   int words_global;                                     // scl2: partial-sum words live in ws (after the LLR stages)
   int fast;                                             // boxplus build only: node-level path-metric updates (use_fast_scl)
+  // row-indexed decode (polar_hybrid.cu): when rows != nullptr, codeword j = 0 .. min(*n_rows, B)-1 is logit row rows[j]
+  // and its outputs go to row rows[j]; no other output row is written.  B is then the host-side upper bound of *n_rows.
+  const int32_t *rows; const int32_t *n_rows;
 };
 
 // =====================================================================================================
@@ -97,12 +101,21 @@ __global__ void __launch_bounds__(128, SCL2_MINB) scl2_kernel(const SclParams P)
     return (s < s_glob) ? (llr_s + off) : (llr_g + (off - g_off));
   };
   const unsigned long long idrow = (unsigned long long)p * 0x0084210842108421ull;   // field s (5 bits) = p, s = 0..11
-  const int64_t nbatch = (P.B + CPW - 1) / CPW;
+  // number of codewords and the row of codeword j; re-read from memory where needed rather than kept live across the
+  // leaf loop, which runs at the 64-register cap
+  auto n_codewords = [&]() -> int64_t {
+    if (!P.rows) return P.B;
+    const int64_t c = *P.n_rows;                                 // written by the previous kernel on the stream
+    return c < 0 ? 0 : (c < P.B ? c : P.B);
+  };
+  auto row_of = [&](int64_t j) -> int64_t { return P.rows ? (int64_t)P.rows[j] : j; };
 
-  for (int64_t bb = gwarp; bb < nbatch; bb += (int64_t)gridDim.x * nwarps) {
-    const int64_t b = bb * CPW + cwl;
-    const bool valid = b < P.B;
-    const float *ch = P.logit + (valid ? b : (P.B - 1)) * (int64_t)n;
+  for (int64_t bb = gwarp; bb < (n_codewords() + CPW - 1) / CPW; bb += (int64_t)gridDim.x * nwarps) {
+    const float *ch;
+    {
+      const int64_t nb = n_codewords(), j = bb * CPW + cwl;
+      ch = P.logit + row_of(j < nb ? j : nb - 1) * (int64_t)n;   // idle lanes of the last group redo a real codeword
+    }
     double pm = (p == 0) ? 0.0 : kLlrMaxD;                       // polar_scl.py:192-194
     unsigned long long rowL = idrow, rowB = idrow;
     uint32_t small = 0u, rootreg = 0u, fword = 0u;
@@ -308,6 +321,9 @@ __global__ void __launch_bounds__(128, SCL2_MINB) scl2_kernel(const SclParams P)
       }
     }
     // lane p of each group now holds rank p: (pm ascending, source path)
+    const int64_t j = bb * CPW + cwl;
+    const bool valid = j < n_codewords();
+    const int64_t b = valid ? row_of(j) : 0;
     if (P.pm_out && valid) P.pm_out[b * L + p] = key;
     const int slot = gbase + src;                                  // slot holding the decisions of rank p
     if (P.list && valid)
@@ -404,6 +420,36 @@ static int launch_scl(SclParams &P, const SclPlan &pl, cudaStream_t st) {
   return POLAR_OK;
 }
 
+static int launch_scl_any(SclParams &P, const SclPlan &pl, int L, cudaStream_t st) {
+  switch (L) {
+    case 1: return launch_scl<1>(P, pl, st);
+    case 2: return launch_scl<2>(P, pl, st);
+    case 4: return launch_scl<4>(P, pl, st);
+    case 8: return launch_scl<8>(P, pl, st);
+    case 16: return launch_scl<16>(P, pl, st);
+    default: return launch_scl<32>(P, pl, st);
+  }
+}
+
+size_t scl2_rows_workspace_bytes(int n, int L, int64_t B) {
+  const SclPlan pl = scl_plan(n, L, B);
+  return (size_t)pl.grid * pl.warps_per_cta * pl.ws_doubles_per_warp * sizeof(double);
+}
+
+int launch_scl2_rows(const float *logit, const uint32_t *fmask, int n, int L, int64_t B, const int32_t *rows,
+                     const int32_t *n_rows, uint32_t *best, float *u_info, const int32_t *info_pos, int k,
+                     const uint32_t *crc_rows, int crc_len, void *ws, int fast, cudaStream_t st) {
+  const SclPlan pl = scl_plan(n, L, B);
+  SclParams P;
+  P.logit = logit; P.fmask = fmask; P.n = n; P.m = ilog2(n); P.B = B;
+  P.best = best; P.u_info = u_info; P.info_pos = info_pos; P.k = k;
+  P.pm_out = nullptr; P.list = nullptr; P.crc_rows = crc_rows; P.crc_len = crc_len;
+  P.ws = (double *)ws; P.ws_doubles_per_warp = pl.ws_doubles_per_warp; P.s_glob = pl.s_glob;
+  P.smem_per_warp = pl.smem_per_warp; P.words_global = pl.words_global; P.fast = fast;
+  P.rows = rows; P.n_rows = n_rows;
+  return launch_scl_any(P, pl, L, st);
+}
+
 }  // namespace polar
 
 using namespace polar;
@@ -473,15 +519,8 @@ static int scl_decode_impl(const float *d_logit, const uint32_t *d_frozen_mask, 
   P.pm_out = d_pm_sorted; P.list = d_list_packed; P.crc_rows = d_crc_rows; P.crc_len = crc_len;
   P.ws = (double *)d_workspace; P.ws_doubles_per_warp = pl.ws_doubles_per_warp; P.s_glob = pl.s_glob;
   P.smem_per_warp = pl.smem_per_warp; P.words_global = pl.words_global; P.fast = fast;
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (L) {
-    case 1: return launch_scl<1>(P, pl, st);
-    case 2: return launch_scl<2>(P, pl, st);
-    case 4: return launch_scl<4>(P, pl, st);
-    case 8: return launch_scl<8>(P, pl, st);
-    case 16: return launch_scl<16>(P, pl, st);
-    default: return launch_scl<32>(P, pl, st);
-  }
+  P.rows = nullptr; P.n_rows = nullptr;
+  return launch_scl_any(P, pl, L, (cudaStream_t)stream);
 }
 
 extern "C" int polar_scl_decode(const float *d_logit, const uint32_t *d_frozen_mask, int n, int L, int64_t B,

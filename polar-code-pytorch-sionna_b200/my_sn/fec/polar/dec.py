@@ -2,7 +2,9 @@
 on the min-sum list kernel it is the composed oracle of SURVEY 8(c) for BASELINE config 3 -- and the Sionna-style boxplus
 SC / SCL decoders (dec.py:13-157 / :158-537, SURVEY 8f row N2).  `use_fast_scl=True` (the default) runs the list kernel
 with the reference's rate-0 / REP node shortcuts (dec.py:269-306, 354-376: node-level path-metric updates, the subtree
-is not descended into); `use_hybrid_sc` is accepted and ignored like dec.py:237-238."""
+is not descended into).  `use_hybrid_sc=True` (dec.py:437-470) decodes every codeword with SC first and list-decodes only
+those whose SC decision fails the CRC (`polar_scl_decode_hybrid`: SC, a CRC check / compaction kernel and the list kernel
+over the failing rows, all on the device)."""
 import numpy as np
 import torch as tc
 from torch import nn
@@ -55,7 +57,11 @@ class SCL_Dec(nn.Module):
   (`polar_scl_decode_boxplus_pruned`), `use_fast_scl=False` updates leaf by leaf (`polar_scl_decode_boxplus`).  Parity
   with the CPU reference is statistical for both (its exp / log are the host's; SURVEY 8c).
   cn_type="minsum": the x_run min-sum list kernel under the same CRC-aided selection -- the composed oracle of
-  BASELINE config 3, bit-exact against `tests/golden/sclcrc_*`."""
+  BASELINE config 3, bit-exact against `tests/golden/sclcrc_*`.
+  use_hybrid_sc=True (needs crc_degree): SC of the same arithmetic on every codeword; a codeword whose SC decision passes
+  the CRC keeps it, the others are list-decoded as above.  Not the same result as full SCL: an SC decision can pass the CRC
+  by chance.  `msg_pm` is then None, and `list_decoded` (device int32 [1]) holds how many codewords the last call
+  list-decoded; reading it synchronises with that call."""
 
   def __init__(self, frozen_pos, n, list_size=8, crc_degree=None, use_hybrid_sc=False, use_fast_scl=True,
                return_crc_status=False, output_dtype=tc.float32, device='cpu', cn_type="boxplus"):
@@ -90,9 +96,15 @@ class SCL_Dec(nn.Module):
     assert self._k >= self._k_crc, "Value of k is too small for given CRC_degree."
     if (crc_degree is None) and return_crc_status:
       raise ValueError("Returning CRC status requires given crc_degree.")
+    if (crc_degree is None) and use_hybrid_sc:
+      raise ValueError("Hybrid SC decoding requires given crc_degree.")
+    self._use_hybrid_sc = bool(use_hybrid_sc)
+    self._hybrid_mode = (dk.HYBRID_MINSUM if not self._boxplus else
+                         dk.HYBRID_BOXPLUS_PRUNED if self._pruned else dk.HYBRID_BOXPLUS)
     self._return_crc_status = return_crc_status
     self._crc_rows = {}
     self.msg_pm = None
+    self.list_decoded = None
 
   @property
   def n(self): return self._n
@@ -119,9 +131,20 @@ class SCL_Dec(nn.Module):
 
   def decode_packed(self, logits, tables, out=None):
     """Device fast path of the on-device Monte-Carlo loop: bit-packed decisions of the (CRC-)selected path."""
+    if self._use_hybrid_sc:
+      return self._decode_hybrid(logits, tables, want_info=False, out_packed=out)["u_packed"]
     rows, ln = self._rows_on(tables.dev)
     return dk.scl_decode(logits, tables, self._list_size, crc_rows=rows, crc_len=ln, want_info=False,
                          want_packed=True, boxplus=self._boxplus, out_packed=out, pruned=self._pruned)["u_packed"]
+
+  def _decode_hybrid(self, logits, tables, want_info, out_packed=None):
+    rows, ln = self._rows_on(tables.dev)
+    if self.list_decoded is None or self.list_decoded.device != tables.dev:
+      self.list_decoded = tc.zeros(1, dtype=tc.int32, device=tables.dev)
+    if logits.numel() == 0:
+      self.list_decoded.zero_()
+    return dk.scl_decode_hybrid(logits, tables, self._list_size, rows, ln, self._hybrid_mode, want_info=want_info,
+                                want_packed=not want_info, out_packed=out_packed, n_list_out=self.list_decoded)
 
   def forward(self, inputs):
     assert inputs.dtype == self.output_dtype, "Invalid input dtype."
@@ -135,7 +158,9 @@ class SCL_Dec(nn.Module):
       if rows is None:
         rows = self._crc_rows[str(dev)] = tc.from_numpy(self._crc_rows_np.view(np.int32).copy()).to(dev)
       ln = self._k_crc
-    if not inputs.is_cuda and not self._boxplus:     # CPU tensor: chunked, overlapped H2D / decode / D2H inside one call
+    if self._use_hybrid_sc:                          # device path for CPU tensors too (plain copy in and out)
+      u_info, self.msg_pm = self._decode_hybrid(inputs, tables, want_info=True)["u_info"], None
+    elif not inputs.is_cuda and not self._boxplus:   # CPU tensor: chunked, overlapped H2D / decode / D2H inside one call
       u_info, self.msg_pm = dk.scl_decode_host(inputs, tables, self._list_size,
                                                crc_rows_np=self._crc_rows_np if self._use_crc else None, crc_len=ln)
     else:
@@ -155,9 +180,9 @@ class Polar5GDecoder(nn.Module):
   """Rate recovery + polar decoding + CRC removal for codewords of `Polar5GEncoder` (my_sn/fec/polar/dec.py:539-667,
   SURVEY 8f row N3).  Channel de-interleaver, de-puncturing (logit 0), de-shortening (logit -100), repetition combining
   and the sub-block de-interleaver are folded into one index plan applied by `polar_rate_recover_f32`; the decoder is the
-  my_sn `SC_Dec` (boxplus SC) or the CRC-aided `SCL_Dec`.  `dec_type="hybSCL"` runs the CRC-aided list decoder (the
-  reference's hybrid branch cannot be constructed); `return_crc_status=True` works here (the reference stops in a
-  stray breakpoint, dec.py:661)."""
+  my_sn `SC_Dec` (boxplus SC) or the CRC-aided `SCL_Dec`.  `dec_type="hybSCL"` runs that `SCL_Dec` with
+  `use_hybrid_sc=True`: SC first, list decoding only of the codewords whose SC decision fails the CRC.
+  `return_crc_status=True` works here (the reference stops in a stray breakpoint, dec.py:661)."""
 
   def __init__(self, enc_polar, dec_type="SC", list_size=8, return_crc_status=False, output_dtype=tc.float32):
     super().__init__()
@@ -175,7 +200,7 @@ class Polar5GDecoder(nn.Module):
       self._polar_dec = SC_Dec(enc_polar._frozen_pos, self._n_polar, device=enc_polar.device)
     elif dec_type in ("SCL", "hybSCL"):
       self._polar_dec = SCL_Dec(enc_polar._frozen_pos, self._n_polar, crc_degree=enc_polar.enc_crc.crc_degree,
-                                list_size=list_size, device=enc_polar.device)
+                                list_size=list_size, use_hybrid_sc=dec_type == "hybSCL", device=enc_polar.device)
     else:
       raise ValueError("Unknown value for dec_type.")
     assert isinstance(return_crc_status, bool), "return_crc_status must be bool."

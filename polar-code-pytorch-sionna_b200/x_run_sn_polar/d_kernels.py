@@ -57,6 +57,8 @@ _SIGNATURES = {
   "polar_scl_boxplus_workspace_bytes": (_sz, [_i32, _i32, _i64]),
   "polar_scl_decode_boxplus": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _sz, _vp]),
   "polar_scl_decode_boxplus_pruned": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _sz, _vp]),
+  "polar_scl_hybrid_workspace_bytes": (_sz, [_i32, _i32, _i64, _i32]),
+  "polar_scl_decode_hybrid": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _i32, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
   "polar_encode_packed": (_i32, [_vp, _i32, _i64, _vp, _vp]),
   "polar_encode_f32": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp]),
   "polar_gather_cols_f32": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp]),
@@ -260,14 +262,44 @@ def scl_decode(logits, tables, list_size, crc_rows=None, crc_len=0, want_info=Tr
     fn_dec = lib().polar_scl_decode if not boxplus else (
       lib().polar_scl_decode_boxplus_pruned if pruned else lib().polar_scl_decode_boxplus)   # pruned: use_fast_scl node shortcuts
     need = int(fn_ws(n, L, B)) if B > 0 else 0
-    ws = None
-    if need:
-      ws = _WS_CACHE.get(str(dev))
-      if ws is None or ws.numel() < need:
-        ws = _WS_CACHE[str(dev)] = tc.empty(need + 256, dtype=tc.uint8, device=dev)
+    ws = _workspace(dev, need)
     check(fn_dec(ptr(x), ptr(tables.frozen_mask), n, L, B, ptr(out["u_packed"]), ptr(out["u_info"]),
                                  ptr(tables.info_pos), tables.k, ptr(out["pm"]), ptr(out["list"]),
                                  ptr(crc_rows), int(crc_len), ptr(ws), need, stream_ptr(dev)))
+  return out
+
+
+def _workspace(dev, need):
+  """The per-device list-decoder workspace (grown, never shrunk), or None when `need` is 0."""
+  if not need:
+    return None
+  ws = _WS_CACHE.get(str(dev))
+  if ws is None or ws.numel() < need:
+    ws = _WS_CACHE[str(dev)] = tc.empty(need + 256, dtype=tc.uint8, device=dev)
+  return ws
+
+
+HYBRID_MINSUM, HYBRID_BOXPLUS, HYBRID_BOXPLUS_PRUNED = 0, 1, 2
+
+
+def scl_decode_hybrid(logits, tables, list_size, crc_rows, crc_len, cn_mode, want_info=True, want_packed=False,
+                      out_packed=None, n_list_out=None):
+  """polar_scl_decode_hybrid: SC on every row, CRC-aided list decoding (L paths) only of the rows whose SC decision fails
+  the CRC.  cn_mode: HYBRID_MINSUM, HYBRID_BOXPLUS or HYBRID_BOXPLUS_PRUNED (both stages in that arithmetic).
+  n_list_out: optional device int32 [1] tensor that receives the number of list-decoded rows (stream ordered).
+  -> dict(u_info fp32 [B,k] | None, u_packed int32 [B,words] | None)."""
+  dev = tables.dev
+  x = _prep_logits(logits, tables.n, dev)
+  B, n, L = x.shape[0], tables.n, int(list_size)
+  out = {"u_info": tc.empty((B, tables.k), dtype=tc.float32, device=dev) if want_info else None,
+         "u_packed": out_packed if out_packed is not None else (
+           tc.empty((B, words(n)), dtype=tc.int32, device=dev) if want_packed else None)}
+  with tc.cuda.device(dev):
+    need = int(lib().polar_scl_hybrid_workspace_bytes(n, L, B, int(cn_mode))) if B > 0 else 0
+    ws = _workspace(dev, need)
+    check(lib().polar_scl_decode_hybrid(ptr(x), ptr(tables.frozen_mask), n, L, B, ptr(out["u_packed"]), ptr(out["u_info"]),
+                                        ptr(tables.info_pos), tables.k, ptr(crc_rows), int(crc_len), int(cn_mode),
+                                        ptr(n_list_out), ptr(ws), need, stream_ptr(dev)))
   return out
 
 
