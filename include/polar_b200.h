@@ -131,7 +131,7 @@ int polar_scl_decode_boxplus_pruned(const float *d_logit, const uint32_t *d_froz
  * so the result is not the full list decoder's.  Four operations enqueued on `stream`, no synchronisation, no allocation:
  *   1. the SC decoder of the chosen arithmetic over all B rows -> d_best_packed (the workspace when NULL) and d_u_info_f32
  *   2. a memset of the failing-row count (d_n_list_out when given, else the workspace)
- *   3. csrc/polar_hybrid.cu: syndrome of every SC row (XOR of d_crc_rows[i] over its set bits i), failing rows compacted
+ *   3. csrc/polar_scl_api.cu: syndrome of every SC row (XOR of d_crc_rows[i] over its set bits i), failing rows compacted
  *   4. the generic list kernel (csrc/polar_scl.cu scl2, in every arithmetic) over the failing rows only, overwriting
  *      their d_best_packed / d_u_info_f32 rows in place; its decisions equal polar_scl_decode*'s for the same row
  *  cn_mode         0: min-sum (polar_sc_decode_f32 + the min-sum list kernel), 1: exact boxplus (polar_sc_decode_boxplus_f32

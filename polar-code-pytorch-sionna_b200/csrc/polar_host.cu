@@ -13,6 +13,7 @@
 #include <vector>
 
 #include "polar_internal.h"
+#include "polar_scl.h"
 
 namespace polar {
 
@@ -234,29 +235,26 @@ extern "C" int polar_sc_decode_host(const float *h_logit, const uint32_t *h_froz
 extern "C" int polar_scl_decode_host_f32(const float *h_logit, const uint32_t *h_frozen_mask, int n, int L, int64_t B,
                                          uint32_t *h_best_packed, float *h_u_info_f32, const int32_t *h_info_pos, int k,
                                          double *h_pm_sorted, const uint32_t *h_crc_rows, int crc_len, int device) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_SCL_MAX_N || !is_pow2(L) || L > POLAR_SCL_MAX_L || B < 0) return set_error(POLAR_EINVAL, "scl host: bad n/L/B");
-  if (B == 0) return POLAR_OK;
+  int rc = check_scl_shape("scl host", n, L, B);
+  if (rc != POLAR_OK || B == 0) return rc;
   if (!h_logit || !h_frozen_mask || (!h_best_packed && !h_u_info_f32)) return set_error(POLAR_EINVAL, "scl host: null pointer");
   if (h_u_info_f32 && (!h_info_pos || k < 1 || k > n)) return set_error(POLAR_EINVAL, "scl host: u_info requested without valid info_pos/k");
   if (device < 0 || device >= 64) return set_error(POLAR_EINVAL, "scl host: bad device");
-  if (B == 0) return POLAR_OK;
   HostCtx &C = g_ctx[device];
   std::lock_guard<std::mutex> lk(C.mu);
   DeviceGuard guard(device);
   if (!guard.ok) return set_error(POLAR_ECUDA, "scl host: cannot select device %d", device);
-  int rc = polar_init(device);
+  rc = polar_init(device);
   if (rc) return rc;
   int64_t chunk = chunk_codewords(n, B, true);        // the list decoder's time per chunk is not hidden by the copy: large chunks
-  if (scl3_supported(n, L) && chunk < B) {
+  const SclPlan whole = scl_plan(n, L, B, SclArith::minsum, true);   // the chunk buffers are cudaMalloc'd: aligned rows
+  if (whole.scl3 && chunk < B) {
     // the list kernel is persistent: every resident warp decodes the same number of 32/L-codeword groups, so a chunk
     // should be a whole number of such rounds (a 128 MB chunk of n = 1024 is 3.46 rounds: 13 % of the last one idle)
-    Scl3Plan p3;
-    if (launch_scl3(nullptr, nullptr, n, L, B, nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, 0, nullptr, nullptr, &p3) == POLAR_OK) {
-      const int64_t round = p3.grid * (32 / L);
-      if (round > 0 && chunk > round) chunk = chunk / round * round;
-    }
+    const int64_t round = whole.grid * (32 / L);
+    if (chunk > round) chunk = chunk / round * round;
   }
-  const size_t ws_need = polar_scl_workspace_bytes(n, L, chunk);
+  const size_t ws_need = scl_plan(n, L, chunk, SclArith::minsum, true).ws_bytes;
   if ((rc = prepare(C, h_frozen_mask, n, h_u_info_f32 ? h_info_pos : nullptr, k))) return rc;
   const bool crc = crc_len > 0 && h_crc_rows;
   if (crc) {

@@ -6,7 +6,7 @@
 // sort the 2L candidates ascending, keep L.  Arithmetic is fp64 like the reference (numpy float64):
 // min-sum f with +-30 clip, g = (1-2u)a+b, exact softplus path metric.
 //
-// This file: the entry point polar_scl_decode and the GENERIC list kernel scl2_kernel<L> (lane = (codeword, path): a warp
+// This file: the GENERIC list kernel scl2_kernel<L> and its launcher (lane = (codeword, path): a warp
 // decodes 32/L codewords, every lane walks all elements of its own path's nodes; nothing is copied on a fork -- a stage is
 // always rewritten by every path at the same time, so a path writes its own slot and a fork only permutes packed pointer
 // rows with a warp shuffle; decisions are recovered at the end from the root partial sums; the 2L candidates are ranked by
@@ -15,8 +15,8 @@
 // tree, counting rank); both return identical bits (tests/test_gpu_parity.py).
 #include <math.h>
 
-#include "polar_hybrid.h"
 #include "polar_internal.h"
+#include "polar_scl.h"
 #include "polar_warp.cuh"
 
 namespace polar {
@@ -25,7 +25,7 @@ constexpr double kLlrMaxD = 30.0;
 
 #if defined(POLAR_F_BOXPLUS)
 // exact boxplus of the Sionna-style list decoder (my_sn/fec/polar/dec.py:331-340, numpy float64): clip to +-30,
-// ln(1+e^(x+y)) - ln(e^x+e^y).  Selected by polar_bp_wrap.cu (namespace polar_bp, entry point polar_scl_decode_boxplus).
+// ln(1+e^(x+y)) - ln(e^x+e^y).  Selected by polar_bp_wrap.cu (namespace polar_bp, launcher launch_scl2_boxplus).
 __device__ __forceinline__ double f_minsum_d(double a, double b) {
   const double x = fmax(fmin(a, 30.0), -30.0), y = fmax(fmin(b, 30.0), -30.0);
   return log(1.0 + exp(x + y)) - log(exp(x) + exp(y));
@@ -47,19 +47,6 @@ __device__ __forceinline__ double pm_penalty(double x_clipped, unsigned u) {
   return log(1.0 + exp(v));
 }
 
-struct SclParams {
-  const float *logit; const uint32_t *fmask; int n, m; int64_t B;
-  uint32_t *best; float *u_info; const int32_t *info_pos; int k;
-  double *pm_out; uint32_t *list; const uint32_t *crc_rows; int crc_len;
-  double *ws; size_t ws_doubles_per_warp; int s_glob;   // LLR stages >= s_glob live in ws
-  size_t smem_per_warp;
-  int words_global;                                     // scl2: partial-sum words live in ws (after the LLR stages)
-  int fast;                                             // boxplus build only: node-level path-metric updates (use_fast_scl)
-  // row-indexed decode (polar_hybrid.cu): when rows != nullptr, codeword j = 0 .. min(*n_rows, B)-1 is logit row rows[j]
-  // and its outputs go to row rows[j]; no other output row is written.  B is then the host-side upper bound of *n_rows.
-  const int32_t *rows; const int32_t *n_rows;
-};
-
 // =====================================================================================================
 // scl2_kernel: lane = (codeword, path).  A warp decodes 32/L codewords at once, every lane owns one path of
 // one codeword and walks ALL elements of its nodes itself.  Same lazy-copy bookkeeping as scl_kernel above
@@ -69,8 +56,6 @@ struct SclParams {
 // issue utilisation -> the kernel was instruction bound).  Per-stage arrays are [element][32 lanes] doubles:
 // a warp access touches 32 consecutive doubles, conflict free.
 // =====================================================================================================
-__host__ __device__ inline size_t scl2_llr_smem_doubles(int s_glob) { return (size_t)32 * ((1u << s_glob) - 1u); }
-
 #ifndef SCL2_MINB
 #define SCL2_MINB 8   // 64 registers per thread: occupancy (latency hiding of the workspace traffic) beats registers
 #endif
@@ -368,175 +353,17 @@ __global__ void __launch_bounds__(128, SCL2_MINB) scl2_kernel(const SclParams P)
   }
 }
 
-struct SclPlan { int s_glob; size_t smem_per_warp; size_t ws_doubles_per_warp; int warps_per_cta; int64_t grid; int words_global = 0; };
-
-static int scl_mode() { return env_int("POLAR_SCL_MODE", 2); }   // 2: scl3 where supported, else scl2 [default]; 1: scl2 always (tests)
-
-static SclPlan scl_plan(int n, int L, int64_t B) {
-  SclPlan pl;
-  const int m = ilog2(n);
-  const int max_smem = device_max_smem_optin();
-  {
-    const int nw = n < 32 ? 1 : n >> 5;
-    const size_t words = (size_t)32 * 2 * nw * 4;
-    const int budget = env_int("POLAR_SCL_SMEM_KB", 4) * 1024;    // per warp
-    pl.words_global = env_int("POLAR_SCL_WORDS_GLOBAL", 1) != 0 && words > 1024;
-    const size_t wsm = pl.words_global ? 0 : words;
-    int s_glob = m;
-    while (s_glob > 0 && scl2_llr_smem_doubles(s_glob) * 8 + wsm > (size_t)budget) --s_glob;
-    pl.s_glob = s_glob;
-    pl.smem_per_warp = ((scl2_llr_smem_doubles(s_glob) * 8 + wsm + 15) / 16) * 16;
-    if (pl.smem_per_warp < 16) pl.smem_per_warp = 16;
-    pl.ws_doubles_per_warp = (size_t)32 * ((1u << m) - (1u << s_glob)) + (pl.words_global ? words / 8 : 0);
-    int wpc = env_int("POLAR_SCL_WARPS", 1);
-    if (wpc < 1) wpc = 1;
-    if (wpc > 4) wpc = 4;
-    while (wpc > 1 && pl.smem_per_warp * wpc > (size_t)max_smem) --wpc;
-    pl.warps_per_cta = wpc;
-    int ctas_per_sm = (int)((size_t)(228 * 1024) / (pl.smem_per_warp * wpc + 1024));
-    if (ctas_per_sm < 1) ctas_per_sm = 1;
-    if (ctas_per_sm > 32) ctas_per_sm = 32;
-    if (ctas_per_sm * wpc > 32) ctas_per_sm = 32 / wpc;          // 64 registers x 32 lanes x 32 warps = the register file
-    const int cpw = 32 / L;
-    const int64_t nbatch = (B + cpw - 1) / cpw;
-    int64_t grid = (nbatch + wpc - 1) / wpc;
-    const int64_t cap = (int64_t)device_sm_count() * ctas_per_sm;
-    if (grid > cap) grid = cap;
-    if (grid < 1) grid = 1;
-    pl.grid = grid;
-    return pl;
-  }
-}
-
-template <int L>
-static int launch_scl(SclParams &P, const SclPlan &pl, cudaStream_t st) {
-  void (*kern)(const SclParams) = scl2_kernel<L>;
-  const size_t smem = pl.smem_per_warp * pl.warps_per_cta;
-  if (smem > (size_t)device_max_smem_optin()) return set_error(POLAR_ENOMEM, "scl: needs %zu B shared memory per CTA", smem);
-  POLAR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<(unsigned)pl.grid, pl.warps_per_cta * 32, smem, st>>>(P);
-  count_launch();
-  POLAR_CHECK_LAUNCH("scl2_kernel");
-  return POLAR_OK;
-}
-
-static int launch_scl_any(SclParams &P, const SclPlan &pl, int L, cudaStream_t st) {
-  switch (L) {
-    case 1: return launch_scl<1>(P, pl, st);
-    case 2: return launch_scl<2>(P, pl, st);
-    case 4: return launch_scl<4>(P, pl, st);
-    case 8: return launch_scl<8>(P, pl, st);
-    case 16: return launch_scl<16>(P, pl, st);
-    default: return launch_scl<32>(P, pl, st);
-  }
-}
-
-size_t scl2_rows_workspace_bytes(int n, int L, int64_t B) {
-  const SclPlan pl = scl_plan(n, L, B);
-  return (size_t)pl.grid * pl.warps_per_cta * pl.ws_doubles_per_warp * sizeof(double);
-}
-
-int launch_scl2_rows(const float *logit, const uint32_t *fmask, int n, int L, int64_t B, const int32_t *rows,
-                     const int32_t *n_rows, uint32_t *best, float *u_info, const int32_t *info_pos, int k,
-                     const uint32_t *crc_rows, int crc_len, void *ws, int fast, cudaStream_t st) {
-  const SclPlan pl = scl_plan(n, L, B);
-  SclParams P;
-  P.logit = logit; P.fmask = fmask; P.n = n; P.m = ilog2(n); P.B = B;
-  P.best = best; P.u_info = u_info; P.info_pos = info_pos; P.k = k;
-  P.pm_out = nullptr; P.list = nullptr; P.crc_rows = crc_rows; P.crc_len = crc_len;
-  P.ws = (double *)ws; P.ws_doubles_per_warp = pl.ws_doubles_per_warp; P.s_glob = pl.s_glob;
-  P.smem_per_warp = pl.smem_per_warp; P.words_global = pl.words_global; P.fast = fast;
-  P.rows = rows; P.n_rows = n_rows;
-  return launch_scl_any(P, pl, L, st);
-}
-
 }  // namespace polar
 
 using namespace polar;
 
-extern "C" size_t polar_scl_workspace_bytes(int n, int L, int64_t B) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_SCL_MAX_N || !is_pow2(L) || L > POLAR_SCL_MAX_L || B <= 0) return 0;
-  const SclPlan pl = scl_plan(n, L, B);
-  size_t need = (size_t)pl.grid * pl.warps_per_cta * pl.ws_doubles_per_warp * sizeof(double);
-#if !defined(POLAR_F_BOXPLUS)      // the boxplus build has no scl3 (its compile time with exp/log inlined ~70 times per
-                                   // instantiation is 19 minutes); boxplus list decoding is scl2 with node pruning
-  if (scl_mode() == 2 && scl3_supported(n, L)) {
-    // scl3 is what runs; rows that are not 16-byte aligned fall back to scl2, which shrinks its grid to the workspace it
-    // is given (at least one CTA per SM), so its much larger default appetite (1.3 GB at n=1024, L=8) is not reserved
-    Scl3Plan p3;
-    if (launch_scl3(nullptr, nullptr, n, L, B, nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, 0, nullptr, nullptr, &p3) == POLAR_OK) {
-      const size_t n3 = (size_t)p3.grid * p3.ws_bytes_per_warp;
-      size_t floor2 = (size_t)device_sm_count() * pl.warps_per_cta * pl.ws_doubles_per_warp * sizeof(double);
-      if (floor2 > need) floor2 = need;
-      need = n3 > floor2 ? n3 : floor2;
-    }
-  }
-#endif
-  return need;
+// launch_scl2 (launch_scl2_boxplus in the boxplus build), declared in polar_scl.h.  At most 4 KB of dynamic shared
+// memory per warp (scl_plan), under the default limit.
+int launch_scl2(const SclParams &P, const SclPlan &pl, int L, cudaStream_t st) {
+  void (*kern)(const SclParams) = L == 1 ? scl2_kernel<1> : L == 2 ? scl2_kernel<2> : L == 4 ? scl2_kernel<4>
+                                  : L == 8 ? scl2_kernel<8> : L == 16 ? scl2_kernel<16> : scl2_kernel<32>;
+  kern<<<(unsigned)pl.grid, 32, P.smem_per_warp, st>>>(P);
+  count_launch();
+  POLAR_CHECK_LAUNCH("scl2_kernel");
+  return POLAR_OK;
 }
-
-static int scl_decode_impl(const float *d_logit, const uint32_t *d_frozen_mask, int n, int L, int64_t B,
-                           uint32_t *d_best_packed, float *d_u_info_f32, const int32_t *d_info_pos, int k,
-                           double *d_pm_sorted, uint32_t *d_list_packed, const uint32_t *d_crc_rows, int crc_len,
-                           void *d_workspace, size_t workspace_bytes, void *stream, int fast) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_SCL_MAX_N) return set_error(POLAR_EINVAL, "scl: n=%d must be a power of two in [2,%d]", n, POLAR_SCL_MAX_N);
-  if (!is_pow2(L) || L > POLAR_SCL_MAX_L) return set_error(POLAR_EINVAL, "scl: list_size=%d must be a power of two <= %d", L, POLAR_SCL_MAX_L);
-  if (B < 0) return set_error(POLAR_EINVAL, "scl: B < 0");
-  if (B == 0) return POLAR_OK;
-  if (!d_logit || !d_frozen_mask) return set_error(POLAR_EINVAL, "scl: null logit / frozen_mask");
-  if (!d_best_packed && !d_u_info_f32 && !d_pm_sorted && !d_list_packed) return set_error(POLAR_EINVAL, "scl: no output buffer");
-  if (d_u_info_f32 && (!d_info_pos || k < 0 || k > n)) return set_error(POLAR_EINVAL, "scl: u_info requested without valid info_pos/k");
-  if (crc_len < 0 || crc_len > 32 || (crc_len > 0 && !d_crc_rows)) return set_error(POLAR_EINVAL, "scl: bad crc_len / crc_rows");
-  if (crc_len > 0 && (k < 1 || k > n)) return set_error(POLAR_EINVAL, "scl: CRC-aided selection needs k (penalty 30 k, dec.py:517-518), got k=%d", k);
-#if !defined(POLAR_F_BOXPLUS)
-  if (!fast && scl_mode() == 2 && scl3_supported(n, L) && ((uintptr_t)d_logit & 15) == 0) {
-    Scl3Plan p3;
-    int rc = launch_scl3(d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, d_pm_sorted, d_list_packed,
-                         d_crc_rows, crc_len, d_workspace, (cudaStream_t)stream, &p3);
-    if (rc != POLAR_OK) return rc;
-    const size_t need3 = (size_t)p3.grid * p3.ws_bytes_per_warp;
-    if (!d_workspace || workspace_bytes < need3) return set_error(POLAR_ENOMEM, "scl: workspace %zu B < required %zu B", workspace_bytes, need3);
-    if ((uintptr_t)d_workspace & 255) return set_error(POLAR_EALIGN, "scl: workspace must be 256-byte aligned");
-    return launch_scl3(d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, d_pm_sorted, d_list_packed,
-                       d_crc_rows, crc_len, d_workspace, (cudaStream_t)stream, nullptr);
-  }
-#endif
-  SclPlan pl = scl_plan(n, L, B);
-  const size_t per_cta = (size_t)pl.warps_per_cta * pl.ws_doubles_per_warp * sizeof(double);
-  const size_t need = (size_t)pl.grid * per_cta;
-  if (need > 0) {
-    if (!d_workspace) return set_error(POLAR_ENOMEM, "scl: workspace %zu B < required %zu B", (size_t)0, need);
-    if ((uintptr_t)d_workspace & 255) return set_error(POLAR_EALIGN, "scl: workspace must be 256-byte aligned");
-    if (workspace_bytes < need) {   // the kernels are persistent: run with as many CTAs as the workspace holds
-      const int64_t fit = (int64_t)(workspace_bytes / per_cta);
-      if (fit < 1) return set_error(POLAR_ENOMEM, "scl: workspace %zu B < required %zu B", workspace_bytes, per_cta);
-      pl.grid = fit;
-    }
-  }
-  SclParams P;
-  P.logit = d_logit; P.fmask = d_frozen_mask; P.n = n; P.m = ilog2(n); P.B = B;
-  P.best = d_best_packed; P.u_info = d_u_info_f32; P.info_pos = d_info_pos; P.k = k;
-  P.pm_out = d_pm_sorted; P.list = d_list_packed; P.crc_rows = d_crc_rows; P.crc_len = crc_len;
-  P.ws = (double *)d_workspace; P.ws_doubles_per_warp = pl.ws_doubles_per_warp; P.s_glob = pl.s_glob;
-  P.smem_per_warp = pl.smem_per_warp; P.words_global = pl.words_global; P.fast = fast;
-  P.rows = nullptr; P.n_rows = nullptr;
-  return launch_scl_any(P, pl, L, (cudaStream_t)stream);
-}
-
-extern "C" int polar_scl_decode(const float *d_logit, const uint32_t *d_frozen_mask, int n, int L, int64_t B,
-                                uint32_t *d_best_packed, float *d_u_info_f32, const int32_t *d_info_pos, int k,
-                                double *d_pm_sorted, uint32_t *d_list_packed, const uint32_t *d_crc_rows, int crc_len,
-                                void *d_workspace, size_t workspace_bytes, void *stream) {
-  return scl_decode_impl(d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, d_pm_sorted, d_list_packed,
-                         d_crc_rows, crc_len, d_workspace, workspace_bytes, stream, 0);
-}
-#if defined(POLAR_F_BOXPLUS)
-// use_fast_scl = True of the Sionna-style decoder: rate-0 / REP nodes update the path metric at node level
-extern "C" int polar_scl_decode_boxplus_pruned(const float *d_logit, const uint32_t *d_frozen_mask, int n, int L, int64_t B,
-                                               uint32_t *d_best_packed, float *d_u_info_f32, const int32_t *d_info_pos, int k,
-                                               double *d_pm_sorted, uint32_t *d_list_packed, const uint32_t *d_crc_rows, int crc_len,
-                                               void *d_workspace, size_t workspace_bytes, void *stream) {
-  return scl_decode_impl(d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, d_pm_sorted, d_list_packed,
-                         d_crc_rows, crc_len, d_workspace, workspace_bytes, stream, 1);
-}
-#endif

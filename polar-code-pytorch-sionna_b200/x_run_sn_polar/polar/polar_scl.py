@@ -1,6 +1,6 @@
 """SCL decoder with the reference call surface (x_run_sn_polar/polar/polar_scl.py:5-234).
 The NumPy recursion with 2L decoder slots and a full-tree copy per information bit is replaced by one
-launch of the sm_100a kernel `polar_scl_decode` (csrc/polar_scl.cu): fp64 tree and path metrics,
+launch of the sm_100a kernel `polar_scl_decode` (csrc/polar_scl_api.cu): fp64 tree and path metrics,
 lazy copy-on-write through per-stage pointer tables, warp bitonic ranking of the 2L candidates."""
 import numpy as np
 import torch as tc

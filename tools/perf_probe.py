@@ -39,16 +39,9 @@ def main():
         L = int(os.environ.get("L", "8"))
         B = int(sys.argv[3]) if len(sys.argv) > 3 else 1 << 15
         _, _, x = dk.awgn_frontend(tables, B, no, 1234)
-        for kb in [int(v) for v in os.environ.get("KBS", "4").split(",")]:
-            for warps in [int(v) for v in os.environ.get("WARPS", "1,2,4").split(",")]:
-                dk.set_option("POLAR_SCL_SMEM_KB", int(str(kb))); dk.set_option("POLAR_SCL_WARPS", int(str(warps)))
-                try:
-                    f = lambda: dk.scl_decode(x, tables, L, want_packed=True, want_info=False)
-                    best, med = timeit(f, iters=3, warm=1)
-                    print("SCL L=%d n=%d B=%d smemKB=%d warps=%d: %8.3f ms  %.3e cw/s  %.3f Gbit/s info" %
-                          (L, n, B, kb, warps, best, B / best * 1e3, B / best * 1e3 * k / 1e9), flush=True)
-                except Exception as e:
-                    print("SCL kb=%d warps=%d failed: %s" % (kb, warps, e))
+        best, med = timeit(lambda: dk.scl_decode(x, tables, L, want_packed=True, want_info=False), iters=3, warm=1)
+        print("SCL L=%d n=%d B=%d: %8.3f ms  %.3e cw/s  %.3f Gbit/s info" %
+              (L, n, B, best, B / best * 1e3, B / best * 1e3 * k / 1e9), flush=True)
     elif what == "sptest":
         import ctypes
         cnt = torch.zeros(3, dtype=torch.int64, device=dev)
