@@ -174,6 +174,26 @@ int polar_gather_cols_f32(const float *d_x, const int32_t *d_idx, int n_in, int 
                           void *stream);
 int polar_rate_recover_f32(const float *d_x, const int32_t *d_src0, const int32_t *d_src1, const float *d_fill,
                            int n_in, int n_out, int64_t B, float *d_out, void *stream);
+/* polar_nr5g_awgn_frontend: the 5G uplink link up to the decoder in one launch, per codeword: Bernoulli(1/2) payload ->
+ * CRC attach -> channel allocation -> polar transform -> rate matching (the gather index above) -> QPSK/AWGN ->
+ * closed-form demapper (as polar_awgn_frontend).  One warp per codeword.
+ *  n               mother-code length, power of two in [32, 1024]; e: channel bits, 1 <= e <= POLAR_MAX_N
+ *  d_payload_mask  [POLAR_WORDS(n)] bit set at the k payload positions (info_pos[:k])
+ *  d_crc_rows      [n] at payload position info_pos[t]: the CRC generator word of payload bit t (MSB = parity bit 0,
+ *                  i.e. bit crc_len-1-j is parity bit j; CRCEncoder(crc_degree, k)._rows); 0 elsewhere
+ *  d_crc_pos       [crc_len] polar position of parity bit j (info_pos[k + j]); 1 <= crc_len <= 32
+ *  d_rm_idx        [e] polar position sent at channel position i; entries must lie in [0, n) (not checked)
+ *  d_u_packed_out  [B, POLAR_WORDS(n)] payload + CRC at their positions, frozen 0: what a correct decoder returns
+ *  d_c_packed_out  [B, (e+31)/32] rate-matched codeword, LSB first, tail bits 0; may be NULL
+ *  d_logit_out     [B, e] fp32, any 4-byte alignment
+ * Random numbers: the payload is a pure function of (seed, offset + b); row b of the logits equals the first e columns
+ * of polar_qpsk_awgn_llr(seed, offset + b, no, c) for that row's rate-matched codeword c zero-padded to a multiple of 4.
+ * POLAR_EINVAL for bad n / e / crc_len, B < 0, no <= 0 or a null table / output pointer.  B == 0 launches nothing.
+ * No allocation, no synchronisation. */
+int polar_nr5g_awgn_frontend(uint64_t seed, uint64_t offset, float no, const uint32_t *d_payload_mask,
+                             const uint32_t *d_crc_rows, const int32_t *d_crc_pos, int crc_len,
+                             const int32_t *d_rm_idx, int n, int e, int64_t B, uint32_t *d_u_packed_out,
+                             uint32_t *d_c_packed_out, float *d_logit_out, void *stream);
 
 /* ---- BPSK/AWGN LLR front end -----------------------------------------------------------------
  * Replaces System_AWGN_model.forward up to the decoder call (z_sys_model/awgn_model.py:33-40):

@@ -110,6 +110,86 @@ __global__ void __launch_bounds__(256) frontend_kernel(uint64_t seed, uint64_t o
   }
 }
 
+// 5G NR uplink front end (TS 38.212 5.3.1 / 5.4.1 as built by Polar5GEncoder): payload bits -> CRC -> channel
+// allocation -> polar transform -> sub-block interleaver + circular buffer + channel interleaver (one gather index) ->
+// QPSK/AWGN -> closed-form demapper.  One warp per codeword, n <= 1024: one 32-bit word per lane.  The codeword is
+// staged in 128 B of shared memory per warp so that every channel position can read its bit through rm_idx.
+// Random numbers: the payload words are the Philox words of frontend_kernel; the noise of channel group g is that of
+// polar_qpsk_awgn_llr for the rate-matched codeword zero-padded to a multiple of 4.
+__global__ void __launch_bounds__(256) nr5g_frontend_kernel(uint64_t seed, uint64_t offset, float sigma, float scale,
+                                                            const uint32_t *__restrict__ payload_mask,
+                                                            const uint32_t *__restrict__ crc_rows,
+                                                            const int32_t *__restrict__ crc_pos, int crc_len,
+                                                            const int32_t *__restrict__ rm_idx, int n, int m, int e,
+                                                            int64_t B, uint32_t *__restrict__ u_out,
+                                                            uint32_t *__restrict__ c_out, float *__restrict__ logit) {
+  __shared__ uint32_t s_cw[8][32];
+  const int lane = threadIdx.x & 31;
+  uint32_t *cw = s_cw[threadIdx.x >> 5];
+  const int nw = n >> 5, ew = (e + 31) >> 5, ngroups = (e + 3) >> 2;
+  const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  const Philox ph(seed);
+  // parity bit `lane` of the CRC (MSB of the syndrome word = parity bit 0) and the polar position it goes to
+  const int my_crc_pos = lane < crc_len ? __ldg(crc_pos + lane) : 0;
+  for (int64_t b = warp0; b < B; b += nwarps) {
+    const uint64_t id = (uint64_t)b + offset;
+    uint32_t w = 0u;
+    if (lane < nw) {
+      const uint4 rb = ph((uint32_t)id, (uint32_t)(id >> 32), (uint32_t)(lane >> 2), kStreamBits);
+      const uint32_t rw = (lane & 3) == 0 ? rb.x : (lane & 3) == 1 ? rb.y : (lane & 3) == 2 ? rb.z : rb.w;
+      w = rw & __ldg(payload_mask + lane);
+    }
+    uint32_t syn = 0u;
+    for (uint32_t t = w; t; t &= t - 1u) syn ^= __ldg(crc_rows + lane * 32 + __ffs(t) - 1);
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) syn ^= __shfl_xor_sync(0xFFFFFFFFu, syn, d);
+    __syncwarp();                                   // the previous codeword's channel reads are done
+    cw[lane] = w;
+    __syncwarp();
+    if (lane < crc_len && ((syn >> (crc_len - 1 - lane)) & 1u)) atomicOr(cw + (my_crc_pos >> 5), 1u << (my_crc_pos & 31));
+    __syncwarp();
+    uint32_t x[1] = {cw[lane]};
+    if (lane < nw) u_out[b * nw + lane] = x[0];
+    warp_polar_transform<1>(x, m, nw);
+    cw[lane] = x[0];
+    __syncwarp();
+    float *row = logit + b * (int64_t)e;
+    const bool vec = ((uintptr_t)row & 15) == 0;
+    for (int g0 = 0; g0 < ngroups; g0 += 32) {
+      const int g = g0 + lane;
+      uint32_t bits4 = 0u;
+      if (g < ngroups) {
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+          const int p = 4 * g + t;
+          if (p < e) {
+            const int i = __ldg(rm_idx + p);
+            bits4 |= ((cw[i >> 5] >> (i & 31)) & 1u) << t;
+          }
+        }
+        const float4 o = noisy_logits(ph, id, (uint32_t)g, bits4, sigma, scale);
+        if (vec && 4 * g + 3 < e) {
+          *reinterpret_cast<float4 *>(row + 4 * g) = o;
+        } else {
+          row[4 * g] = o.x;
+          if (4 * g + 1 < e) row[4 * g + 1] = o.y;
+          if (4 * g + 2 < e) row[4 * g + 2] = o.z;
+          if (4 * g + 3 < e) row[4 * g + 3] = o.w;
+        }
+      }
+      if (c_out) {                                  // 8 consecutive lanes hold the 32 bits of one codeword word
+        uint32_t cword = bits4 << (4 * (lane & 7));
+        cword |= __shfl_xor_sync(0xFFFFFFFFu, cword, 1);
+        cword |= __shfl_xor_sync(0xFFFFFFFFu, cword, 2);
+        cword |= __shfl_xor_sync(0xFFFFFFFFu, cword, 4);
+        const int wq = g >> 3;
+        if ((lane & 7) == 0 && wq < ew) c_out[b * ew + wq] = cword;
+      }
+    }
+  }
+}
+
 // channel + demapper for caller-supplied codewords (fp32 0/1)
 template <bool BEC = false>
 __global__ void __launch_bounds__(256) qpsk_awgn_kernel(uint64_t seed, uint64_t offset, float sigma, float scale,
@@ -173,6 +253,26 @@ extern "C" int polar_awgn_frontend(uint64_t seed, uint64_t offset, float no, con
 #undef POLAR_FE_LAUNCH
   count_launch();
   POLAR_CHECK_LAUNCH("frontend");
+  return POLAR_OK;
+}
+
+extern "C" int polar_nr5g_awgn_frontend(uint64_t seed, uint64_t offset, float no, const uint32_t *d_payload_mask,
+                                        const uint32_t *d_crc_rows, const int32_t *d_crc_pos, int crc_len,
+                                        const int32_t *d_rm_idx, int n, int e, int64_t B, uint32_t *d_u_packed_out,
+                                        uint32_t *d_c_packed_out, float *d_logit_out, void *stream) {
+  if (!is_pow2(n) || n < 32 || n > 1024) return set_error(POLAR_EINVAL, "nr5g frontend: n=%d must be a power of two in [32,1024]", n);
+  if (e < 1 || e > POLAR_MAX_N) return set_error(POLAR_EINVAL, "nr5g frontend: e=%d outside [1,%d]", e, POLAR_MAX_N);
+  if (crc_len < 1 || crc_len > 32) return set_error(POLAR_EINVAL, "nr5g frontend: crc_len=%d outside [1,32]", crc_len);
+  if (B < 0 || !(no > 0.0f)) return set_error(POLAR_EINVAL, "nr5g frontend: B < 0 or no <= 0");
+  if (!d_payload_mask || !d_crc_rows || !d_crc_pos || !d_rm_idx) return set_error(POLAR_EINVAL, "nr5g frontend: null table pointer");
+  if (B == 0) return POLAR_OK;
+  if (!d_u_packed_out || !d_logit_out) return set_error(POLAR_EINVAL, "nr5g frontend: null output pointer");
+  const float sigma = sqrtf(no * 0.5f), scale = -2.0f * 1.41421356237309505f / no;
+  nr5g_frontend_kernel<<<fe_grid(nr5g_frontend_kernel, B), 256, 0, (cudaStream_t)stream>>>(
+      seed, offset, sigma, scale, d_payload_mask, d_crc_rows, d_crc_pos, crc_len, d_rm_idx, n, ilog2(n), e, B,
+      d_u_packed_out, d_c_packed_out, d_logit_out);
+  count_launch();
+  POLAR_CHECK_LAUNCH("nr5g_frontend");
   return POLAR_OK;
 }
 

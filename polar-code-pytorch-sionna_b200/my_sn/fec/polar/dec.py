@@ -182,7 +182,8 @@ class Polar5GDecoder(nn.Module):
   and the sub-block de-interleaver are folded into one index plan applied by `polar_rate_recover_f32`; the decoder is the
   my_sn `SC_Dec` (boxplus SC) or the CRC-aided `SCL_Dec`.  `dec_type="hybSCL"` runs that `SCL_Dec` with
   `use_hybrid_sc=True`: SC first, list decoding only of the codewords whose SC decision fails the CRC.
-  `return_crc_status=True` works here (the reference stops in a stray breakpoint, dec.py:661)."""
+  `return_crc_status=True` works here (the reference stops in a stray breakpoint, dec.py:661).  `decode_packed` (rate
+  recovery, then the inner decoder's packed path) lets `sim_ber` run a 5G link model on the on-device loop."""
 
   def __init__(self, enc_polar, dec_type="SC", list_size=8, return_crc_status=False, output_dtype=tc.float32):
     super().__init__()
@@ -208,6 +209,7 @@ class Polar5GDecoder(nn.Module):
     if return_crc_status:
       self._dec_crc = self._polar_dec._crc_decoder if dec_type in ("SCL", "hybSCL") else CRCDecoder(enc_polar.enc_crc)
     self._plan_dev = {}
+    self._rec_dev = {}
 
   def _init_interleavers(self):
     """Inverse interleaver patterns (dec.py:584-598) and the fused rate-recovery plan: for polar position j,
@@ -234,10 +236,26 @@ class Polar5GDecoder(nn.Module):
   def rate_recover(self, inputs):
     """[B, n_target] channel logits -> [B, n_polar] decoder logits (dec.py:607-634), on the GPU."""
     dev = inputs.device if inputs.is_cuda else dk.cuda_device(self._enc_polar.device)
+    return dk.rate_recover(inputs.to(device=dev, dtype=tc.float32).reshape(-1, self._n_target), *self._plan_on(dev))
+
+  def _plan_on(self, dev):
     plan = self._plan_dev.get(str(dev))
     if plan is None:
       plan = self._plan_dev[str(dev)] = tuple(tc.from_numpy(a).to(dev) for a in self._plan)
-    return dk.rate_recover(inputs.to(device=dev, dtype=tc.float32).reshape(-1, self._n_target), *plan)
+    return plan
+
+  def decode_packed(self, logits, tables, out=None):
+    """Device fast path of the on-device Monte-Carlo loop: channel logits [B, n_target] -> rate recovery into a
+    per-device buffer (grown, never shrunk) -> the inner decoder's `decode_packed` (SC, SCL or hybrid SCL) with the
+    mother code's `tables`.  Returns the bit-packed decisions [B, words(n_polar)] over all n_polar positions."""
+    dev = tables.dev
+    x = logits.reshape(-1, self._n_target)
+    B = x.shape[0]
+    buf = self._rec_dev.get(str(dev))
+    if buf is None or buf.shape[0] < B:
+      buf = self._rec_dev[str(dev)] = tc.empty((B, self._n_polar), dtype=tc.float32, device=dev)
+    rec = dk.rate_recover(x, *self._plan_on(dev), out=buf[:B])
+    return self._polar_dec.decode_packed(rec, tables, out=out)
 
   def forward(self, inputs):
     inputs = inputs.to(tc.float32)

@@ -45,7 +45,8 @@ _PI_IL_MAX = np.array([0, 2, 4, 7, 9, 14, 19, 20, 24, 25, 26, 28, 31, 34, 42, 45
 class Polar5GEncoder(PolarEncoder):
   """CRC concatenation + polar encoding + 5G rate matching to n coded bits (uplink UCI scheme; the downlink variant
   builds its tables but `forward` raises, exactly like the reference, enc.py:374-376).  No code segmentation, the
-  3 parity-check bits for 12 <= k <= 19 are not used (enc.py:128-134)."""
+  3 parity-check bits for 12 <= k <= 19 are not used (enc.py:128-134).  `frontend_plan()` describes the code to the fused
+  5G front end of `System_AWGN_model` (payload and CRC positions, CRC generator words, the rate-matching index)."""
 
   def __init__(self, k, n, channel_type="uplink", verbose=False, dtype=tc.float32, device='cpu'):
     k = int(k); n = int(n)
@@ -60,6 +61,7 @@ class Polar5GEncoder(PolarEncoder):
     super().__init__(frozen_pos, n_polar, dtype=dtype, device=device)
     self._enc_crc = CRCEncoder(crc_degree, k=k, dtype=dtype)
     self._idx_dev = {}
+    self._fe_plan = None
 
   @property
   def enc_crc(self): return self._enc_crc
@@ -179,6 +181,22 @@ class Polar5GEncoder(PolarEncoder):
       print(f"Polar mother code: k_polar = {k_polar}, n_polar = {n_polar}")
       print("Using", crc_pol); print("Frozen positions: ", frozen_pos); print("Channel type: " + self._channel_type)
     return crc_pol, n_polar, frozen_pos, idx, ind_input
+
+  def frontend_plan(self, dev=None):
+    """The code as the fused 5G front end (`polar_nr5g_awgn_frontend`) sees it, built from this encoder's own tables:
+    the payload occupies info_pos[:k] and the CRC parity bits info_pos[k:] (CRC attach + channel allocation of
+    `forward`), and channel position i sends polar position `_ind_rate_matching[i]`.  Returns the host plan
+    (`d_kernels.NR5GPlan`, numpy), or with `dev` its device copy (built once per device).  Downlink raises like
+    `forward` does."""
+    if self._channel_type == "downlink":
+      raise Exception('error...')                                            # enc.py:374-376
+    plan = self._fe_plan
+    if plan is None:
+      k, info = self._k_target, np.asarray(self.info_pos)
+      plan = self._fe_plan = dk.NR5GPlan(self._n, self._n_target, info[:k],
+                                         self._enc_crc.syndrome_rows(info[:k], self._n), info[k:],
+                                         self._ind_rate_matching)
+    return plan if dev is None else plan.on(dev)
 
   def forward(self, u):
     """info bits [...,k] -> rate-matched codewords [...,n] (enc.py:363-392)."""

@@ -157,10 +157,16 @@ def sim_ber_device(model, ebno_dbs, batch_size, max_mc_iter, target_bit_errs=Non
   verbose = verbose and rank0
   dev = dk.cuda_device(model.device)
   dec = model.decoder
-  frozen_pos = getattr(model.encoder, "frozen_pos", None)
-  if frozen_pos is None:
-    frozen_pos = dec.frozen_pos
-  tables = dk.code_tables(frozen_pos, model.n, dev)
+  if callable(getattr(model, "loop_geometry", None)):
+    # decoder-domain geometry from the link model: a rate-matched code sends E channel bits of a mother code of length
+    # n_polar and counts only its payload bits
+    tables, n_ch, count_mask, k_count = model.loop_geometry(dev)
+  else:
+    frozen_pos = getattr(model.encoder, "frozen_pos", None)
+    if frozen_pos is None:
+      frozen_pos = dec.frozen_pos
+    tables = dk.code_tables(frozen_pos, model.n, dev)
+    n_ch, count_mask, k_count = model.n, tables.info_mask, tables.k
   if model._seed is None:
     model._seed = int(tc.randint(0, 2 ** 62, (1,)).item())
   ebno_dbs = np.asarray(ebno_dbs, dtype=np.float32)
@@ -178,9 +184,9 @@ def sim_ber_device(model, ebno_dbs, batch_size, max_mc_iter, target_bit_errs=Non
   DEPTH = 2 if lookahead else 1
   gmax = 1
   if lookahead:
-    gmax = int(max(1, min(dk.MC_GROUP_MAX, (int(group_mb) << 20) // max(B * model.n * 4, 1), P * max_mc_iter)))
+    gmax = int(max(1, min(dk.MC_GROUP_MAX, (int(group_mb) << 20) // max(B * n_ch * 4, 1), P * max_mc_iter)))
   planner = SweepPlanner(P, target_bit_errs, target_block_errs, max_mc_iter,
-                         per_iter_max=(0.5 * B * tables.k * world, 1.0 * B * world))
+                         per_iter_max=(0.5 * B * k_count * world, 1.0 * B * world))
   if P == 0:
     z = tc.zeros(0, dtype=tc.float32)
     return (z, z, counters, status, iters) if return_counters else (z, z)
@@ -188,14 +194,14 @@ def sim_ber_device(model, ebno_dbs, batch_size, max_mc_iter, target_bit_errs=Non
   n_items = n_groups = 0
   marks = []                                                 # profile: (n_items, 6 timing events) per group
   with tc.cuda.device(dev):
-    nw = dk.words(model.n)
+    nw = dk.words(tables.n)
     state = tc.zeros((P, 8), dtype=tc.int64, device=dev)
     sweep = tc.zeros(8, dtype=tc.int64, device=dev)
-    sizes = tc.tensor([0, 0, B * tables.k, B], dtype=tc.int64, device=dev)
+    sizes = tc.tensor([0, 0, B * k_count, B], dtype=tc.int64, device=dev)
     slots = []
     for _ in range(DEPTH):
       slots.append(dict(u_tx=tc.empty((gmax * B, nw), dtype=tc.int32, device=dev),
-                        llr=tc.empty((gmax * B, model.n), dtype=tc.float32, device=dev),
+                        llr=tc.empty((gmax * B, n_ch), dtype=tc.float32, device=dev),
                         u_hat=tc.empty((gmax * B, nw), dtype=tc.int32, device=dev),
                         delta=tc.zeros((gmax, 4), dtype=tc.int64, device=dev),
                         host=tc.zeros((P + 1, 8), dtype=tc.int64).pin_memory(), event=tc.cuda.Event()))
@@ -219,8 +225,8 @@ def sim_ber_device(model, ebno_dbs, batch_size, max_mc_iter, target_bit_errs=Non
       delta = slot["delta"][:G]
       delta.copy_(sizes.expand(G, 4))                        # (0, 0, bits, blocks) of this rank's shard, per item
       for j in range(G):
-        dk.count_errors_packed(slot["u_tx"][j * B:(j + 1) * B], slot["u_hat"][j * B:(j + 1) * B], tables.info_mask,
-                               model.n, delta[j])
+        dk.count_errors_packed(slot["u_tx"][j * B:(j + 1) * B], slot["u_hat"][j * B:(j + 1) * B], count_mask,
+                               tables.n, delta[j])
       mark(row)
       if dist is not None:
         dist.all_reduce(delta)                               # stream-ordered NCCL all-reduce of G x 4 int64

@@ -7,6 +7,7 @@ are turned into raw device pointers: every decoder / encoder / link-model class 
 calls the CUDA kernels through the functions below.  There is NO CPU fallback: if the library is
 missing, or no CUDA device is present when a kernel is requested, these functions raise.
 """
+import copy
 import ctypes
 import os
 
@@ -64,6 +65,7 @@ _SIGNATURES = {
   "polar_gather_cols_f32": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp]),
   "polar_rate_recover_f32": (_i32, [_vp, _vp, _vp, _vp, _i32, _i32, _i64, _vp, _vp]),
   "polar_awgn_frontend": (_i32, [_u64, _u64, _f32, _vp, _i32, _i64, _vp, _vp, _vp, _vp]),
+  "polar_nr5g_awgn_frontend": (_i32, [_u64, _u64, _f32, _vp, _vp, _vp, _i32, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _vp]),
   "polar_bec_frontend": (_i32, [_u64, _u64, _f32, _f32, _vp, _i32, _i64, _vp, _vp, _vp, _vp]),
   "polar_bec_llr": (_i32, [_u64, _u64, _f32, _f32, _vp, _i32, _i64, _vp, _vp]),
   "polar_qpsk_awgn_llr": (_i32, [_u64, _u64, _f32, _vp, _i32, _i64, _vp, _vp]),
@@ -198,6 +200,40 @@ class CodeTables:
     self.info_rank = tc.from_numpy(rank).to(dev)
     info_mask = (~self.mask_np) & (np.uint32(0xFFFFFFFF) if self.n >= 32 else np.uint32((1 << self.n) - 1))
     self.info_mask = tc.from_numpy(np.asarray(info_mask, dtype=np.uint32).view(np.int32).copy()).to(dev)
+
+
+class NR5GPlan:
+  """What polar_nr5g_awgn_frontend needs to know about one rate-matched 5G code (Polar5GEncoder.frontend_plan).
+  Host fields (numpy): n (mother code), e (channel bits), k (payload bits), crc_len, payload_pos [k], payload_mask
+  [words(n)] uint32, crc_rows [n] uint32, crc_pos [crc_len], rm_idx [e].  `on(dev)` returns the plan with the device
+  copies payload_mask_d / crc_rows_d / crc_pos_d / rm_idx_d / payload_pos_d (int32), built once per device; `dev` is
+  None on the host plan."""
+
+  def __init__(self, n, e, payload_pos, crc_rows, crc_pos, rm_idx):
+    self.n, self.e = int(n), int(e)
+    self.payload_pos = np.asarray(payload_pos, dtype=np.int64)
+    self.k = int(self.payload_pos.shape[0])
+    self.crc_rows = np.asarray(crc_rows, dtype=np.uint32)
+    self.crc_pos = np.asarray(crc_pos, dtype=np.int64)
+    self.crc_len = int(self.crc_pos.shape[0])
+    self.rm_idx = np.asarray(rm_idx, dtype=np.int64)
+    f = np.zeros(max(self.n, 32), dtype=np.uint8)
+    f[self.payload_pos] = 1
+    self.payload_mask = np.packbits(f.reshape(-1, 32), axis=1, bitorder="little").view(np.uint32).reshape(-1)[:words(self.n)].copy()
+    self.dev = None
+    self._on = {}
+
+  def on(self, dev):
+    p = self._on.get(str(dev))
+    if p is None:
+      init_device(dev)
+      p = self._on[str(dev)] = copy.copy(self)
+      p.dev, p._on = dev, None
+      i32 = lambda a: tc.from_numpy(np.ascontiguousarray(a).astype(np.int64).astype(np.int32)).to(dev)
+      p.payload_mask_d = tc.from_numpy(self.payload_mask.view(np.int32).copy()).to(dev)
+      p.crc_rows_d = tc.from_numpy(self.crc_rows.view(np.int32).copy()).to(dev)
+      p.crc_pos_d, p.rm_idx_d, p.payload_pos_d = i32(self.crc_pos), i32(self.rm_idx), i32(self.payload_pos)
+    return p
 
 
 _TABLE_CACHE = {}
@@ -379,6 +415,22 @@ def awgn_frontend(tables, batch_size, no, seed, offset=0, want_codeword=False, o
   return u, c, logit
 
 
+def nr5g_awgn_frontend(plan, batch_size, no, seed, offset=0, want_codeword=False, out=None):
+  """polar_nr5g_awgn_frontend for a device plan (NR5GPlan.on(dev)) -> (u_packed int32 [B, words(n)], c_packed int32
+  [B, (e+31)//32] | None, logits fp32 [B, e]).  u_packed holds payload + CRC at their polar positions.
+  out = (u_packed, logits): caller-owned buffers (Monte-Carlo loop: no allocation per call)."""
+  dev = plan.dev
+  B, n, e = int(batch_size), plan.n, plan.e
+  u = out[0] if out is not None else tc.empty((B, words(n)), dtype=tc.int32, device=dev)
+  c = tc.empty((B, (e + 31) // 32), dtype=tc.int32, device=dev) if want_codeword else None
+  logit = out[1] if out is not None else tc.empty((B, e), dtype=tc.float32, device=dev)
+  with tc.cuda.device(dev):
+    check(lib().polar_nr5g_awgn_frontend(int(seed) & 0xFFFFFFFFFFFFFFFF, int(offset), float(no), ptr(plan.payload_mask_d),
+                                         ptr(plan.crc_rows_d), ptr(plan.crc_pos_d), plan.crc_len, ptr(plan.rm_idx_d), n, e, B,
+                                         ptr(u), ptr(c), ptr(logit), stream_ptr(dev)))
+  return u, c, logit
+
+
 def bec_frontend(tables, batch_size, pe, seed, offset=0, llr_max=100.0, want_codeword=False, out=None):
   """polar_bec_frontend -> (u_packed int32 [B,words], c_packed | None, logits fp32 [B,n] in {0, +-llr_max})."""
   dev = tables.dev
@@ -457,11 +509,13 @@ def gather_cols(x, idx):
   return out
 
 
-def rate_recover(x, src0, src1, fill):
-  """polar_rate_recover_f32: out[b, j] = (src0[j] >= 0 ? x[b, src0[j]] : fill[j]) + (src1[j] >= 0 ? x[b, src1[j]] : 0)."""
+def rate_recover(x, src0, src1, fill, out=None):
+  """polar_rate_recover_f32: out[b, j] = (src0[j] >= 0 ? x[b, src0[j]] : fill[j]) + (src1[j] >= 0 ? x[b, src1[j]] : 0).
+  out: optional caller-owned fp32 [B, len(src0)] buffer."""
   dev = x.device
   x2 = x.to(tc.float32).reshape(-1, x.shape[-1]).contiguous()
-  out = tc.empty((x2.shape[0], src0.shape[0]), dtype=tc.float32, device=dev)
+  if out is None:
+    out = tc.empty((x2.shape[0], src0.shape[0]), dtype=tc.float32, device=dev)
   with tc.cuda.device(dev):
     check(lib().polar_rate_recover_f32(ptr(x2), ptr(src0), ptr(src1), ptr(fill), x2.shape[1], src0.shape[0], x2.shape[0],
                                        ptr(out), stream_ptr(dev)))
