@@ -231,26 +231,21 @@ int polar_count_errors_f32(const float *d_b, const float *d_b_hat, int k, int64_
                            unsigned long long *d_counters, void *stream);
 
 /* ---- Monte-Carlo stop rules on the device ----------------------------------------------------------
- * Replaces the per-iteration host logic of sim_ber (my_sn/sim.py:90-123): accumulate this iteration's counters
- * and evaluate the target-bit-error / target-block-error / max-iteration rules in a one-thread kernel, so the
- * host can keep iterations queued without reading counters back (SURVEY 8f row N1).
- *  d_delta4  uint64[4]: (bit errors, block errors, bits, blocks) of the iteration (all-reduced over ranks when the
- *            batch is sharded); cleared by the call.
- *  d_state8  int64[8]: [0..3] running totals, [4] stop flag, [5] status (1 max iter, 3 bit target, 4 block target,
- *            sim.py:63-66), [6] iterations counted, [7] reserved.  Once [4] is set, later calls only clear d_delta4.
- *  target_* < 0: rule disabled. */
-int polar_mc_control(unsigned long long *d_delta4, long long *d_state8, long long target_bit_errs,
-                     long long target_block_errs, long long max_mc_iter, void *stream);
-
-/* The same rules for a group of 1..POLAR_MC_GROUP_MAX queued iterations that may span SNR points (the Monte-Carlo loop packs
- * several iterations into one decoder launch so that a small per-rank batch still fills the GPU; the outer loop of
- * sim.py:79-133 and its early stop :128-133 move to the device with it).
- *  d_delta        uint64[n_items,4]: counters of each iteration (all-reduced when sharded); cleared by the call.
+ * Replaces the host logic of sim_ber (my_sn/sim.py:79-133): accumulate the counters of a group of 1..POLAR_MC_GROUP_MAX
+ * queued iterations that may span SNR points and evaluate the target-bit-error / target-block-error / max-iteration
+ * rules and the early stop (:128-133) in a one-thread kernel, so the host can keep iterations queued without reading
+ * counters back (SURVEY 8f row N1).  The Monte-Carlo loop packs several iterations into one decoder launch so that a
+ * small per-rank batch still fills the GPU.
+ *  d_delta        uint64[n_items,4]: (bit errors, block errors, bits, blocks) of each iteration (all-reduced over ranks
+ *                 when the batch is sharded); cleared by the call.
  *  h_item_point   HOST int32[n_items]: SNR-point index each iteration was simulated for (read during the call).
- *  d_state        int64[n_points,8]: one polar_mc_control state row per SNR point (status 2 = no errors, early stop).
+ *  d_state        int64[n_points,8]: one state row per SNR point: [0..3] running totals, [4] stop flag, [5] status
+ *                 (1 max iter, 2 no errors (early stop), 3 bit target, 4 block target, sim.py:63-66), [6] iterations
+ *                 counted, [7] reserved.  Once [4] is set, later iterations of that point are ignored.
  *  d_sweep8       int64[8]: [0] current point, [1] sweep ended, [2] iterations counted so far (= position in the random
  *                 number sequence), [3] groups seen, [4] iterations of this group that counted.
  *  expect_q       value of d_sweep8[2] the group was planned for; on a mismatch nothing counts.
+ *  target_*       < 0: rule disabled.
  * Iteration j counts only if all earlier ones of the group did, the sweep has not ended and the loop is at point
  * h_item_point[j]; the first that does not ends the group. */
 #define POLAR_MC_GROUP_MAX 32

@@ -98,27 +98,13 @@ __global__ void __launch_bounds__(256) count_f32_kernel(const float *__restrict_
   }
 }
 
-// Stop rules of sim_ber (my_sn/sim.py:90-118) evaluated on the device, one thread.  state (int64[8]):
-// [0] bit errors [1] block errors [2] bits [3] blocks [4] stop flag [5] status code [6] iterations counted.
-// delta (uint64[4]): this iteration's (bit errors, block errors, bits, blocks), summed over ranks when sharded.
-// Once `stop` is set later iterations are ignored, so the host may enqueue iterations ahead of the counters.
-__global__ void mc_control_kernel(unsigned long long *__restrict__ delta, long long *__restrict__ state,
-                                  long long target_bit, long long target_block, long long max_iter) {
-  if (threadIdx.x != 0 || blockIdx.x != 0) return;
-  if (!state[4]) {
-    state[0] += (long long)delta[0]; state[1] += (long long)delta[1];
-    state[2] += (long long)delta[2]; state[3] += (long long)delta[3];
-    const long long it = ++state[6];
-    if (target_bit >= 0 && state[0] >= target_bit) { state[5] = 3; state[4] = 1; }             // sim.py:107-112
-    else if (target_block >= 0 && state[1] >= target_block) { state[5] = 4; state[4] = 1; }    // sim.py:113-118
-    else if (it >= max_iter) { state[5] = 1; state[4] = 1; }                                   // sim.py:120-123
-  }
-  delta[0] = 0; delta[1] = 0; delta[2] = 0; delta[3] = 0;
-}
-
-// The same rules for a GROUP of queued iterations that may span SNR points (my_sn/sim.py::sim_ber_device packs several
-// iterations -- of one point, or of consecutive points that are predicted to stop -- into one decoder launch so that a
-// small per-rank batch still fills the GPU).  Iteration j of the group was simulated at the noise level of point
+// Stop rules of sim_ber (my_sn/sim.py:90-133) evaluated on the device, one thread, for a GROUP of queued iterations that
+// may span SNR points (my_sn/sim.py::sim_ber_device packs several iterations -- of one point, or of consecutive points
+// that are predicted to stop -- into one decoder launch so that a small per-rank batch still fills the GPU).
+// state (int64[P,8], one row per point): [0] bit errors [1] block errors [2] bits [3] blocks [4] stop flag [5] status code
+// [6] iterations counted.  delta (uint64[G,4]): each iteration's (bit errors, block errors, bits, blocks), summed over
+// ranks when sharded.  Once a point's stop flag is set its later iterations are ignored, so the host may enqueue
+// iterations ahead of the counters.  Iteration j of the group was simulated at the noise level of point
 // item.point[j] with the random numbers of sequence position expect_q + j.  It counts only if it is what the sequential
 // loop (sim.py:79-133) would have run at that position: the sweep has not ended, every earlier iteration of the group
 // counted, and the loop is at that point.  The first iteration that does not count ends the group (its successors sit at
@@ -169,16 +155,6 @@ extern "C" int polar_mc_control_group(unsigned long long *d_delta, const int32_t
                                                               target_bit_errs, target_block_errs, max_mc_iter, early_stop);
   count_launch();
   POLAR_CHECK_LAUNCH("mc_control_group");
-  return POLAR_OK;
-}
-
-extern "C" int polar_mc_control(unsigned long long *d_delta4, long long *d_state8, long long target_bit_errs,
-                                long long target_block_errs, long long max_mc_iter, void *stream) {
-  if (!d_delta4 || !d_state8) return set_error(POLAR_EINVAL, "mc_control: null pointer");
-  if (max_mc_iter < 1) return set_error(POLAR_EINVAL, "mc_control: max_mc_iter < 1");
-  mc_control_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(d_delta4, d_state8, target_bit_errs, target_block_errs, max_mc_iter);
-  count_launch();
-  POLAR_CHECK_LAUNCH("mc_control");
   return POLAR_OK;
 }
 

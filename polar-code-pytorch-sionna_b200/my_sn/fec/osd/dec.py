@@ -35,7 +35,7 @@ class OSDecoder(nn.Module):
       raise ResourceWarning("OSD cant run this (complexity too high). Please use a smaller value for t.")
     # the error patterns themselves (dec.py:54-56) are enumerated inside the kernel, in itertools.combinations order
     self._gm_rows_np = dk.pack_rows(self._gm.detach().cpu().numpy())
-    self._gm_rows = {}
+    self._gm_rows_on = dk.PerDevice(lambda dev: dk.to_device(self._gm_rows_np, dev))
 
   @property
   def gm(self): return self._gm
@@ -46,17 +46,11 @@ class OSDecoder(nn.Module):
   @property
   def t(self): return self._t
 
-  def _rows_on(self, dev):
-    key = (dev.type, dev.index)
-    if key not in self._gm_rows:
-      self._gm_rows[key] = tc.from_numpy(self._gm_rows_np).to(dev)
-    return self._gm_rows[key]
-
   def forward(self, inputs):
     """inputs [..., n] channel logits ln P(1)/P(0) -> [..., n] hard decisions of all codeword bits (dec.py:149-191)."""
     input_shape = inputs.shape
     dev = dk.cuda_device(inputs.device if inputs.is_cuda else None)
     x = inputs.reshape(-1, self._n).to(self.dtype)
-    res = dk.osd_decode(x, self._rows_on(dev), self._n, self._k, self._t)
+    res = dk.osd_decode(x, self._gm_rows_on(dev), self._n, self._k, self._t)
     c_hat = res["c"].reshape(input_shape).to(self.dtype)
     return c_hat if inputs.is_cuda else c_hat.to(inputs.device)

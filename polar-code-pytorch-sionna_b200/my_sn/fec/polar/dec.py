@@ -102,7 +102,7 @@ class SCL_Dec(nn.Module):
     self._hybrid_mode = (dk.HYBRID_MINSUM if not self._boxplus else
                          dk.HYBRID_BOXPLUS_PRUNED if self._pruned else dk.HYBRID_BOXPLUS)
     self._return_crc_status = return_crc_status
-    self._crc_rows = {}
+    self._crc_rows_on = dk.PerDevice(lambda dev: dk.to_device(self._crc_rows_np, dev))
     self.msg_pm = None
     self.list_decoded = None
 
@@ -122,12 +122,7 @@ class SCL_Dec(nn.Module):
   def list_size(self): return self._list_size
 
   def _rows_on(self, dev):
-    if not self._use_crc:
-      return None, 0
-    rows = self._crc_rows.get(str(dev))
-    if rows is None:
-      rows = self._crc_rows[str(dev)] = tc.from_numpy(self._crc_rows_np.view(np.int32).copy()).to(dev)
-    return rows, self._k_crc
+    return (self._crc_rows_on(dev), self._k_crc) if self._use_crc else (None, 0)
 
   def decode_packed(self, logits, tables, out=None):
     """Device fast path of the on-device Monte-Carlo loop: bit-packed decisions of the (CRC-)selected path."""
@@ -152,12 +147,7 @@ class SCL_Dec(nn.Module):
     assert inputs.dim() > 1
     dev = inputs.device if inputs.is_cuda else dk.cuda_device(self.device)
     tables = dk.code_tables(self._frozen_pos, self._n, dev)
-    rows, ln = None, 0
-    if self._use_crc:
-      rows = self._crc_rows.get(str(dev))
-      if rows is None:
-        rows = self._crc_rows[str(dev)] = tc.from_numpy(self._crc_rows_np.view(np.int32).copy()).to(dev)
-      ln = self._k_crc
+    rows, ln = self._rows_on(dev)
     if self._use_hybrid_sc:                          # device path for CPU tensors too (plain copy in and out)
       u_info, self.msg_pm = self._decode_hybrid(inputs, tables, want_info=True)["u_info"], None
     elif not inputs.is_cuda and not self._boxplus:   # CPU tensor: chunked, overlapped H2D / decode / D2H inside one call
@@ -208,8 +198,8 @@ class Polar5GDecoder(nn.Module):
     self._return_crc_status = return_crc_status
     if return_crc_status:
       self._dec_crc = self._polar_dec._crc_decoder if dec_type in ("SCL", "hybSCL") else CRCDecoder(enc_polar.enc_crc)
-    self._plan_dev = {}
-    self._rec_dev = {}
+    self._plan_on = dk.PerDevice(lambda dev: tuple(dk.to_device(a, dev) for a in self._plan))
+    self._rec = dk.DeviceBuffer(tc.float32)
 
   def _init_interleavers(self):
     """Inverse interleaver patterns (dec.py:584-598) and the fused rate-recovery plan: for polar position j,
@@ -238,12 +228,6 @@ class Polar5GDecoder(nn.Module):
     dev = inputs.device if inputs.is_cuda else dk.cuda_device(self._enc_polar.device)
     return dk.rate_recover(inputs.to(device=dev, dtype=tc.float32).reshape(-1, self._n_target), *self._plan_on(dev))
 
-  def _plan_on(self, dev):
-    plan = self._plan_dev.get(str(dev))
-    if plan is None:
-      plan = self._plan_dev[str(dev)] = tuple(tc.from_numpy(a).to(dev) for a in self._plan)
-    return plan
-
   def decode_packed(self, logits, tables, out=None):
     """Device fast path of the on-device Monte-Carlo loop: channel logits [B, n_target] -> rate recovery into a
     per-device buffer (grown, never shrunk) -> the inner decoder's `decode_packed` (SC, SCL or hybrid SCL) with the
@@ -251,10 +235,8 @@ class Polar5GDecoder(nn.Module):
     dev = tables.dev
     x = logits.reshape(-1, self._n_target)
     B = x.shape[0]
-    buf = self._rec_dev.get(str(dev))
-    if buf is None or buf.shape[0] < B:
-      buf = self._rec_dev[str(dev)] = tc.empty((B, self._n_polar), dtype=tc.float32, device=dev)
-    rec = dk.rate_recover(x, *self._plan_on(dev), out=buf[:B])
+    buf = self._rec(dev, B * self._n_polar)[:B * self._n_polar].view(B, self._n_polar)
+    rec = dk.rate_recover(x, *self._plan_on(dev), out=buf)
     return self._polar_dec.decode_packed(rec, tables, out=out)
 
   def forward(self, inputs):

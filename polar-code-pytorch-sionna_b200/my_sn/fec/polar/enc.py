@@ -60,7 +60,7 @@ class Polar5GEncoder(PolarEncoder):
     self._ind_input_int = idx_input
     super().__init__(frozen_pos, n_polar, dtype=dtype, device=device)
     self._enc_crc = CRCEncoder(crc_degree, k=k, dtype=dtype)
-    self._idx_dev = {}
+    self._idx_on = dk.PerDevice(lambda dev: dk.to_device(self._ind_rate_matching.astype(np.int32), dev))
     self._fe_plan = None
 
   @property
@@ -205,11 +205,7 @@ class Polar5GEncoder(PolarEncoder):
     if self._channel_type == "downlink":
       raise Exception('error...')                                            # enc.py:374-376
     c = super().forward(u_crc)                                               # channel allocation + polar transform (GPU)
-    dev = c.device
-    idx = self._idx_dev.get(str(dev))
-    if idx is None:
-      idx = self._idx_dev[str(dev)] = tc.from_numpy(self._ind_rate_matching.astype(np.int32)).to(dev)
-    out = dk.gather_cols(c, idx)                                             # sub-block + circular buffer + channel interleaver
+    out = dk.gather_cols(c, self._idx_on(c.device))                          # sub-block + circular buffer + channel interleaver
     shape = list(u.shape[:-1]) + [self._n_target]
     shape[0] = -1
     return out.reshape(shape).to(self.dtype)

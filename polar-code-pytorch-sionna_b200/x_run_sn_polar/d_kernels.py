@@ -71,7 +71,6 @@ _SIGNATURES = {
   "polar_qpsk_awgn_llr": (_i32, [_u64, _u64, _f32, _vp, _i32, _i64, _vp, _vp]),
   "polar_count_errors_packed": (_i32, [_vp, _vp, _vp, _i32, _i64, _vp, _vp]),
   "polar_count_errors_f32": (_i32, [_vp, _vp, _i32, _i64, _vp, _vp]),
-  "polar_mc_control": (_i32, [_vp, _vp, ctypes.c_longlong, ctypes.c_longlong, ctypes.c_longlong, _vp]),
   "polar_mc_control_group": (_i32, [_vp, _vp, _i32, _vp, _i32, _vp, ctypes.c_longlong, ctypes.c_longlong, ctypes.c_longlong,
                                     ctypes.c_longlong, _i32, _vp]),
   "polar_osd_decode": (_i32, [_vp, _vp, _i32, _i32, _i32, _i64, _vp, _vp, _vp, _vp]),
@@ -153,12 +152,64 @@ def to_numpy_pos(frozen_pos):
   return np.asarray(frozen_pos).astype(np.int64)
 
 
-def frozen_mask_words(frozen_pos, n):
-  """uint32[words(n)]: bit (i % 32) of word (i // 32) set <=> position i frozen (as int32 bit pattern)."""
-  f = np.zeros(max(n, 32), dtype=np.uint8)
-  f[to_numpy_pos(frozen_pos)] = 1
-  w = np.packbits(f.reshape(-1, 32), axis=1, bitorder="little").view(np.uint32).reshape(-1)
-  return w[:words(n)].copy()
+def pack_rows(m):
+  """0/1 matrix [r, n] (numpy) -> uint32 bit-packed rows [r, (n+31)//32], position i = bit i%32 of word i//32 (as int32).
+  The one bit packer of the host tables: frozen masks, 5G payload masks, OSD generator rows."""
+  m = np.asarray(m) != 0
+  r, n = m.shape
+  bits = np.zeros((r, (n + 31) // 32 * 32), dtype=np.uint8)
+  bits[:, :n] = m
+  return np.packbits(bits.reshape(r, -1, 32), axis=2, bitorder="little").view(np.int32).reshape(r, -1)
+
+
+def frozen_mask_words(pos, n):
+  """uint32[words(n)]: bit (i % 32) of word (i // 32) set <=> position i in `pos` (the frozen set of a code, or the payload
+  positions of a 5G code)."""
+  row = np.zeros((1, n), dtype=np.uint8)
+  row[0, to_numpy_pos(pos)] = 1
+  return pack_rows(row)[0].view(np.uint32)
+
+
+def to_device(a, dev):
+  """Device copy of host array `a`; uint32 bit patterns are stored as int32, the type the kernel wrappers pass."""
+  a = np.asarray(a)
+  return tc.from_numpy((a.view(np.int32) if a.dtype == np.uint32 else a).copy()).to(dev)
+
+
+def _indexed(dev):
+  """`dev` as a torch.device with an explicit index (`cuda` = the current device): the key of every per-device store."""
+  dev = tc.device(dev)
+  return tc.device("cuda", tc.cuda.current_device()) if dev.type == "cuda" and dev.index is None else dev
+
+
+class PerDevice:
+  """Objects made by `build(dev, *key)` once per (device, key) and kept: device copies of host tables, or objects derived
+  from them.  Each owner (a decoder, a plan, this module) holds its own."""
+
+  def __init__(self, build):
+    self._build, self._made = build, {}
+
+  def __call__(self, dev, *key):
+    k = (_indexed(dev),) + key
+    obj = self._made.get(k)
+    if obj is None:
+      obj = self._made[k] = self._build(*k)
+    return obj
+
+
+class DeviceBuffer:
+  """Scratch memory: one flat `dtype` buffer per device, replaced by one of `numel + slack` elements whenever a call needs
+  more than it holds, never shrunk.  All streams of a device share it, so two streams must not use it at the same time."""
+
+  def __init__(self, dtype, slack=0):
+    self._dtype, self._slack, self._bufs = dtype, slack, {}
+
+  def __call__(self, dev, numel):
+    dev = _indexed(dev)
+    buf = self._bufs.get(dev)
+    if buf is None or buf.numel() < numel:
+      buf = self._bufs[dev] = tc.empty(numel + self._slack, dtype=self._dtype, device=dev)
+    return buf
 
 
 _INITIALISED = set()
@@ -195,11 +246,10 @@ class CodeTables:
     self.mask_np = frozen_mask_words(fp, self.n)
     rank = np.full(self.n, -1, dtype=np.int32)
     rank[self.info_pos_np] = np.arange(self.k, dtype=np.int32)
-    self.frozen_mask = tc.from_numpy(self.mask_np.view(np.int32).copy()).to(dev)
-    self.info_pos = tc.from_numpy(self.info_pos_np.astype(np.int32)).to(dev)
-    self.info_rank = tc.from_numpy(rank).to(dev)
-    info_mask = (~self.mask_np) & (np.uint32(0xFFFFFFFF) if self.n >= 32 else np.uint32((1 << self.n) - 1))
-    self.info_mask = tc.from_numpy(np.asarray(info_mask, dtype=np.uint32).view(np.int32).copy()).to(dev)
+    self.frozen_mask = to_device(self.mask_np, dev)
+    self.info_pos = to_device(self.info_pos_np.astype(np.int32), dev)
+    self.info_rank = to_device(rank, dev)
+    self.info_mask = to_device((~self.mask_np) & (np.uint32(0xFFFFFFFF) if self.n >= 32 else np.uint32((1 << self.n) - 1)), dev)
 
 
 class NR5GPlan:
@@ -217,42 +267,70 @@ class NR5GPlan:
     self.crc_pos = np.asarray(crc_pos, dtype=np.int64)
     self.crc_len = int(self.crc_pos.shape[0])
     self.rm_idx = np.asarray(rm_idx, dtype=np.int64)
-    f = np.zeros(max(self.n, 32), dtype=np.uint8)
-    f[self.payload_pos] = 1
-    self.payload_mask = np.packbits(f.reshape(-1, 32), axis=1, bitorder="little").view(np.uint32).reshape(-1)[:words(self.n)].copy()
+    self.payload_mask = frozen_mask_words(self.payload_pos, self.n)
     self.dev = None
-    self._on = {}
+    self._on = PerDevice(self._device_copy)
 
   def on(self, dev):
-    p = self._on.get(str(dev))
-    if p is None:
-      init_device(dev)
-      p = self._on[str(dev)] = copy.copy(self)
-      p.dev, p._on = dev, None
-      i32 = lambda a: tc.from_numpy(np.ascontiguousarray(a).astype(np.int64).astype(np.int32)).to(dev)
-      p.payload_mask_d = tc.from_numpy(self.payload_mask.view(np.int32).copy()).to(dev)
-      p.crc_rows_d = tc.from_numpy(self.crc_rows.view(np.int32).copy()).to(dev)
-      p.crc_pos_d, p.rm_idx_d, p.payload_pos_d = i32(self.crc_pos), i32(self.rm_idx), i32(self.payload_pos)
+    return self._on(dev)
+
+  def _device_copy(self, dev):
+    init_device(dev)
+    p = copy.copy(self)
+    p.dev = dev
+    p.payload_mask_d, p.crc_rows_d = to_device(self.payload_mask, dev), to_device(self.crc_rows, dev)
+    p.crc_pos_d, p.rm_idx_d, p.payload_pos_d = (to_device(a.astype(np.int32), dev)
+                                                for a in (self.crc_pos, self.rm_idx, self.payload_pos))
     return p
 
 
-_TABLE_CACHE = {}
+_code_tables = PerDevice(lambda dev, fp, n: CodeTables(np.frombuffer(fp, dtype=np.int64), n, dev))
 
 
 def code_tables(frozen_pos, n, dev):
-  key = (to_numpy_pos(frozen_pos).tobytes(), int(n), str(dev))
-  tb = _TABLE_CACHE.get(key)
-  if tb is None:
-    tb = _TABLE_CACHE[key] = CodeTables(frozen_pos, n, dev)
-  return tb
+  """The CodeTables of (frozen set, n) on `dev`, built on first use."""
+  return _code_tables(dev, to_numpy_pos(frozen_pos).tobytes(), int(n))
 
 
 # ---- kernel wrappers (device tensors in, device tensors out) -------------------------------------------
+_workspace = DeviceBuffer(tc.uint8, slack=256)      # the list decoders' workspace
+
+
+def _call(dev, name, *args, workspace=None):
+  """Run library function `name` on `dev` with `args` and the device's current stream; raise on its error code.
+  workspace = (size function name, its args): the list-decoder workspace (NULL when 0 bytes) and its size go before the
+  stream.  The size is asked on `dev`: it depends on the device's SM count."""
+  with tc.cuda.device(dev):
+    if workspace is not None:
+      need = int(getattr(lib(), workspace[0])(*workspace[1]))
+      args += (ptr(_workspace(dev, need)) if need else None, need)
+    check(getattr(lib(), name)(*args, stream_ptr(dev)))
+
+
+def _out(dev, shape, dtype, want=True, given=None):
+  """An output of a wrapper: the caller-owned buffer `given` if any, else a new tensor if the output is wanted, else None."""
+  if given is not None:
+    return given
+  return tc.empty(shape, dtype=dtype, device=dev) if want else None
+
+
+def _philox_key(seed):
+  return int(seed) & 0xFFFFFFFFFFFFFFFF
+
+
+def _stop_target(target):
+  return -1 if target is None else int(target)     # -1: the rule is disabled
+
+
 def _prep_logits(x, n, dev):
   x = x.to(device=dev, dtype=tc.float32).reshape(-1, n)
   if not x.is_contiguous() or x.data_ptr() % 16:
     x = x.contiguous().clone() if x.data_ptr() % 16 else x.contiguous()
   return x
+
+
+def _rows(x):
+  return x.to(tc.float32).reshape(-1, x.shape[-1]).contiguous()
 
 
 def sc_decode(logits, tables, want_info=True, want_packed=False, boxplus=False, out_packed=None):
@@ -262,17 +340,11 @@ def sc_decode(logits, tables, want_info=True, want_packed=False, boxplus=False, 
   dev = tables.dev
   x = _prep_logits(logits, tables.n, dev)
   B = x.shape[0]
-  u_info = tc.empty((B, tables.k), dtype=tc.float32, device=dev) if want_info else None
-  u_packed = out_packed if out_packed is not None else (
-    tc.empty((B, words(tables.n)), dtype=tc.int32, device=dev) if want_packed else None)
-  with tc.cuda.device(dev):
-    fn = lib().polar_sc_decode_boxplus_f32 if boxplus else lib().polar_sc_decode_f32
-    check(fn(ptr(x), ptr(tables.frozen_mask), tables.n, B, ptr(u_packed), ptr(u_info), ptr(tables.info_pos), tables.k,
-             stream_ptr(dev)))
+  u_info = _out(dev, (B, tables.k), tc.float32, want_info)
+  u_packed = _out(dev, (B, words(tables.n)), tc.int32, want_packed, out_packed)
+  _call(dev, "polar_sc_decode_boxplus_f32" if boxplus else "polar_sc_decode_f32", ptr(x), ptr(tables.frozen_mask), tables.n,
+        B, ptr(u_packed), ptr(u_info), ptr(tables.info_pos), tables.k)
   return u_info, u_packed
-
-
-_WS_CACHE = {}
 
 
 def scl_decode(logits, tables, list_size, crc_rows=None, crc_len=0, want_info=True, want_packed=False,
@@ -282,37 +354,16 @@ def scl_decode(logits, tables, list_size, crc_rows=None, crc_len=0, want_info=Tr
   dev = tables.dev
   x = _prep_logits(logits, tables.n, dev)
   B, n, L = x.shape[0], tables.n, int(list_size)
-  out = {"u_info": None, "u_packed": None, "pm": None, "list": None}
-  if want_info:
-    out["u_info"] = tc.empty((B, tables.k), dtype=tc.float32, device=dev)
-  if out_packed is not None:
-    out["u_packed"] = out_packed
-  elif want_packed:
-    out["u_packed"] = tc.empty((B, words(n)), dtype=tc.int32, device=dev)
-  if want_pm:
-    out["pm"] = tc.empty((B, L), dtype=tc.float64, device=dev)
-  if want_list:
-    out["list"] = tc.empty((B, L, words(n)), dtype=tc.int32, device=dev)
-  with tc.cuda.device(dev):
-    fn_ws = lib().polar_scl_boxplus_workspace_bytes if boxplus else lib().polar_scl_workspace_bytes
-    fn_dec = lib().polar_scl_decode if not boxplus else (
-      lib().polar_scl_decode_boxplus_pruned if pruned else lib().polar_scl_decode_boxplus)   # pruned: use_fast_scl node shortcuts
-    need = int(fn_ws(n, L, B)) if B > 0 else 0
-    ws = _workspace(dev, need)
-    check(fn_dec(ptr(x), ptr(tables.frozen_mask), n, L, B, ptr(out["u_packed"]), ptr(out["u_info"]),
-                                 ptr(tables.info_pos), tables.k, ptr(out["pm"]), ptr(out["list"]),
-                                 ptr(crc_rows), int(crc_len), ptr(ws), need, stream_ptr(dev)))
+  out = {"u_info": _out(dev, (B, tables.k), tc.float32, want_info),
+         "u_packed": _out(dev, (B, words(n)), tc.int32, want_packed, out_packed),
+         "pm": _out(dev, (B, L), tc.float64, want_pm),
+         "list": _out(dev, (B, L, words(n)), tc.int32, want_list)}
+  name = "polar_scl_decode" if not boxplus else (
+    "polar_scl_decode_boxplus_pruned" if pruned else "polar_scl_decode_boxplus")   # pruned: use_fast_scl node shortcuts
+  ws = "polar_scl_boxplus_workspace_bytes" if boxplus else "polar_scl_workspace_bytes"
+  _call(dev, name, ptr(x), ptr(tables.frozen_mask), n, L, B, ptr(out["u_packed"]), ptr(out["u_info"]), ptr(tables.info_pos),
+        tables.k, ptr(out["pm"]), ptr(out["list"]), ptr(crc_rows), int(crc_len), workspace=(ws, (n, L, B)))
   return out
-
-
-def _workspace(dev, need):
-  """The per-device list-decoder workspace (grown, never shrunk), or None when `need` is 0."""
-  if not need:
-    return None
-  ws = _WS_CACHE.get(str(dev))
-  if ws is None or ws.numel() < need:
-    ws = _WS_CACHE[str(dev)] = tc.empty(need + 256, dtype=tc.uint8, device=dev)
-  return ws
 
 
 HYBRID_MINSUM, HYBRID_BOXPLUS, HYBRID_BOXPLUS_PRUNED = 0, 1, 2
@@ -327,15 +378,11 @@ def scl_decode_hybrid(logits, tables, list_size, crc_rows, crc_len, cn_mode, wan
   dev = tables.dev
   x = _prep_logits(logits, tables.n, dev)
   B, n, L = x.shape[0], tables.n, int(list_size)
-  out = {"u_info": tc.empty((B, tables.k), dtype=tc.float32, device=dev) if want_info else None,
-         "u_packed": out_packed if out_packed is not None else (
-           tc.empty((B, words(n)), dtype=tc.int32, device=dev) if want_packed else None)}
-  with tc.cuda.device(dev):
-    need = int(lib().polar_scl_hybrid_workspace_bytes(n, L, B, int(cn_mode))) if B > 0 else 0
-    ws = _workspace(dev, need)
-    check(lib().polar_scl_decode_hybrid(ptr(x), ptr(tables.frozen_mask), n, L, B, ptr(out["u_packed"]), ptr(out["u_info"]),
-                                        ptr(tables.info_pos), tables.k, ptr(crc_rows), int(crc_len), int(cn_mode),
-                                        ptr(n_list_out), ptr(ws), need, stream_ptr(dev)))
+  out = {"u_info": _out(dev, (B, tables.k), tc.float32, want_info),
+         "u_packed": _out(dev, (B, words(n)), tc.int32, want_packed, out_packed)}
+  _call(dev, "polar_scl_decode_hybrid", ptr(x), ptr(tables.frozen_mask), n, L, B, ptr(out["u_packed"]), ptr(out["u_info"]),
+        ptr(tables.info_pos), tables.k, ptr(crc_rows), int(crc_len), int(cn_mode), ptr(n_list_out),
+        workspace=("polar_scl_hybrid_workspace_bytes", (n, L, B, int(cn_mode))))
   return out
 
 
@@ -347,12 +394,9 @@ def _host_logits(x, n):
   return x.contiguous()
 
 
-def sc_decode_host(logits_cpu, tables, boxplus=False):
+def sc_decode_host(logits_cpu, tables):
   """SC_Dec.forward on a CPU tensor: polar_sc_decode_host_f32 (chunked H2D -> decode -> D2H on two streams inside the call).
   Returns the [B, k] fp32 API tensor in page-locked host memory (torch's caching host allocator recycles it)."""
-  if boxplus:      # the boxplus decoders have no host-buffer entry point: plain copy, decode, copy back
-    u, _ = sc_decode(logits_cpu, tables, want_info=True, boxplus=True)
-    return u.cpu()
   x = _host_logits(logits_cpu, tables.n)
   B = x.shape[0]
   out = tc.empty((B, tables.k), dtype=tc.float32, pin_memory=B > 0)
@@ -385,33 +429,34 @@ def encode_f32(u, tables, want_packed=False):
   dev = tables.dev
   u = u.to(device=dev, dtype=tc.float32).reshape(-1, tables.k).contiguous()
   B = u.shape[0]
-  c = tc.empty((B, tables.n), dtype=tc.float32, device=dev)
-  cp = tc.empty((B, words(tables.n)), dtype=tc.int32, device=dev) if want_packed else None
-  with tc.cuda.device(dev):
-    check(lib().polar_encode_f32(ptr(u), ptr(tables.info_rank), tables.n, tables.k, B, ptr(c), ptr(cp), stream_ptr(dev)))
+  c = _out(dev, (B, tables.n), tc.float32)
+  cp = _out(dev, (B, words(tables.n)), tc.int32, want_packed)
+  _call(dev, "polar_encode_f32", ptr(u), ptr(tables.info_rank), tables.n, tables.k, B, ptr(c), ptr(cp))
   return (c, cp) if want_packed else c
 
 
 def encode_packed(u_full_packed, n):
-  dev = u_full_packed.device
   x = u_full_packed.contiguous()
   out = tc.empty_like(x)
-  with tc.cuda.device(dev):
-    check(lib().polar_encode_packed(ptr(x), int(n), x.shape[0], ptr(out), stream_ptr(dev)))
+  _call(x.device, "polar_encode_packed", ptr(x), int(n), x.shape[0], ptr(out))
   return out
+
+
+def _frontend_out(dev, B, n, e, want_codeword, out):
+  """(u_packed int32 [B, words(n)], c_packed int32 [B, (e+31)//32] | None, logits fp32 [B, e]) of a front end;
+  out = (u_packed, logits): caller-owned buffers (Monte-Carlo loop: no allocation per call)."""
+  u, logit = out if out is not None else (None, None)
+  return (_out(dev, (B, words(n)), tc.int32, given=u), _out(dev, (B, (e + 31) // 32), tc.int32, want_codeword),
+          _out(dev, (B, e), tc.float32, given=logit))
 
 
 def awgn_frontend(tables, batch_size, no, seed, offset=0, want_codeword=False, out=None):
   """polar_awgn_frontend -> (u_packed int32 [B,words], c_packed | None, logits fp32 [B,n]).
   out = (u_packed, logits): caller-owned buffers (Monte-Carlo loop: no allocation per call)."""
-  dev = tables.dev
-  B, n = int(batch_size), tables.n
-  u = out[0] if out is not None else tc.empty((B, words(n)), dtype=tc.int32, device=dev)
-  c = tc.empty((B, words(n)), dtype=tc.int32, device=dev) if want_codeword else None
-  logit = out[1] if out is not None else tc.empty((B, n), dtype=tc.float32, device=dev)
-  with tc.cuda.device(dev):
-    check(lib().polar_awgn_frontend(int(seed) & 0xFFFFFFFFFFFFFFFF, int(offset), float(no), ptr(tables.frozen_mask), n, B,
-                                    ptr(u), ptr(c), ptr(logit), stream_ptr(dev)))
+  dev, B, n = tables.dev, int(batch_size), tables.n
+  u, c, logit = _frontend_out(dev, B, n, n, want_codeword, out)
+  _call(dev, "polar_awgn_frontend", _philox_key(seed), int(offset), float(no), ptr(tables.frozen_mask), n, B, ptr(u), ptr(c),
+        ptr(logit))
   return u, c, logit
 
 
@@ -419,66 +464,49 @@ def nr5g_awgn_frontend(plan, batch_size, no, seed, offset=0, want_codeword=False
   """polar_nr5g_awgn_frontend for a device plan (NR5GPlan.on(dev)) -> (u_packed int32 [B, words(n)], c_packed int32
   [B, (e+31)//32] | None, logits fp32 [B, e]).  u_packed holds payload + CRC at their polar positions.
   out = (u_packed, logits): caller-owned buffers (Monte-Carlo loop: no allocation per call)."""
-  dev = plan.dev
-  B, n, e = int(batch_size), plan.n, plan.e
-  u = out[0] if out is not None else tc.empty((B, words(n)), dtype=tc.int32, device=dev)
-  c = tc.empty((B, (e + 31) // 32), dtype=tc.int32, device=dev) if want_codeword else None
-  logit = out[1] if out is not None else tc.empty((B, e), dtype=tc.float32, device=dev)
-  with tc.cuda.device(dev):
-    check(lib().polar_nr5g_awgn_frontend(int(seed) & 0xFFFFFFFFFFFFFFFF, int(offset), float(no), ptr(plan.payload_mask_d),
-                                         ptr(plan.crc_rows_d), ptr(plan.crc_pos_d), plan.crc_len, ptr(plan.rm_idx_d), n, e, B,
-                                         ptr(u), ptr(c), ptr(logit), stream_ptr(dev)))
+  dev, B, n, e = plan.dev, int(batch_size), plan.n, plan.e
+  u, c, logit = _frontend_out(dev, B, n, e, want_codeword, out)
+  _call(dev, "polar_nr5g_awgn_frontend", _philox_key(seed), int(offset), float(no), ptr(plan.payload_mask_d), ptr(plan.crc_rows_d),
+        ptr(plan.crc_pos_d), plan.crc_len, ptr(plan.rm_idx_d), n, e, B, ptr(u), ptr(c), ptr(logit))
   return u, c, logit
 
 
 def bec_frontend(tables, batch_size, pe, seed, offset=0, llr_max=100.0, want_codeword=False, out=None):
   """polar_bec_frontend -> (u_packed int32 [B,words], c_packed | None, logits fp32 [B,n] in {0, +-llr_max})."""
-  dev = tables.dev
-  B, n = int(batch_size), tables.n
-  u = out[0] if out is not None else tc.empty((B, words(n)), dtype=tc.int32, device=dev)
-  c = tc.empty((B, words(n)), dtype=tc.int32, device=dev) if want_codeword else None
-  logit = out[1] if out is not None else tc.empty((B, n), dtype=tc.float32, device=dev)
-  with tc.cuda.device(dev):
-    check(lib().polar_bec_frontend(int(seed) & 0xFFFFFFFFFFFFFFFF, int(offset), float(pe), float(llr_max),
-                                   ptr(tables.frozen_mask), n, B, ptr(u), ptr(c), ptr(logit), stream_ptr(dev)))
+  dev, B, n = tables.dev, int(batch_size), tables.n
+  u, c, logit = _frontend_out(dev, B, n, n, want_codeword, out)
+  _call(dev, "polar_bec_frontend", _philox_key(seed), int(offset), float(pe), float(llr_max), ptr(tables.frozen_mask), n, B,
+        ptr(u), ptr(c), ptr(logit))
   return u, c, logit
 
 
 def bec_llr(c, pe, seed, offset=0, llr_max=100.0):
-  dev = c.device
-  c2 = c.to(tc.float32).reshape(-1, c.shape[-1]).contiguous()
+  c2 = _rows(c)
   out = tc.empty_like(c2)
-  with tc.cuda.device(dev):
-    check(lib().polar_bec_llr(int(seed) & 0xFFFFFFFFFFFFFFFF, int(offset), float(pe), float(llr_max), ptr(c2), c2.shape[1],
-                              c2.shape[0], ptr(out), stream_ptr(dev)))
+  _call(c.device, "polar_bec_llr", _philox_key(seed), int(offset), float(pe), float(llr_max), ptr(c2), c2.shape[1], c2.shape[0],
+        ptr(out))
   return out.reshape(c.shape)
 
 
 def qpsk_awgn_llr(c, no, seed, offset=0):
-  dev = c.device
-  c2 = c.to(tc.float32).reshape(-1, c.shape[-1]).contiguous()
+  c2 = _rows(c)
   out = tc.empty_like(c2)
-  with tc.cuda.device(dev):
-    check(lib().polar_qpsk_awgn_llr(int(seed) & 0xFFFFFFFFFFFFFFFF, int(offset), float(no), ptr(c2), c2.shape[1], c2.shape[0],
-                                    ptr(out), stream_ptr(dev)))
+  _call(c.device, "polar_qpsk_awgn_llr", _philox_key(seed), int(offset), float(no), ptr(c2), c2.shape[1], c2.shape[0], ptr(out))
   return out.reshape(c.shape)
 
 
 def unpack_info(packed, pos, n):
   dev = packed.device
   B, k = packed.shape[0], pos.shape[0]
-  out = tc.empty((B, k), dtype=tc.float32, device=dev)
-  with tc.cuda.device(dev):
-    check(lib().polar_unpack_info_f32(ptr(packed.contiguous()), ptr(pos), int(n), k, B, ptr(out), stream_ptr(dev)))
+  out = _out(dev, (B, k), tc.float32)
+  _call(dev, "polar_unpack_info_f32", ptr(packed.contiguous()), ptr(pos), int(n), k, B, ptr(out))
   return out
 
 
 def pack_bits(x):
-  dev = x.device
-  x2 = x.to(tc.float32).reshape(-1, x.shape[-1]).contiguous()
-  out = tc.empty((x2.shape[0], words(x2.shape[1])), dtype=tc.int32, device=dev)
-  with tc.cuda.device(dev):
-    check(lib().polar_pack_bits_f32(ptr(x2), x2.shape[1], x2.shape[0], ptr(out), stream_ptr(dev)))
+  x2 = _rows(x)
+  out = _out(x.device, (x2.shape[0], words(x2.shape[1])), tc.int32)
+  _call(x.device, "polar_pack_bits_f32", ptr(x2), x2.shape[1], x2.shape[0], ptr(out))
   return out
 
 
@@ -488,47 +516,30 @@ def count_errors_f32(b, b_hat, counters):
   k = b.shape[-1]
   b2 = b.to(device=dev, dtype=tc.float32).reshape(-1, k).contiguous()
   h2 = b_hat.to(device=dev, dtype=tc.float32).reshape(-1, k).contiguous()
-  with tc.cuda.device(dev):
-    check(lib().polar_count_errors_f32(ptr(b2), ptr(h2), k, b2.shape[0], ptr(counters), stream_ptr(dev)))
+  _call(dev, "polar_count_errors_f32", ptr(b2), ptr(h2), k, b2.shape[0], ptr(counters))
 
 
 def count_errors_packed(a, b, mask, n, counters):
-  dev = counters.device
-  with tc.cuda.device(dev):
-    check(lib().polar_count_errors_packed(ptr(a.contiguous()), ptr(b.contiguous()), ptr(mask), int(n), a.shape[0],
-                                          ptr(counters), stream_ptr(dev)))
+  _call(counters.device, "polar_count_errors_packed", ptr(a.contiguous()), ptr(b.contiguous()), ptr(mask), int(n), a.shape[0],
+        ptr(counters))
 
 
 def gather_cols(x, idx):
   """polar_gather_cols_f32: out[b, e] = x[b, idx[e]] (idx int32 device tensor)."""
-  dev = x.device
-  x2 = x.to(tc.float32).reshape(-1, x.shape[-1]).contiguous()
-  out = tc.empty((x2.shape[0], idx.shape[0]), dtype=tc.float32, device=dev)
-  with tc.cuda.device(dev):
-    check(lib().polar_gather_cols_f32(ptr(x2), ptr(idx), x2.shape[1], idx.shape[0], x2.shape[0], ptr(out), stream_ptr(dev)))
+  x2 = _rows(x)
+  out = _out(x.device, (x2.shape[0], idx.shape[0]), tc.float32)
+  _call(x.device, "polar_gather_cols_f32", ptr(x2), ptr(idx), x2.shape[1], idx.shape[0], x2.shape[0], ptr(out))
   return out
 
 
 def rate_recover(x, src0, src1, fill, out=None):
   """polar_rate_recover_f32: out[b, j] = (src0[j] >= 0 ? x[b, src0[j]] : fill[j]) + (src1[j] >= 0 ? x[b, src1[j]] : 0).
   out: optional caller-owned fp32 [B, len(src0)] buffer."""
-  dev = x.device
-  x2 = x.to(tc.float32).reshape(-1, x.shape[-1]).contiguous()
-  if out is None:
-    out = tc.empty((x2.shape[0], src0.shape[0]), dtype=tc.float32, device=dev)
-  with tc.cuda.device(dev):
-    check(lib().polar_rate_recover_f32(ptr(x2), ptr(src0), ptr(src1), ptr(fill), x2.shape[1], src0.shape[0], x2.shape[0],
-                                       ptr(out), stream_ptr(dev)))
+  x2 = _rows(x)
+  out = _out(x.device, (x2.shape[0], src0.shape[0]), tc.float32, given=out)
+  _call(x.device, "polar_rate_recover_f32", ptr(x2), ptr(src0), ptr(src1), ptr(fill), x2.shape[1], src0.shape[0],
+        x2.shape[0], ptr(out))
   return out
-
-
-def mc_control(delta, state, target_bit_errs, target_block_errs, max_mc_iter):
-  """polar_mc_control: fold `delta` (int64[4]) into `state` (int64[8]) and evaluate sim_ber's stop rules on the device."""
-  dev = state.device
-  tb = -1 if target_bit_errs is None else int(target_bit_errs)
-  tk = -1 if target_block_errs is None else int(target_block_errs)
-  with tc.cuda.device(dev):
-    check(lib().polar_mc_control(ptr(delta), ptr(state), tb, tk, int(max_mc_iter), stream_ptr(dev)))
 
 
 MC_GROUP_MAX = 32
@@ -537,23 +548,10 @@ MC_GROUP_MAX = 32
 def mc_control_group(delta, item_points, state, sweep, expect_q, target_bit_errs, target_block_errs, max_mc_iter, early_stop):
   """polar_mc_control_group: fold the counters delta [G,4] of a group of queued iterations (SNR point of iteration j =
   item_points[j]) into the per-point states [P,8] and the sweep cursor [8], with sim_ber's stop rules, on the device."""
-  dev = state.device
-  tb = -1 if target_bit_errs is None else int(target_bit_errs)
-  tk = -1 if target_block_errs is None else int(target_block_errs)
   pts = (ctypes.c_int32 * len(item_points))(*[int(p) for p in item_points])
-  with tc.cuda.device(dev):
-    check(lib().polar_mc_control_group(ptr(delta), ctypes.cast(pts, ctypes.c_void_p), len(item_points), ptr(state), state.shape[0],
-                                       ptr(sweep), int(expect_q), tb, tk, int(max_mc_iter), 1 if early_stop else 0, stream_ptr(dev)))
-
-
-def pack_rows(m):
-  """0/1 matrix [r, n] (numpy) -> uint32 bit-packed rows [r, (n+31)//32], position i = bit i%32 of word i//32 (as int32)."""
-  m = (np.asarray(m) != 0).astype(np.uint8)
-  r, n = m.shape
-  nw = (n + 31) // 32
-  pad = np.zeros((r, nw * 32), dtype=np.uint8)
-  pad[:, :n] = m
-  return np.packbits(pad.reshape(r, nw, 32), axis=2, bitorder="little").view(np.uint32).reshape(r, nw).view(np.int32).copy()
+  _call(state.device, "polar_mc_control_group", ptr(delta), ctypes.cast(pts, ctypes.c_void_p), len(item_points), ptr(state),
+        state.shape[0], ptr(sweep), int(expect_q), _stop_target(target_bit_errs), _stop_target(target_block_errs), int(max_mc_iter),
+        1 if early_stop else 0)
 
 
 def osd_decode(logits, gm_rows, n, k, t, want_f32=True, want_packed=False, want_dist=False):
@@ -561,13 +559,10 @@ def osd_decode(logits, gm_rows, n, k, t, want_f32=True, want_packed=False, want_
   dev = gm_rows.device
   x = _prep_logits(logits, n, dev)
   B = x.shape[0]
-  nw = (n + 31) // 32
-  out = {"c": tc.empty((B, n), dtype=tc.float32, device=dev) if want_f32 else None,
-         "c_packed": tc.empty((B, nw), dtype=tc.int32, device=dev) if want_packed else None,
-         "dist": tc.empty((B,), dtype=tc.float32, device=dev) if want_dist else None}
-  with tc.cuda.device(dev):
-    check(lib().polar_osd_decode(ptr(x), ptr(gm_rows), n, k, int(t), B, ptr(out["c_packed"]), ptr(out["c"]), ptr(out["dist"]),
-                                 stream_ptr(dev)))
+  out = {"c": _out(dev, (B, n), tc.float32, want_f32),
+         "c_packed": _out(dev, (B, (n + 31) // 32), tc.int32, want_packed),
+         "dist": _out(dev, (B,), tc.float32, want_dist)}
+  _call(dev, "polar_osd_decode", ptr(x), ptr(gm_rows), n, k, int(t), B, ptr(out["c_packed"]), ptr(out["c"]), ptr(out["dist"]))
   return out
 
 

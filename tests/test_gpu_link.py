@@ -304,7 +304,7 @@ def test_full_size_properties_sc():
 
 @pytest.mark.parametrize("dec_kind", ["sc", "scl4", "scl8_crc"])
 def test_on_device_monte_carlo_loop_equals_host_loop(dec_kind):
-    """SURVEY 8(f) N1: sim_ber_device (stop rules evaluated by polar_mc_control on the GPU, one iteration queued ahead)
+    """SURVEY 8(f) N1: sim_ber_device (stop rules evaluated by polar_mc_control_group on the GPU, iterations queued ahead)
     must reproduce the host loop counter for counter -- same seed, same number of counted iterations, same status."""
     torch, dk, po, co, dev = _env()
     from polar.enc import PolarEncoder
@@ -381,7 +381,7 @@ def test_device_loop_lookahead_and_bec_model():
 
 
 def test_on_device_loop_with_process_group_of_one():
-    """The sharded path (stream-ordered NCCL all-reduce of the 4 counters before polar_mc_control) with world size 1."""
+    """The sharded path (stream-ordered NCCL all-reduce of the counters before polar_mc_control_group) with world size 1."""
     torch, dk, po, co, dev = _env()
     import torch.distributed as dist
     from polar.enc import PolarEncoder
