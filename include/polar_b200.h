@@ -153,6 +153,25 @@ int polar_scl_decode_hybrid(const float *d_logit, const uint32_t *d_frozen_mask,
                             const uint32_t *d_crc_rows, int crc_len, int cn_mode, int32_t *d_n_list_out,
                             void *d_workspace, size_t workspace_bytes, void *stream);
 
+/* ---- belief-propagation decoder (Sionna's PolarBPDecoder; dec_type="BP" of Polar5GDecoder) ------------------------
+ * num_iter iterations of flooding BP on the encoder's factor graph in natural order (csrc/polar_belief.cu states the
+ * schedule), f of the SC decoder of the same arithmetic, fp32 sums, no early stop.  The only decoder here with soft
+ * information bits.  Output in the logit convention: soft = -(L0[i] + R0[i]) at the information positions, hard bit
+ * = [soft > 0] (sim.hard_decisions of the soft output; SC's leaf rule differs only at an exact 0).
+ *  cn_mode          0: min-sum f (polar_sc_decode_f32's), 1: exact boxplus f (polar_sc_decode_boxplus_f32's)
+ *  d_logit          [B, n] fp32, finite, 16-byte aligned rows for n >= 4 (POLAR_EALIGN)
+ *  d_u_packed       [B, POLAR_WORDS(n)] hard decisions of all n positions, frozen = 0; may be NULL
+ *  d_u_info_f32     [B, k] fp32 0./1. at ascending d_info_pos; may be NULL
+ *  d_llr_info_f32   [B, k] fp32 soft output at ascending d_info_pos; may be NULL (not all three outputs)
+ *  d_info_pos       [k] int32, required when a [B, k] output is given
+ *  n power of two, 2 <= n <= POLAR_BP_MAX_N; num_iter >= 1.  POLAR_EINVAL (checked before any CUDA call) for bad n,
+ *  num_iter, cn_mode, B < 0 or pointers.  B == 0 launches nothing.  One launch, no workspace, no allocation, no
+ *  synchronisation. */
+#define POLAR_BP_MAX_N 1024
+int polar_belief_decode_f32(const float *d_logit, const uint32_t *d_frozen_mask, int n, int64_t B, int num_iter,
+                            int cn_mode, uint32_t *d_u_packed, float *d_u_info_f32, float *d_llr_info_f32,
+                            const int32_t *d_info_pos, int k, void *stream);
+
 /* ---- encoder-----------------------------------------------------------------------------
  * polar_encode_packed: x = u.G over GF(2) on bit-packed rows (XOR butterfly; the transform of
  * my_sn/fec/polar/enc.py:85-96 == (c @ G) % 2 of x_run_sn_polar/polar/enc.py:42).

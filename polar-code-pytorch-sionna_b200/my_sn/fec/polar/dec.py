@@ -4,7 +4,8 @@ SC / SCL decoders (dec.py:13-157 / :158-537, SURVEY 8f row N2).  `use_fast_scl=T
 with the reference's rate-0 / REP node shortcuts (dec.py:269-306, 354-376: node-level path-metric updates, the subtree
 is not descended into).  `use_hybrid_sc=True` (dec.py:437-470) decodes every codeword with SC first and list-decodes only
 those whose SC decision fails the CRC (`polar_scl_decode_hybrid`: SC, a CRC check / compaction kernel and the list kernel
-over the failing rows, all on the device)."""
+over the failing rows, all on the device).  `BP_Dec` is the belief-propagation decoder of Sionna's `PolarBPDecoder`
+(`polar_belief_decode_f32`), the only decoder here that can return soft information bits."""
 import numpy as np
 import torch as tc
 from torch import nn
@@ -48,6 +49,71 @@ class SC_Dec(nn.Module):
     out = u_hat.reshape(output_shape).to(dtype=self.output_dtype)
     return out if inputs.is_cuda else out.to(inputs.device)
 
+
+class BP_Dec(nn.Module):
+  """Belief-propagation decoder (Sionna's PolarBPDecoder(frozen_pos, n, num_iter, hard_out)): `num_iter` flooding
+  iterations on the encoder's factor graph, no early stop (the schedule is stated in csrc/polar_belief.cu).
+  cn_type="boxplus" (default): the exact boxplus f of the Sionna-style SC_Dec; cn_type="minsum": the min-sum f of the
+  x_run SC_Dec.  hard_out=True returns the 0./1. information bits, hard_out=False their soft estimates as logits
+  (ln P(1)/P(0), the decoder input's convention), so that `sim.hard_decisions(soft)` equals the hard output.
+  n is a power of two in [2, 1024].  Runs `polar_belief_decode_f32` for CPU and CUDA tensors alike."""
+
+  def __init__(self, frozen_pos, n, num_iter=20, hard_out=True, output_dtype=tc.float32, device='cpu', cn_type="boxplus"):
+    super().__init__()
+    if output_dtype not in (tc.float16, tc.float32, tc.float64):
+      raise ValueError('output_dtype must be {tf.float16, tf.float32, tf.float64}.')
+    assert cn_type in ("boxplus", "minsum"), "cn_type must be 'boxplus' or 'minsum'."
+    assert isinstance(hard_out, bool), "hard_out must be bool."
+    assert isinstance(num_iter, (int, np.integer)) and not isinstance(num_iter, bool) and num_iter >= 1, \
+      "num_iter must be a positive integer."
+    n = int(n)
+    assert len(frozen_pos) <= n, "Num. of elements in frozen_pos cannot be greater than n."
+    assert n >= 2 and np.log2(n) == int(np.log2(n)), "n must be a power of 2."
+    assert n <= dk.BP_MAX_N, "n must not exceed %d." % dk.BP_MAX_N
+    self.output_dtype = output_dtype
+    self.device = device
+    self._n = n
+    self._frozen_pos = frozen_pos
+    self._k = self._n - len(self._frozen_pos)
+    self._info_pos = np.setdiff1d(np.arange(self._n), dk.to_numpy_pos(frozen_pos))
+    assert self._k == len(self._info_pos), "Internal error: invalid info_pos generated."
+    self._num_iter = int(num_iter)
+    self._hard_out = hard_out
+    self._boxplus = cn_type == "boxplus"
+    self._llr_max = 30.
+
+  @property
+  def n(self): return self._n
+  @property
+  def k(self): return self._k
+  @property
+  def frozen_pos(self): return self._frozen_pos
+  @property
+  def info_pos(self): return self._info_pos
+  @property
+  def num_iter(self): return self._num_iter
+  @property
+  def hard_out(self): return self._hard_out
+  @property
+  def llr_max(self): return self._llr_max
+
+  def decode_packed(self, logits, tables, out=None):
+    """Device fast path of the on-device Monte-Carlo loop: bit-packed hard decisions of all n positions, frozen = 0."""
+    return dk.belief_decode(logits, tables, self._num_iter, self._boxplus, want_info=False, want_packed=True,
+                            out_packed=out)["u_packed"]
+
+  def forward(self, inputs):
+    assert inputs.shape[-1] == self._n, "Last input dimension must be of length n."
+    assert inputs.dim() > 1
+    dev = inputs.device if inputs.is_cuda else dk.cuda_device(self.device)
+    tables = dk.code_tables(self._frozen_pos, self._n, dev)
+    res = dk.belief_decode(inputs, tables, self._num_iter, self._boxplus, want_info=self._hard_out,
+                           want_soft=not self._hard_out)
+    output_shape = list(inputs.shape)
+    output_shape[-1] = self._k
+    output_shape[0] = -1
+    out = res["u_info" if self._hard_out else "soft"].reshape(output_shape).to(dtype=self.output_dtype)
+    return out if inputs.is_cuda else out.to(inputs.device)
 
 
 class SCL_Dec(nn.Module):
@@ -170,12 +236,13 @@ class Polar5GDecoder(nn.Module):
   """Rate recovery + polar decoding + CRC removal for codewords of `Polar5GEncoder` (my_sn/fec/polar/dec.py:539-667,
   SURVEY 8f row N3).  Channel de-interleaver, de-puncturing (logit 0), de-shortening (logit -100), repetition combining
   and the sub-block de-interleaver are folded into one index plan applied by `polar_rate_recover_f32`; the decoder is the
-  my_sn `SC_Dec` (boxplus SC) or the CRC-aided `SCL_Dec`.  `dec_type="hybSCL"` runs that `SCL_Dec` with
-  `use_hybrid_sc=True`: SC first, list decoding only of the codewords whose SC decision fails the CRC.
+  my_sn `SC_Dec` (boxplus SC), the CRC-aided `SCL_Dec` or `BP_Dec` (boxplus BP, `num_iter` iterations, hard output).
+  `dec_type="hybSCL"` runs that `SCL_Dec` with `use_hybrid_sc=True`: SC first, list decoding only of the codewords whose
+  SC decision fails the CRC.
   `return_crc_status=True` works here (the reference stops in a stray breakpoint, dec.py:661).  `decode_packed` (rate
   recovery, then the inner decoder's packed path) lets `sim_ber` run a 5G link model on the on-device loop."""
 
-  def __init__(self, enc_polar, dec_type="SC", list_size=8, return_crc_status=False, output_dtype=tc.float32):
+  def __init__(self, enc_polar, dec_type="SC", list_size=8, return_crc_status=False, output_dtype=tc.float32, num_iter=20):
     super().__init__()
     self._output_dtype = output_dtype
     self._n_target = enc_polar.n_target; self._k_target = enc_polar.k_target
@@ -192,6 +259,9 @@ class Polar5GDecoder(nn.Module):
     elif dec_type in ("SCL", "hybSCL"):
       self._polar_dec = SCL_Dec(enc_polar._frozen_pos, self._n_polar, crc_degree=enc_polar.enc_crc.crc_degree,
                                 list_size=list_size, use_hybrid_sc=dec_type == "hybSCL", device=enc_polar.device)
+    elif dec_type == "BP":
+      self._polar_dec = BP_Dec(enc_polar._frozen_pos, self._n_polar, num_iter=num_iter, hard_out=True,
+                               device=enc_polar.device)
     else:
       raise ValueError("Unknown value for dec_type.")
     assert isinstance(return_crc_status, bool), "return_crc_status must be bool."
@@ -230,7 +300,7 @@ class Polar5GDecoder(nn.Module):
 
   def decode_packed(self, logits, tables, out=None):
     """Device fast path of the on-device Monte-Carlo loop: channel logits [B, n_target] -> rate recovery into a
-    per-device buffer (grown, never shrunk) -> the inner decoder's `decode_packed` (SC, SCL or hybrid SCL) with the
+    per-device buffer (grown, never shrunk) -> the inner decoder's `decode_packed` (SC, SCL, hybrid SCL or BP) with the
     mother code's `tables`.  Returns the bit-packed decisions [B, words(n_polar)] over all n_polar positions."""
     dev = tables.dev
     x = logits.reshape(-1, self._n_target)

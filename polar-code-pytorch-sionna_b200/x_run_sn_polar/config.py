@@ -21,6 +21,7 @@ class PolarConfig:
   snr_end: float = 5
   mc_iter: int = 10
   list_size: int = 8   # scl list size
+  bp_iter: int = 20    # belief-propagation iterations of the `bp` curve
   mode: str = "max"
   spec: bool = False
   seed: int = 42       # main.py:24 (module-level constant in the reference)

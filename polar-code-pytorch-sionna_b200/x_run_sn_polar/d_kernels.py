@@ -39,7 +39,7 @@ LIB_PATH = os.environ.get("POLAR_B200_LIB", os.path.join(_PKG_DIR, "libpolar_b20
 _lib = None
 
 POLAR_OK, POLAR_EINVAL, POLAR_EALIGN, POLAR_ENOMEM, POLAR_ECUDA = 0, -1, -2, -3, -4
-SC_MAX_N, SCL_MAX_N, SCL_MAX_L = 8192, 4096, 32
+SC_MAX_N, SCL_MAX_N, SCL_MAX_L, BP_MAX_N = 8192, 4096, 32, 1024
 
 _vp, _i32, _i64, _u64, _f32, _sz = (ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_uint64,
                                     ctypes.c_float, ctypes.c_size_t)
@@ -60,6 +60,7 @@ _SIGNATURES = {
   "polar_scl_decode_boxplus_pruned": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _sz, _vp]),
   "polar_scl_hybrid_workspace_bytes": (_sz, [_i32, _i32, _i64, _i32]),
   "polar_scl_decode_hybrid": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _i32, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
+  "polar_belief_decode_f32": (_i32, [_vp, _vp, _i32, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp]),
   "polar_encode_packed": (_i32, [_vp, _i32, _i64, _vp, _vp]),
   "polar_encode_f32": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp]),
   "polar_gather_cols_f32": (_i32, [_vp, _vp, _i32, _i32, _i64, _vp, _vp]),
@@ -383,6 +384,21 @@ def scl_decode_hybrid(logits, tables, list_size, crc_rows, crc_len, cn_mode, wan
   _call(dev, "polar_scl_decode_hybrid", ptr(x), ptr(tables.frozen_mask), n, L, B, ptr(out["u_packed"]), ptr(out["u_info"]),
         ptr(tables.info_pos), tables.k, ptr(crc_rows), int(crc_len), int(cn_mode), ptr(n_list_out),
         workspace=("polar_scl_hybrid_workspace_bytes", (n, L, B, int(cn_mode))))
+  return out
+
+
+def belief_decode(logits, tables, num_iter, boxplus, want_info=True, want_soft=False, want_packed=False, out_packed=None):
+  """polar_belief_decode_f32: `num_iter` iterations of belief propagation with the min-sum or the exact boxplus f.
+  -> dict(u_info fp32 [B,k] 0./1. | None, soft fp32 [B,k] logits at info_pos | None, u_packed int32 [B,words] | None).
+  out_packed: caller-owned int32 [B, words(n)] buffer for the packed decisions (Monte-Carlo loop: no allocation per call)."""
+  dev = tables.dev
+  x = _prep_logits(logits, tables.n, dev)
+  B = x.shape[0]
+  out = {"u_info": _out(dev, (B, tables.k), tc.float32, want_info),
+         "soft": _out(dev, (B, tables.k), tc.float32, want_soft),
+         "u_packed": _out(dev, (B, words(tables.n)), tc.int32, want_packed, out_packed)}
+  _call(dev, "polar_belief_decode_f32", ptr(x), ptr(tables.frozen_mask), tables.n, B, int(num_iter), 1 if boxplus else 0,
+        ptr(out["u_packed"]), ptr(out["u_info"]), ptr(out["soft"]), ptr(tables.info_pos), tables.k)
   return out
 
 

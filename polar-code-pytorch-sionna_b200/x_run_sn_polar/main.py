@@ -1,5 +1,6 @@
-"""CLI of the experiment (mirrors x_run_sn_polar/main.py:25-78): SC (always) and SCL BLER curves over
-Eb/N0 = 0:0.5:snr_end for an RM-rule polar code, on the GPU.
+"""CLI of the experiment (mirrors x_run_sn_polar/main.py:25-78): SC (always), SCL and belief-propagation BLER curves over
+Eb/N0 = 0:0.5:snr_end for an RM-rule polar code, on the GPU.  `--algos [scl,bp]` picks the extra curves; `bp` adds
+`BP-<bp_iter>` (boxplus BP, my_sn BP_Dec).
 
   python x_run_sn_polar/main.py --k 32 --n 64 --algos [scl] --bs 100 --mc_iter 1      (README command)
   torchrun --nproc-per-node 8 x_run_sn_polar/main.py ...   shards every batch over the ranks (bs is per rank)
@@ -19,6 +20,7 @@ from my_sn.plotting import PlotBER
 from polar.enc import PolarEncoder as PolarEnc2
 from polar.polar_scl import SCL_Dec
 from polar.polar_sc import SC_Dec
+from my_sn.fec.polar.dec import BP_Dec
 from config import PolarConfig, device
 from z_sys_model.awgn_model import System_AWGN_model
 from d_kernels import *  # noqa: F401,F403  F2, F4.., gen_arikan (main.py:30)
@@ -38,6 +40,7 @@ def gen_code(c, Gn, name, mode='sc'):
   enc = PolarEnc2(frozen_pos, c.n, G_, device=device)
   if mode == "sc": dec = SC_Dec(frozen_pos, c.n, device=device)
   elif mode == "scl": dec = SCL_Dec(frozen_pos, c.n, c.list_size, device=device)
+  elif mode == "bp": dec = BP_Dec(frozen_pos, c.n, num_iter=c.bp_iter, device=device)
   else: raise Exception('error...')
   return [System_AWGN_model(c.n, c.k, enc, dec, device=device), name]
 
@@ -71,6 +74,8 @@ def main(c: PolarConfig):
   codes_under_test = [gen_code(c, F2, "SC", mode="sc")]
   if 'scl' in c.algos:
     codes_under_test.append(gen_code(c, F2, f"SCL-{c.list_size}", mode="scl"))
+  if 'bp' in c.algos:
+    codes_under_test.append(gen_code(c, F2, f"BP-{c.bp_iter}", mode="bp"))
   ber_plot = PlotBER(f"Performance of Short Len Codes (k={k}, n={n})")
   for code in codes_under_test:
     if rank == 0: print("\nRunning: " + code[-1])
