@@ -73,8 +73,9 @@ int polar_sc_decode_f32(const float *d_logit, const uint32_t *d_frozen_mask, int
 
 /* Same call, exact-boxplus check-node update f = ln(1+e^(x+y)) - ln(e^x+e^y) (inputs clipped to +-30, fp32) instead
  * of min-sum: the arithmetic of the Sionna-style SC_Dec in my_sn/fec/polar/dec.py:13-157 (SURVEY 8f row N2).  Same
- * kernels compiled a second time (csrc/polar_bp_wrap.cu).  Parity with the CPU reference is statistical for this
- * mode: its exp/log come from the host libm and the boxplus difference cancels to rounding noise near ties. */
+ * kernels compiled a second time into namespace polar_bp (csrc/polar_bp_wrap.cu) behind the same entry code
+ * (csrc/polar_sc_api.cu).  Parity with the CPU reference is statistical for this mode: its exp/log come from the host
+ * libm and the boxplus difference cancels to rounding noise near ties. */
 int polar_sc_decode_boxplus_f32(const float *d_logit, const uint32_t *d_frozen_mask, int n, int64_t B,
                                 uint32_t *d_u_packed, float *d_u_info_f32, const int32_t *d_info_pos, int k,
                                 void *stream);

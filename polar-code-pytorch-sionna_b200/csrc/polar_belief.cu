@@ -1,7 +1,7 @@
 // polar_belief.cu -- belief-propagation (BP) polar decoder with soft output and a fixed number of iterations
 // (Sionna's PolarBPDecoder, dec_type="BP" of its Polar5GDecoder).  Compiled twice: with the min-sum f into namespace
-// polar (launch_belief) and, through polar_bp_wrap.cu, with the exact boxplus f into namespace polar_bp
-// (launch_belief_boxplus).  The C entry point is polar_belief_decode_f32 (polar_belief_api.cu).
+// polar (polar::launch_belief) and, through polar_bp_wrap.cu, with the exact boxplus f into namespace polar_bp
+// (polar_bp::launch_belief).  The C entry point is polar_belief_decode_f32 (polar_belief_api.cu).
 //
 // Factor graph: the encoder's butterfly (polar_enc.cu) in natural order, columns 0 (u side) .. m (channel side).  Stage
 // s joins columns s and s+1 through the processing elements (PEs) (i, j = i + 2^s), one for every i with bit s clear.
@@ -24,6 +24,7 @@
 // boundary is a CTA barrier.
 #include "polar_common.cuh"
 #include "polar_internal.h"
+#include "polar_launch.h"
 #include "polar_belief.h"
 
 namespace polar {
@@ -126,10 +127,7 @@ __global__ void __launch_bounds__(kBeliefMaxThreads) belief_kernel(const BeliefP
 
 }  // namespace
 
-}  // namespace polar
-
-int launch_belief(const polar::BeliefParams &P, cudaStream_t st) {
-  using namespace polar;
+int launch_belief(const BeliefParams &P, cudaStream_t st) {
   const int m = ilog2(P.n), half = P.n / 2;
   const int threads = half > 256 ? half : 256;
   const int cpb = threads / half;
@@ -137,8 +135,7 @@ int launch_belief(const polar::BeliefParams &P, cudaStream_t st) {
   int64_t grid = (P.B + cpb - 1) / cpb;
   if (grid > ((int64_t)1 << 30)) grid = (int64_t)1 << 30;                        // the kernel loops over the rest
   POLAR_CUDA(cudaFuncSetAttribute(belief_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  belief_kernel<<<(unsigned)grid, threads, smem, st>>>(P);
-  count_launch();
-  POLAR_CHECK_LAUNCH("belief_kernel");
-  return POLAR_OK;
+  return launch("belief_kernel", belief_kernel, (unsigned)grid, threads, smem, st, P);
 }
+
+}  // namespace polar

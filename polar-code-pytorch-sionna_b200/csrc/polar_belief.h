@@ -3,7 +3,7 @@
 //
 // polar_belief.cu is compiled twice (min-sum into namespace polar, exact boxplus into namespace polar_bp through
 // polar_bp_wrap.cu).  polar_bp_wrap.cu includes this header before it renames the namespace, so both builds share the
-// parameter type; the boxplus launcher is renamed launch_belief_boxplus.
+// parameter type and define the launcher declared here in both namespaces.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -15,8 +15,11 @@ struct BeliefParams {
   uint32_t *u_packed; float *u_info; float *llr_info; const int32_t *info_pos; int k;   // any output may be null
 };
 
+// polar_belief.cu: belief_kernel over P, with the min-sum f here and the exact boxplus f in polar_bp
+int launch_belief(const BeliefParams &P, cudaStream_t st);
+
 }  // namespace polar
 
-// polar_belief.cu: belief_kernel over P, with the min-sum f and with the exact boxplus f
+namespace polar_bp {
 int launch_belief(const polar::BeliefParams &P, cudaStream_t st);
-int launch_belief_boxplus(const polar::BeliefParams &P, cudaStream_t st);
+}

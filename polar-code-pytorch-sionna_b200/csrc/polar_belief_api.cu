@@ -1,7 +1,7 @@
 // polar_belief_api.cu -- the C entry point of the belief-propagation decoder (include/polar_b200.h,
 // polar_belief_decode_f32): argument check, then the kernel of the chosen arithmetic (polar_belief.cu: launch_belief,
-// and launch_belief_boxplus from the same source compiled through polar_bp_wrap.cu).
-#include "polar_internal.h"
+// in namespace polar with min-sum and in namespace polar_bp, compiled through polar_bp_wrap.cu, with exact boxplus).
+#include "polar_launch.h"
 #include "polar_belief.h"
 
 using namespace polar;
@@ -9,7 +9,7 @@ using namespace polar;
 extern "C" int polar_belief_decode_f32(const float *d_logit, const uint32_t *d_frozen_mask, int n, int64_t B, int num_iter,
                                        int cn_mode, uint32_t *d_u_packed, float *d_u_info_f32, float *d_llr_info_f32,
                                        const int32_t *d_info_pos, int k, void *stream) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_BP_MAX_N) return set_error(POLAR_EINVAL, "belief: n=%d must be a power of two in [2,%d]", n, POLAR_BP_MAX_N);
+  if (const int rc = check_pow2_n("belief", n, 2, POLAR_BP_MAX_N)) return rc;
   if (num_iter < 1) return set_error(POLAR_EINVAL, "belief: num_iter=%d must be >= 1", num_iter);
   if (cn_mode != 0 && cn_mode != 1) return set_error(POLAR_EINVAL, "belief: cn_mode=%d must be 0 (min-sum) or 1 (boxplus)", cn_mode);
   if (B < 0) return set_error(POLAR_EINVAL, "belief: B=%lld < 0", (long long)B);
@@ -23,5 +23,5 @@ extern "C" int polar_belief_decode_f32(const float *d_logit, const uint32_t *d_f
   P.logit = d_logit; P.fmask = d_frozen_mask; P.n = n; P.B = B; P.iters = num_iter;
   P.u_packed = d_u_packed; P.u_info = d_u_info_f32; P.llr_info = d_llr_info_f32; P.info_pos = d_info_pos; P.k = k;
   const cudaStream_t st = (cudaStream_t)stream;
-  return cn_mode == 0 ? launch_belief(P, st) : launch_belief_boxplus(P, st);
+  return (Arith)cn_mode == Arith::minsum ? launch_belief(P, st) : polar_bp::launch_belief(P, st);
 }

@@ -1,23 +1,20 @@
-// polar_bp_wrap.cu -- compiles one SC translation unit a second time with the exact-boxplus f
-// (my_sn/fec/polar/dec.py:33-46) instead of min-sum: every kernel, launcher and device symbol of the unit lands
-// in namespace polar_bp; the SC C entry point is renamed polar_sc_decode_boxplus_f32 (SURVEY 8f row N2), the list
-// kernel's launcher launch_scl2_boxplus and the belief-propagation kernel's launcher launch_belief_boxplus.
+// polar_bp_wrap.cu -- compiles one decoder translation unit a second time with the exact-boxplus f
+// (my_sn/fec/polar/dec.py:33-46) instead of min-sum (SURVEY 8f row N2): every kernel, launcher and device symbol of the
+// unit lands in namespace polar_bp, so the boxplus launchers are the min-sum ones' namesakes, polar_bp::launch_sc4,
+// polar_bp::launch_scl2, polar_bp::launch_belief and so on.
 //   nvcc ... -DPOLAR_BP_SRC=\"polar_sc4.cu\" -c polar_bp_wrap.cu -o polar_sc4_bp.o
+// Every internal header (*.h) that a unit compiled here includes must be included below, before `polar` is renamed:
+// otherwise its #pragma once declarations land in namespace polar_bp.  The device headers (*.cuh) are left to the unit,
+// so that they are compiled with the boxplus f.
 #include "polar_internal.h"      // host plumbing stays in ::polar (set_error, env_int, device queries ...)
-#include "polar_scl.h"           // so do the list decoder's parameter and plan types
-#include "polar_belief.h"        // and the belief-propagation decoder's parameters
+#include "polar_launch.h"        // so do the launch helpers and the Arith enum
+#include "polar_sc.h"            // and the declarations of the launchers in both namespaces
+#include "polar_scl.h"
+#include "polar_belief.h"
 namespace polar_bp { using namespace polar; }
 #define POLAR_F_BOXPLUS 1
 #define polar polar_bp
-#define polar_sc_decode_f32 polar_sc_decode_boxplus_f32
+// the debug hooks are extern "C", outside any namespace: a second copy needs its own name
 #define polar_sc4_debug_read polar_sc4_bp_debug_read
 #define polar_sc5_debug_read polar_sc5_bp_debug_read
-#define launch_scl2 launch_scl2_boxplus
-#define launch_belief launch_belief_boxplus
-namespace polar {                // the launchers the units call across files, redeclared in the boxplus namespace
-int launch_sc5(const float *logit, const uint32_t *fmask, int n, int64_t B, uint32_t *u_packed, float *u_info,
-               const int32_t *info_pos, int k, int warps, cudaStream_t st);
-int launch_sc4(const float *logit, const uint32_t *fmask, int n, int64_t B, uint32_t *u_packed, float *u_info,
-               const int32_t *info_pos, int k, int warps, cudaStream_t st);
-}
 #include POLAR_BP_SRC

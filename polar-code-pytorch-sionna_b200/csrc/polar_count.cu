@@ -2,7 +2,7 @@
 // Replaces count_errors / count_block_errors (my_sn/sim.py:7-18): sum(b != b_hat) and
 // sum(any(b != b_hat, -1)).  Popcount over packed words (or a compare over the fp32 API tensors),
 // per-warp accumulation in registers, one atomicAdd pair per warp at the end.
-#include "polar_internal.h"
+#include "polar_launch.h"
 
 namespace polar {
 
@@ -151,19 +151,8 @@ extern "C" int polar_mc_control_group(unsigned long long *d_delta, const int32_t
   if (max_mc_iter < 1 || n_points < 1) return set_error(POLAR_EINVAL, "mc_control_group: max_mc_iter < 1 or n_points < 1");
   McItems it;
   for (int j = 0; j < kMcGroupMax; ++j) it.point[j] = j < n_items ? h_item_point[j] : -1;
-  mc_control_group_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(d_delta, it, n_items, d_state, d_sweep8, expect_q, n_points,
-                                                              target_bit_errs, target_block_errs, max_mc_iter, early_stop);
-  count_launch();
-  POLAR_CHECK_LAUNCH("mc_control_group");
-  return POLAR_OK;
-}
-
-static unsigned cnt_grid(int64_t rows) {
-  int64_t g = (rows + 7) / 8;
-  const int64_t cap = (int64_t)device_sm_count() * 8;
-  if (g > cap) g = cap;
-  if (g < 1) g = 1;
-  return (unsigned)g;
+  return launch("mc_control_group", mc_control_group_kernel, 1, 32, 0, (cudaStream_t)stream, d_delta, it, n_items, d_state,
+                d_sweep8, expect_q, n_points, target_bit_errs, target_block_errs, max_mc_iter, early_stop);
 }
 
 extern "C" int polar_count_errors_packed(const uint32_t *d_a, const uint32_t *d_b, const uint32_t *d_mask, int n,
@@ -173,28 +162,16 @@ extern "C" int polar_count_errors_packed(const uint32_t *d_a, const uint32_t *d_
   if (!d_a || !d_b || !d_counters) return set_error(POLAR_EINVAL, "count: null pointer");
   const int nw = POLAR_WORDS(n);
   const bool vec = nw >= 4 && nw <= 128 && ((((uintptr_t)d_a | (uintptr_t)d_b | (uintptr_t)d_mask) & 15) == 0) && B * (int64_t)nw < ((int64_t)1 << 36);
+  const cudaStream_t st = (cudaStream_t)stream;
   if (vec) {
     const int64_t pieces = B * (int64_t)(nw / 4);
-    int64_t g = (pieces + 255) / 256;
-    const int64_t cap = (int64_t)device_sm_count() * 8;
-    if (g > cap) g = cap;
-    if (g < 1) g = 1;
-    const uint4 *pa = reinterpret_cast<const uint4 *>(d_a), *pb = reinterpret_cast<const uint4 *>(d_b), *pm = reinterpret_cast<const uint4 *>(d_mask);
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (nw / 4) {
-      case 1: count_packed_vec_kernel<1><<<(unsigned)g, 256, 0, st>>>(pa, pb, pm, pieces, d_counters); break;
-      case 2: count_packed_vec_kernel<2><<<(unsigned)g, 256, 0, st>>>(pa, pb, pm, pieces, d_counters); break;
-      case 4: count_packed_vec_kernel<4><<<(unsigned)g, 256, 0, st>>>(pa, pb, pm, pieces, d_counters); break;
-      case 8: count_packed_vec_kernel<8><<<(unsigned)g, 256, 0, st>>>(pa, pb, pm, pieces, d_counters); break;
-      case 16: count_packed_vec_kernel<16><<<(unsigned)g, 256, 0, st>>>(pa, pb, pm, pieces, d_counters); break;
-      default: count_packed_vec_kernel<32><<<(unsigned)g, 256, 0, st>>>(pa, pb, pm, pieces, d_counters); break;
-    }
-  } else {
-    count_packed_kernel<<<cnt_grid(B), 256, 0, (cudaStream_t)stream>>>(d_a, d_b, d_mask, nw, B, d_counters);
+    const int q = nw / 4;
+    const auto kern = q == 1 ? count_packed_vec_kernel<1> : q == 2 ? count_packed_vec_kernel<2> : q == 4 ? count_packed_vec_kernel<4>
+                      : q == 8 ? count_packed_vec_kernel<8> : q == 16 ? count_packed_vec_kernel<16> : count_packed_vec_kernel<32>;
+    return launch("count_packed", kern, grid_for(pieces, 256, 8), 256, 0, st, reinterpret_cast<const uint4 *>(d_a),
+                  reinterpret_cast<const uint4 *>(d_b), reinterpret_cast<const uint4 *>(d_mask), pieces, d_counters);
   }
-  count_launch();
-  POLAR_CHECK_LAUNCH("count_packed");
-  return POLAR_OK;
+  return launch("count_packed", count_packed_kernel, grid_for(B, 8, 8), 256, 0, st, d_a, d_b, d_mask, nw, B, d_counters);
 }
 
 extern "C" int polar_count_errors_f32(const float *d_b, const float *d_b_hat, int k, int64_t B,
@@ -202,8 +179,5 @@ extern "C" int polar_count_errors_f32(const float *d_b, const float *d_b_hat, in
   if (k < 1 || B < 0) return set_error(POLAR_EINVAL, "count: bad k/B");
   if (B == 0) return POLAR_OK;
   if (!d_b || !d_b_hat || !d_counters) return set_error(POLAR_EINVAL, "count: null pointer");
-  count_f32_kernel<<<cnt_grid(B), 256, 0, (cudaStream_t)stream>>>(d_b, d_b_hat, k, B, d_counters);
-  count_launch();
-  POLAR_CHECK_LAUNCH("count_f32");
-  return POLAR_OK;
+  return launch("count_f32", count_f32_kernel, grid_for(B, 8, 8), 256, 0, (cudaStream_t)stream, d_b, d_b_hat, k, B, d_counters);
 }

@@ -4,7 +4,7 @@
 // my_sn/fec/polar/enc.py:85-113 (gather/xor stages).  c_j = XOR_{i superset j} u_i.
 // One warp per codeword, 32 positions per lane-word; stages below 32 are in-register shifts,
 // stages 32..1023 are __shfl_xor, stages above are register-to-register.  HBM-bound.
-#include "polar_internal.h"
+#include "polar_launch.h"
 #include "polar_warp.cuh"
 
 namespace polar {
@@ -157,20 +157,12 @@ __global__ void __launch_bounds__(256) unpack_info_kernel(const uint32_t *__rest
   }
 }
 
-static unsigned grid_for(int64_t work_items, int per_block, int max_ctas_per_sm = 8) {
-  int64_t g = (work_items + per_block - 1) / per_block;
-  const int64_t cap = (int64_t)device_sm_count() * max_ctas_per_sm;
-  if (g > cap) g = cap;
-  if (g < 1) g = 1;
-  return (unsigned)g;
-}
-
 }  // namespace polar
 
 using namespace polar;
 
 extern "C" int polar_encode_packed(const uint32_t *d_u, int n, int64_t B, uint32_t *d_c, void *stream) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_MAX_N) return set_error(POLAR_EINVAL, "encode: n=%d must be a power of two in [2,%d]", n, POLAR_MAX_N);
+  if (const int rc = check_pow2_n("encode", n, 2, POLAR_MAX_N)) return rc;
   if (B < 0) return set_error(POLAR_EINVAL, "encode: B < 0");
   if (B == 0) return POLAR_OK;
   if (!d_u || !d_c) return set_error(POLAR_EINVAL, "encode: null pointer");
@@ -178,51 +170,34 @@ extern "C" int polar_encode_packed(const uint32_t *d_u, int n, int64_t B, uint32
   const int m = ilog2(n), nw = POLAR_WORDS(n);
   if (n <= 1024) {
     const int64_t total = B * nw;
-    enc_packed_small_kernel<<<grid_for((total + 31) / 32, 8), 256, 0, st>>>(d_u, m, nw, total, d_c);
-  } else if (n == 2048) {
-    enc_packed_kernel<2><<<grid_for(B, 8), 256, 0, st>>>(d_u, m, B, d_c);
-  } else if (n == 4096) {
-    enc_packed_kernel<4><<<grid_for(B, 8), 256, 0, st>>>(d_u, m, B, d_c);
-  } else {
-    enc_packed_kernel<8><<<grid_for(B, 8), 256, 0, st>>>(d_u, m, B, d_c);
+    return launch("enc_packed", enc_packed_small_kernel, grid_for((total + 31) / 32, 8, 8), 256, 0, st, d_u, m, nw, total, d_c);
   }
-  count_launch();
-  POLAR_CHECK_LAUNCH("enc_packed");
-  return POLAR_OK;
+  const auto kern = n == 2048 ? enc_packed_kernel<2> : n == 4096 ? enc_packed_kernel<4> : enc_packed_kernel<8>;
+  return launch("enc_packed", kern, grid_for(B, 8, 8), 256, 0, st, d_u, m, B, d_c);
 }
 
 extern "C" int polar_encode_f32(const float *d_u, const int32_t *d_info_rank, int n, int k, int64_t B, float *d_c,
                                 uint32_t *d_c_packed, void *stream) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_MAX_N) return set_error(POLAR_EINVAL, "encode: n=%d must be a power of two in [2,%d]", n, POLAR_MAX_N);
+  if (const int rc = check_pow2_n("encode", n, 2, POLAR_MAX_N)) return rc;
   if (B < 0 || k < 0 || k > n) return set_error(POLAR_EINVAL, "encode: bad B/k");
   if (B == 0) return POLAR_OK;
   if (!d_u || !d_info_rank || !d_c) return set_error(POLAR_EINVAL, "encode: null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int m = ilog2(n);
-  const unsigned g = grid_for(B, 8);
-  if (n <= 1024) enc_f32_kernel<1><<<g, 256, 0, st>>>(d_u, d_info_rank, n, m, k, B, d_c, d_c_packed);
-  else if (n == 2048) enc_f32_kernel<2><<<g, 256, 0, st>>>(d_u, d_info_rank, n, m, k, B, d_c, d_c_packed);
-  else if (n == 4096) enc_f32_kernel<4><<<g, 256, 0, st>>>(d_u, d_info_rank, n, m, k, B, d_c, d_c_packed);
-  else enc_f32_kernel<8><<<g, 256, 0, st>>>(d_u, d_info_rank, n, m, k, B, d_c, d_c_packed);
-  count_launch();
-  POLAR_CHECK_LAUNCH("enc_f32");
-  return POLAR_OK;
+  const auto kern = n <= 1024 ? enc_f32_kernel<1> : n == 2048 ? enc_f32_kernel<2> : n == 4096 ? enc_f32_kernel<4> : enc_f32_kernel<8>;
+  return launch("enc_f32", kern, grid_for(B, 8, 8), 256, 0, (cudaStream_t)stream, d_u, d_info_rank, n, ilog2(n), k, B, d_c,
+                d_c_packed);
 }
 
 extern "C" int polar_pack_bits_f32(const float *d_x, int n, int64_t B, uint32_t *d_packed, void *stream) {
   if (n < 1 || B < 0 || (n > 32 && (n & 31))) return set_error(POLAR_EINVAL, "pack: n must be <= 32 or a multiple of 32");
   if (B == 0) return POLAR_OK;
   if (!d_x || !d_packed) return set_error(POLAR_EINVAL, "pack: null pointer");
-  const int nw = POLAR_WORDS(n);
+  const cudaStream_t st = (cudaStream_t)stream;
   if ((n & 127) == 0 && ((uintptr_t)d_x & 15) == 0) {
     const int64_t chunks = B * (int64_t)(n >> 7);
-    pack_bits_vec_kernel<<<grid_for(chunks, 8), 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const float4 *>(d_x), chunks, d_packed);
-  } else {
-    pack_bits_kernel<<<grid_for(B * nw, 8), 256, 0, (cudaStream_t)stream>>>(d_x, n, B, d_packed);
+    return launch("pack_bits", pack_bits_vec_kernel, grid_for(chunks, 8, 8), 256, 0, st, reinterpret_cast<const float4 *>(d_x),
+                  chunks, d_packed);
   }
-  count_launch();
-  POLAR_CHECK_LAUNCH("pack_bits");
-  return POLAR_OK;
+  return launch("pack_bits", pack_bits_kernel, grid_for(B * POLAR_WORDS(n), 8, 8), 256, 0, st, d_x, n, B, d_packed);
 }
 
 extern "C" int polar_unpack_info_f32(const uint32_t *d_packed, const int32_t *d_pos, int n, int k, int64_t B,
@@ -231,12 +206,9 @@ extern "C" int polar_unpack_info_f32(const uint32_t *d_packed, const int32_t *d_
   if (B == 0 || k == 0) return POLAR_OK;
   if (!d_packed || !d_pos || !d_out) return set_error(POLAR_EINVAL, "unpack: null pointer");
   const bool vec = (k & 3) == 0 && (((uintptr_t)d_pos | (uintptr_t)d_out) & 15) == 0;
-  const unsigned grid = grid_for(B, 8);                    // one warp per row, 8 warps per CTA
-  if (vec) unpack_info_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(d_packed, d_pos, POLAR_WORDS(n), k, B, d_out);
-  else unpack_info_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(d_packed, d_pos, POLAR_WORDS(n), k, B, d_out);
-  count_launch();
-  POLAR_CHECK_LAUNCH("unpack_info");
-  return POLAR_OK;
+  const auto kern = vec ? unpack_info_kernel<true> : unpack_info_kernel<false>;
+  return launch("unpack_info", kern, grid_for(B, 8, 8), 256, 0, (cudaStream_t)stream,   // one warp per row, 8 warps per CTA
+                d_packed, d_pos, POLAR_WORDS(n), k, B, d_out);
 }
 
 
@@ -278,24 +250,14 @@ __global__ void __launch_bounds__(256) rate_recover_kernel(const float *__restri
 }
 }  // namespace polar
 
-static unsigned perm_grid(int64_t rows) {              // one warp per row, 8 warps per CTA
-  int64_t g = (rows + 7) / 8;
-  const int64_t cap = (int64_t)polar::device_sm_count() * 16;
-  if (g > cap) g = cap;
-  if (g < 1) g = 1;
-  return (unsigned)g;
-}
-
 extern "C" int polar_gather_cols_f32(const float *d_x, const int32_t *d_idx, int n_in, int n_out, int64_t B, float *d_out,
                                      void *stream) {
   using namespace polar;
   if (n_in < 1 || n_out < 1 || B < 0) return set_error(POLAR_EINVAL, "gather: bad sizes");
   if (B == 0) return POLAR_OK;
   if (!d_x || !d_idx || !d_out) return set_error(POLAR_EINVAL, "gather: null pointer");
-  gather_cols_kernel<<<perm_grid(B), 256, 0, (cudaStream_t)stream>>>(d_x, d_idx, n_in, n_out, B, d_out);
-  count_launch();
-  POLAR_CHECK_LAUNCH("gather_cols");
-  return POLAR_OK;
+  return launch("gather_cols", gather_cols_kernel, grid_for(B, 8, 16), 256, 0, (cudaStream_t)stream, d_x, d_idx, n_in, n_out,
+                B, d_out);
 }
 
 extern "C" int polar_rate_recover_f32(const float *d_x, const int32_t *d_src0, const int32_t *d_src1, const float *d_fill,
@@ -304,8 +266,6 @@ extern "C" int polar_rate_recover_f32(const float *d_x, const int32_t *d_src0, c
   if (n_in < 1 || n_out < 1 || B < 0) return set_error(POLAR_EINVAL, "rate_recover: bad sizes");
   if (B == 0) return POLAR_OK;
   if (!d_x || !d_src0 || !d_src1 || !d_fill || !d_out) return set_error(POLAR_EINVAL, "rate_recover: null pointer");
-  rate_recover_kernel<<<perm_grid(B), 256, 0, (cudaStream_t)stream>>>(d_x, d_src0, d_src1, d_fill, n_in, n_out, B, d_out);
-  count_launch();
-  POLAR_CHECK_LAUNCH("rate_recover");
-  return POLAR_OK;
+  return launch("rate_recover", rate_recover_kernel, grid_for(B, 8, 16), 256, 0, (cudaStream_t)stream, d_x, d_src0, d_src1,
+                d_fill, n_in, n_out, B, d_out);
 }

@@ -11,7 +11,7 @@
 // -> two Box-Muller pairs -> one 128-bit store).  HBM-bound on the [B,n] fp32 logit write.
 #include <atomic>
 
-#include "polar_internal.h"
+#include "polar_launch.h"
 #include "polar_warp.cuh"
 
 namespace polar {
@@ -216,51 +216,58 @@ __global__ void __launch_bounds__(256) qpsk_awgn_kernel(uint64_t seed, uint64_t 
 
 using namespace polar;
 
-// Persistent grid-stride kernels: exactly as many CTAs as are resident at once (the kernel needs 40 registers, so 6 CTAs of
-// 256 threads per SM, not 8 -- with 8 x SMs CTAs a third of them ran as a second, mostly empty wave).
+// The front ends are persistent grid-stride kernels, one warp per codeword: exactly as many CTAs as are resident at once
+// (the kernel needs 40 registers, so 6 CTAs of 256 threads per SM, not 8 -- with 8 x SMs CTAs a third of them ran as a
+// second, mostly empty wave).  The occupancy query runs once per instantiation of this template, i.e. per kernel type:
+// the first frontend_kernel<R, BEC> launched sets it for all of them, nr5g_frontend_kernel has its own.
 template <class K>
-static unsigned fe_grid(K kern, int64_t warps_needed) {
-  static std::atomic<int> per_sm{0};                     // one value per kernel instantiation (function-local static of a template)
+static int frontend_ctas_per_sm(K kern) {
+  static std::atomic<int> per_sm{0};
   int r = per_sm.load(std::memory_order_relaxed);
   if (r <= 0) {
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&r, kern, 256, 0) != cudaSuccess || r <= 0) { (void)cudaGetLastError(); r = 4; }
+    r = resident_ctas(kern, 256, 0);
     per_sm.store(r, std::memory_order_relaxed);
   }
-  int64_t g = (warps_needed + 7) / 8;
-  const int64_t cap = (int64_t)device_sm_count() * r;
-  if (g > cap) g = cap;
-  if (g < 1) g = 1;
-  return (unsigned)g;
+  return r;
+}
+
+// the AWGN (a = sigma, b = scale) and the BEC (a = pe, b = llr_max) front end
+template <bool BEC>
+static int launch_frontend(const char *what, uint64_t seed, uint64_t offset, float a, float b, const uint32_t *fmask, int n,
+                           int64_t B, uint32_t *u_out, uint32_t *c_out, float *logit, void *stream) {
+  const auto kern = n <= 1024 ? frontend_kernel<1, BEC> : n == 2048 ? frontend_kernel<2, BEC>
+                    : n == 4096 ? frontend_kernel<4, BEC> : frontend_kernel<8, BEC>;
+  return launch(what, kern, grid_for(B, 8, frontend_ctas_per_sm(kern)), 256, 0, (cudaStream_t)stream, seed, offset, a, b,
+                fmask, n, ilog2(n), B, u_out, c_out, logit);
+}
+
+// the channel alone, on caller-supplied codewords: QPSK/AWGN (a = sigma, b = scale) or BEC (a = pe, b = llr_max)
+template <bool BEC>
+static int launch_channel(const char *what, uint64_t seed, uint64_t offset, float a, float b, const float *c, int n, int64_t B,
+                          float *logit, void *stream) {
+  return launch(what, qpsk_awgn_kernel<BEC>, grid_for(B * (int64_t)(n >> 2), 256, 8), 256, 0, (cudaStream_t)stream, seed,
+                offset, a, b, c, n, B, logit);
 }
 
 extern "C" int polar_awgn_frontend(uint64_t seed, uint64_t offset, float no, const uint32_t *d_frozen_mask, int n,
                                    int64_t B, uint32_t *d_u_packed_out, uint32_t *d_c_packed_out, float *d_logit_out,
                                    void *stream) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_MAX_N) return set_error(POLAR_EINVAL, "frontend: n=%d must be a power of two in [2,%d]", n, POLAR_MAX_N);
+  if (const int rc = check_pow2_n("frontend", n, 2, POLAR_MAX_N)) return rc;
   if (B < 0 || !(no > 0.0f)) return set_error(POLAR_EINVAL, "frontend: B < 0 or no <= 0");
   if (B == 0) return POLAR_OK;
   if (!d_frozen_mask || !d_logit_out) return set_error(POLAR_EINVAL, "frontend: null pointer");
   if (n >= 4 && ((uintptr_t)d_logit_out & 15)) return set_error(POLAR_EALIGN, "frontend: logit_out must be 16-byte aligned");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int m = ilog2(n);
   const float sigma = sqrtf(no * 0.5f);                   // std per real dimension (utils.py:12-13, awgn.py:27)
   const float scale = -2.0f * 1.41421356237309505f / no;  // closed-form demapper
-#define POLAR_FE_LAUNCH(R) frontend_kernel<R><<<fe_grid(frontend_kernel<R>, B), 256, 0, st>>>(seed, offset, sigma, scale, d_frozen_mask, n, m, B, d_u_packed_out, d_c_packed_out, d_logit_out)
-  if (n <= 1024) POLAR_FE_LAUNCH(1);
-  else if (n == 2048) POLAR_FE_LAUNCH(2);
-  else if (n == 4096) POLAR_FE_LAUNCH(4);
-  else POLAR_FE_LAUNCH(8);
-#undef POLAR_FE_LAUNCH
-  count_launch();
-  POLAR_CHECK_LAUNCH("frontend");
-  return POLAR_OK;
+  return launch_frontend<false>("frontend", seed, offset, sigma, scale, d_frozen_mask, n, B, d_u_packed_out, d_c_packed_out,
+                                d_logit_out, stream);
 }
 
 extern "C" int polar_nr5g_awgn_frontend(uint64_t seed, uint64_t offset, float no, const uint32_t *d_payload_mask,
                                         const uint32_t *d_crc_rows, const int32_t *d_crc_pos, int crc_len,
                                         const int32_t *d_rm_idx, int n, int e, int64_t B, uint32_t *d_u_packed_out,
                                         uint32_t *d_c_packed_out, float *d_logit_out, void *stream) {
-  if (!is_pow2(n) || n < 32 || n > 1024) return set_error(POLAR_EINVAL, "nr5g frontend: n=%d must be a power of two in [32,1024]", n);
+  if (const int rc = check_pow2_n("nr5g frontend", n, 32, 1024)) return rc;
   if (e < 1 || e > POLAR_MAX_N) return set_error(POLAR_EINVAL, "nr5g frontend: e=%d outside [1,%d]", e, POLAR_MAX_N);
   if (crc_len < 1 || crc_len > 32) return set_error(POLAR_EINVAL, "nr5g frontend: crc_len=%d outside [1,32]", crc_len);
   if (B < 0 || !(no > 0.0f)) return set_error(POLAR_EINVAL, "nr5g frontend: B < 0 or no <= 0");
@@ -268,12 +275,10 @@ extern "C" int polar_nr5g_awgn_frontend(uint64_t seed, uint64_t offset, float no
   if (B == 0) return POLAR_OK;
   if (!d_u_packed_out || !d_logit_out) return set_error(POLAR_EINVAL, "nr5g frontend: null output pointer");
   const float sigma = sqrtf(no * 0.5f), scale = -2.0f * 1.41421356237309505f / no;
-  nr5g_frontend_kernel<<<fe_grid(nr5g_frontend_kernel, B), 256, 0, (cudaStream_t)stream>>>(
-      seed, offset, sigma, scale, d_payload_mask, d_crc_rows, d_crc_pos, crc_len, d_rm_idx, n, ilog2(n), e, B,
-      d_u_packed_out, d_c_packed_out, d_logit_out);
-  count_launch();
-  POLAR_CHECK_LAUNCH("nr5g_frontend");
-  return POLAR_OK;
+  const unsigned grid = grid_for(B, 8, frontend_ctas_per_sm(nr5g_frontend_kernel));
+  return launch("nr5g_frontend", nr5g_frontend_kernel, grid, 256, 0, (cudaStream_t)stream, seed, offset, sigma, scale,
+                d_payload_mask, d_crc_rows, d_crc_pos, crc_len, d_rm_idx, n, ilog2(n), e, B, d_u_packed_out, d_c_packed_out,
+                d_logit_out);
 }
 
 extern "C" int polar_qpsk_awgn_llr(uint64_t seed, uint64_t offset, float no, const float *d_c, int n, int64_t B,
@@ -283,36 +288,20 @@ extern "C" int polar_qpsk_awgn_llr(uint64_t seed, uint64_t offset, float no, con
   if (!d_c || !d_logit_out) return set_error(POLAR_EINVAL, "qpsk_awgn: null pointer");
   if (((uintptr_t)d_c & 15) || ((uintptr_t)d_logit_out & 15)) return set_error(POLAR_EALIGN, "qpsk_awgn: buffers must be 16-byte aligned");
   const float sigma = sqrtf(no * 0.5f), scale = -2.0f * 1.41421356237309505f / no;
-  const int64_t total = B * (int64_t)(n >> 2);
-  int64_t g = (total + 255) / 256;
-  const int64_t cap = (int64_t)device_sm_count() * 8;
-  if (g > cap) g = cap;
-  qpsk_awgn_kernel<false><<<(unsigned)g, 256, 0, (cudaStream_t)stream>>>(seed, offset, sigma, scale, d_c, n, B, d_logit_out);
-  count_launch();
-  POLAR_CHECK_LAUNCH("qpsk_awgn");
-  return POLAR_OK;
+  return launch_channel<false>("qpsk_awgn", seed, offset, sigma, scale, d_c, n, B, d_logit_out, stream);
 }
 
 // ---- binary erasure channel (SURVEY 8f row N4, channel half) ------------------------------------------------------
 extern "C" int polar_bec_frontend(uint64_t seed, uint64_t offset, float pe, float llr_max, const uint32_t *d_frozen_mask,
                                   int n, int64_t B, uint32_t *d_u_packed_out, uint32_t *d_c_packed_out, float *d_logit_out,
                                   void *stream) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_MAX_N) return set_error(POLAR_EINVAL, "bec frontend: n=%d must be a power of two in [2,%d]", n, POLAR_MAX_N);
+  if (const int rc = check_pow2_n("bec frontend", n, 2, POLAR_MAX_N)) return rc;
   if (B < 0 || !(pe >= 0.0f && pe <= 1.0f) || !(llr_max >= 0.0f)) return set_error(POLAR_EINVAL, "bec frontend: B < 0, pe outside [0,1] or llr_max < 0");
   if (B == 0) return POLAR_OK;
   if (!d_frozen_mask || !d_logit_out) return set_error(POLAR_EINVAL, "bec frontend: null pointer");
   if (n >= 4 && ((uintptr_t)d_logit_out & 15)) return set_error(POLAR_EALIGN, "bec frontend: logit_out must be 16-byte aligned");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int m = ilog2(n);
-#define POLAR_FE_LAUNCH(R) frontend_kernel<R, true><<<fe_grid(frontend_kernel<R, true>, B), 256, 0, st>>>(seed, offset, pe, llr_max, d_frozen_mask, n, m, B, d_u_packed_out, d_c_packed_out, d_logit_out)
-  if (n <= 1024) POLAR_FE_LAUNCH(1);
-  else if (n == 2048) POLAR_FE_LAUNCH(2);
-  else if (n == 4096) POLAR_FE_LAUNCH(4);
-  else POLAR_FE_LAUNCH(8);
-#undef POLAR_FE_LAUNCH
-  count_launch();
-  POLAR_CHECK_LAUNCH("bec_frontend");
-  return POLAR_OK;
+  return launch_frontend<true>("bec_frontend", seed, offset, pe, llr_max, d_frozen_mask, n, B, d_u_packed_out, d_c_packed_out,
+                               d_logit_out, stream);
 }
 
 extern "C" int polar_bec_llr(uint64_t seed, uint64_t offset, float pe, float llr_max, const float *d_c, int n, int64_t B,
@@ -321,12 +310,5 @@ extern "C" int polar_bec_llr(uint64_t seed, uint64_t offset, float pe, float llr
   if (B == 0) return POLAR_OK;
   if (!d_c || !d_logit_out) return set_error(POLAR_EINVAL, "bec: null pointer");
   if (((uintptr_t)d_c & 15) || ((uintptr_t)d_logit_out & 15)) return set_error(POLAR_EALIGN, "bec: buffers must be 16-byte aligned");
-  const int64_t total = B * (int64_t)(n >> 2);
-  int64_t g = (total + 255) / 256;
-  const int64_t cap = (int64_t)device_sm_count() * 8;
-  if (g > cap) g = cap;
-  qpsk_awgn_kernel<true><<<(unsigned)g, 256, 0, (cudaStream_t)stream>>>(seed, offset, pe, llr_max, d_c, n, B, d_logit_out);
-  count_launch();
-  POLAR_CHECK_LAUNCH("bec_llr");
-  return POLAR_OK;
+  return launch_channel<true>("bec_llr", seed, offset, pe, llr_max, d_c, n, B, d_logit_out, stream);
 }

@@ -13,6 +13,7 @@
 #include <vector>
 
 #include "polar_internal.h"
+#include "polar_sc.h"
 #include "polar_scl.h"
 
 namespace polar {
@@ -159,8 +160,8 @@ static int run_chunks(HostCtx &C, const HostJob &J, int64_t chunk, size_t ws_nee
                              (const int32_t *)C.pos, k, J.h_pm ? (double *)C.pm[idx] : nullptr, nullptr, J.crc_dev, J.crc_len,
                              ws_need ? C.ws[idx] : nullptr, ws_need ? C.ws_bytes : 0, st);
       else
-        r = polar_sc_decode_f32((const float *)C.logit[idx], (const uint32_t *)C.mask, n, nb, d_out, d_info,
-                                (const int32_t *)C.pos, k, st);
+        r = sc_decode(Arith::minsum, (const float *)C.logit[idx], (const uint32_t *)C.mask, n, nb, d_out, d_info,
+                      (const int32_t *)C.pos, k, st);
       if (r) return r;
       if (J.h_packed)
         POLAR_CUDA(cudaMemcpyAsync(out_staged ? C.h_out[idx] : (void *)(J.h_packed + b0 * nw), C.out[idx], (size_t)nb * nw * 4,
@@ -208,17 +209,15 @@ using namespace polar;
 extern "C" int polar_sc_decode_host_f32(const float *h_logit, const uint32_t *h_frozen_mask, int n, int64_t B,
                                         uint32_t *h_u_packed, float *h_u_info_f32, const int32_t *h_info_pos, int k,
                                         int device) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_MAX_N || B < 0) return set_error(POLAR_EINVAL, "sc host: bad n/B");
-  if (B == 0) return POLAR_OK;
-  if (!h_logit || !h_frozen_mask || (!h_u_packed && !h_u_info_f32)) return set_error(POLAR_EINVAL, "sc host: null pointer");
-  if (h_u_info_f32 && (!h_info_pos || k < 1 || k > n)) return set_error(POLAR_EINVAL, "sc host: u_info requested without valid info_pos/k");
+  int rc = check_sc_args("sc host", n, B, h_logit, h_frozen_mask, h_u_packed || h_u_info_f32, h_u_info_f32, h_info_pos, k);
+  if (rc != POLAR_OK || B == 0) return rc;
+  if (h_u_info_f32 && k < 1) return set_error(POLAR_EINVAL, "sc host: u_info requested without valid info_pos/k");
   if (device < 0 || device >= 64) return set_error(POLAR_EINVAL, "sc host: bad device");
-  if (B == 0) return POLAR_OK;
   HostCtx &C = g_ctx[device];
   std::lock_guard<std::mutex> lk(C.mu);
   DeviceGuard guard(device);
   if (!guard.ok) return set_error(POLAR_ECUDA, "sc host: cannot select device %d", device);
-  int rc = polar_init(device);
+  rc = polar_init(device);
   if (rc) return rc;
   if ((rc = prepare(C, h_frozen_mask, n, h_u_info_f32 ? h_info_pos : nullptr, k))) return rc;
   POLAR_CUDA(cudaStreamSynchronize(C.st[0]));
@@ -247,14 +246,14 @@ extern "C" int polar_scl_decode_host_f32(const float *h_logit, const uint32_t *h
   rc = polar_init(device);
   if (rc) return rc;
   int64_t chunk = chunk_codewords(n, B, true);        // the list decoder's time per chunk is not hidden by the copy: large chunks
-  const SclPlan whole = scl_plan(n, L, B, SclArith::minsum, true);   // the chunk buffers are cudaMalloc'd: aligned rows
+  const SclPlan whole = scl_plan(n, L, B, Arith::minsum, true);   // the chunk buffers are cudaMalloc'd: aligned rows
   if (whole.scl3 && chunk < B) {
     // the list kernel is persistent: every resident warp decodes the same number of 32/L-codeword groups, so a chunk
     // should be a whole number of such rounds (a 128 MB chunk of n = 1024 is 3.46 rounds: 13 % of the last one idle)
     const int64_t round = whole.grid * (32 / L);
     if (chunk > round) chunk = chunk / round * round;
   }
-  const size_t ws_need = scl_plan(n, L, chunk, SclArith::minsum, true).ws_bytes;
+  const size_t ws_need = scl_plan(n, L, chunk, Arith::minsum, true).ws_bytes;
   if ((rc = prepare(C, h_frozen_mask, n, h_u_info_f32 ? h_info_pos : nullptr, k))) return rc;
   const bool crc = crc_len > 0 && h_crc_rows;
   if (crc) {

@@ -17,7 +17,7 @@
 // the reference's to rounding, and so does the decision except where two candidates are closer than that (the tests
 // skip exactly those, like the list decoder's ill-conditioned lists).
 #include "polar_common.cuh"
-#include "polar_internal.h"
+#include "polar_launch.h"
 
 namespace polar {
 namespace {
@@ -282,15 +282,8 @@ extern "C" int polar_osd_decode(const float *d_logit, const uint32_t *d_gm_rows,
   const OsdLayout lay = osd_layout(n, k);
   if (lay.total > (size_t)device_max_smem_optin()) return set_error(POLAR_ENOMEM, "osd: n=%d k=%d does not fit in shared memory", n, k);
   POLAR_CUDA(cudaFuncSetAttribute(osd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lay.total));
-  int per_sm = 0;                                        // persistent CTAs: as many as are resident at once
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, osd_kernel, kOsdThreads, lay.total) != cudaSuccess || per_sm <= 0) {
-    (void)cudaGetLastError();
-    per_sm = 4;
-  }
-  int64_t grid = (int64_t)device_sm_count() * per_sm;
-  if (grid > B) grid = B;
-  osd_kernel<<<(unsigned)grid, kOsdThreads, lay.total, (cudaStream_t)stream>>>(d_logit, d_gm_rows, n, k, t, B, d_c_packed, d_c_f32, d_dist);
-  count_launch();
-  POLAR_CHECK_LAUNCH("osd_kernel");
-  return POLAR_OK;
+  // persistent CTAs: as many as are resident at once, queried on every call because the shared memory depends on n and k
+  const unsigned grid = grid_for(B, 1, resident_ctas(osd_kernel, kOsdThreads, lay.total));
+  return launch("osd_kernel", osd_kernel, grid, kOsdThreads, lay.total, (cudaStream_t)stream, d_logit, d_gm_rows, n, k, t, B,
+                d_c_packed, d_c_f32, d_dist);
 }

@@ -1,16 +1,14 @@
-// polar_sc.cu -- SC decoder entry point for sm_100a (fp32 min-sum, bit-exact with the reference) and the kernels for
-// the short codes.
+// polar_sc.cu -- SC decoder kernels for the short codes, n <= 64: one thread per codeword, the whole tree in registers
+// (fp32 min-sum, bit-exact with the reference; exact boxplus in the polar_bp build, polar_bp_wrap.cu).
 //
 // Replaces x_run_sn_polar/polar/polar_sc.py:54-133 (recursion, f/g, leaf rule, partial sums, info gather).
-// Semantics: SURVEY.md Appendix A.  Three mappings behind polar_sc_decode_f32, chosen by the code length alone:
-//   n <= 64           one thread per codeword, the whole tree in registers (this file);
-//   128 <= n <= 512   a warp per 32 codewords, everything on chip: shared memory / tensor memory / registers (polar_sc4.cu);
-//   n >= 1024         the same with TMA-staged fused descents through the top stages and a global scratch hierarchy for
-//                     the stages that do not fit on chip (polar_sc5.cu).
+// Semantics: SURVEY.md Appendix A.  The entry points and the choice of mapping by code length are in polar_sc_api.cu;
+// the longer codes run on polar_sc4.cu (128 <= n <= 512) and polar_sc5.cu (n >= 1024).
 // Rate-0 nodes (all frozen) are skipped and rate-1 subtrees take the hard-decision shortcut when no LLR is exactly 0 (both
 // exact, see polar_common.cuh).
 #include "polar_common.cuh"
 #include "polar_internal.h"
+#include "polar_sc.h"
 
 namespace polar {
 
@@ -79,51 +77,13 @@ __global__ void __launch_bounds__(128) sc64_kernel(const float *__restrict__ log
   }
 }
 
-static unsigned small_grid(int64_t B) {
-  int64_t grid = (B + 127) / 128;
-  const int64_t cap = (int64_t)device_sm_count() * 16;
-  if (grid > cap) grid = cap;
-  if (grid < 1) grid = 1;
-  return (unsigned)grid;
-}
-
-template <int T>
-static int launch_small(const float *logit, const uint32_t *fmask, int64_t B, uint32_t *u_packed, float *u_info,
-                        const int32_t *info_pos, int k, cudaStream_t st) {
-  sc_small_kernel<T><<<small_grid(B), 128, 0, st>>>(logit, fmask, B, u_packed, u_info, info_pos, k);
-  count_launch();
-  POLAR_CHECK_LAUNCH("sc_small_kernel");
-  return POLAR_OK;
+int launch_sc_small(const float *logit, const uint32_t *fmask, int n, int64_t B, uint32_t *u_packed, float *u_info,
+                    const int32_t *info_pos, int k, cudaStream_t st) {
+  const unsigned grid = grid_for(B, 128, 16);
+  if (n == 64) return launch("sc64_kernel", sc64_kernel, grid, 128, 0, st, logit, fmask, B, u_packed, u_info, info_pos, k);
+  const auto kern = n == 2 ? sc_small_kernel<1> : n == 4 ? sc_small_kernel<2> : n == 8 ? sc_small_kernel<3>
+                    : n == 16 ? sc_small_kernel<4> : sc_small_kernel<5>;
+  return launch("sc_small_kernel", kern, grid, 128, 0, st, logit, fmask, B, u_packed, u_info, info_pos, k);
 }
 
 }  // namespace polar
-
-extern "C" int polar_sc_decode_f32(const float *d_logit, const uint32_t *d_frozen_mask, int n, int64_t B,
-                                   uint32_t *d_u_packed, float *d_u_info_f32, const int32_t *d_info_pos,
-                                   int k, void *stream) {
-  using namespace polar;
-  if (!is_pow2(n) || n < 2 || n > POLAR_MAX_N) return set_error(POLAR_EINVAL, "sc: n=%d must be a power of two in [2,%d]", n, POLAR_MAX_N);
-  if (B < 0) return set_error(POLAR_EINVAL, "sc: B=%lld < 0", (long long)B);
-  if (B == 0) return POLAR_OK;
-  if (!d_logit || !d_frozen_mask) return set_error(POLAR_EINVAL, "sc: null logit / frozen_mask");
-  if (!d_u_packed && !d_u_info_f32) return set_error(POLAR_EINVAL, "sc: no output buffer");
-  if (d_u_info_f32 && (!d_info_pos || k < 0 || k > n)) return set_error(POLAR_EINVAL, "sc: u_info requested without valid info_pos/k");
-  if (n >= 4 && ((uintptr_t)d_logit & 15)) return set_error(POLAR_EALIGN, "sc: logit must be 16-byte aligned");
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (n) {
-    case 2: return launch_small<1>(d_logit, d_frozen_mask, B, d_u_packed, d_u_info_f32, d_info_pos, k, st);
-    case 4: return launch_small<2>(d_logit, d_frozen_mask, B, d_u_packed, d_u_info_f32, d_info_pos, k, st);
-    case 8: return launch_small<3>(d_logit, d_frozen_mask, B, d_u_packed, d_u_info_f32, d_info_pos, k, st);
-    case 16: return launch_small<4>(d_logit, d_frozen_mask, B, d_u_packed, d_u_info_f32, d_info_pos, k, st);
-    case 32: return launch_small<5>(d_logit, d_frozen_mask, B, d_u_packed, d_u_info_f32, d_info_pos, k, st);
-    case 64:
-      sc64_kernel<<<small_grid(B), 128, 0, st>>>(d_logit, d_frozen_mask, B, d_u_packed, d_u_info_f32, d_info_pos, k);
-      count_launch();
-      POLAR_CHECK_LAUNCH("sc64_kernel");
-      return POLAR_OK;
-    default: break;
-  }
-  const int warps = env_int("POLAR_SC_WARPS_SM", 0);      // autonomous warps per SM (0 = as many as the on-chip storage holds)
-  if (n <= 512) return polar::launch_sc4(d_logit, d_frozen_mask, n, B, d_u_packed, d_u_info_f32, d_info_pos, k, warps, st);
-  return polar::launch_sc5(d_logit, d_frozen_mask, n, B, d_u_packed, d_u_info_f32, d_info_pos, k, warps, st);
-}

@@ -21,6 +21,7 @@
 #define POLAR_BT5_UNROLL 1
 #include "polar_common.cuh"
 #include "polar_internal.h"
+#include "polar_launch.h"
 
 namespace polar {
 
@@ -500,15 +501,9 @@ int launch_sc4_t(const float *logit, const uint32_t *fmask, int64_t B, uint32_t 
   size_t smem = lay.total;
   if (TM && smem < (size_t)116 * 1024) smem = (size_t)116 * 1024;
   POLAR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int sms = device_sm_count();
   const int64_t nbatches = (B + 31) / 32;
-  int64_t grid = (nbatches + warps - 1) / warps;
-  if (grid > sms) grid = sms;
-  if (grid < 1) grid = 1;
-  kern<<<(unsigned)grid, warps * 32, smem, st>>>(logit, fmask, B, nbatches, u_packed, u_info, info_pos, k);
-  count_launch();
-  POLAR_CHECK_LAUNCH("sc4_kernel");
-  return POLAR_OK;
+  return launch("sc4_kernel", kern, grid_for(nbatches, warps, 1), warps * 32, smem, st, logit, fmask, B, nbatches, u_packed,
+                u_info, info_pos, k);
 }
 
 }  // namespace

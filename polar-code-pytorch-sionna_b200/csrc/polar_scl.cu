@@ -25,7 +25,7 @@ constexpr double kLlrMaxD = 30.0;
 
 #if defined(POLAR_F_BOXPLUS)
 // exact boxplus of the Sionna-style list decoder (my_sn/fec/polar/dec.py:331-340, numpy float64): clip to +-30,
-// ln(1+e^(x+y)) - ln(e^x+e^y).  Selected by polar_bp_wrap.cu (namespace polar_bp, launcher launch_scl2_boxplus).
+// ln(1+e^(x+y)) - ln(e^x+e^y).  Selected by polar_bp_wrap.cu (namespace polar_bp, launcher polar_bp::launch_scl2).
 __device__ __forceinline__ double f_minsum_d(double a, double b) {
   const double x = fmax(fmin(a, 30.0), -30.0), y = fmax(fmin(b, 30.0), -30.0);
   return log(1.0 + exp(x + y)) - log(exp(x) + exp(y));
@@ -353,17 +353,11 @@ __global__ void __launch_bounds__(128, SCL2_MINB) scl2_kernel(const SclParams P)
   }
 }
 
-}  // namespace polar
-
-using namespace polar;
-
-// launch_scl2 (launch_scl2_boxplus in the boxplus build), declared in polar_scl.h.  At most 4 KB of dynamic shared
-// memory per warp (scl_plan), under the default limit.
+// At most 4 KB of dynamic shared memory per warp (scl_plan), under the default limit.
 int launch_scl2(const SclParams &P, const SclPlan &pl, int L, cudaStream_t st) {
-  void (*kern)(const SclParams) = L == 1 ? scl2_kernel<1> : L == 2 ? scl2_kernel<2> : L == 4 ? scl2_kernel<4>
-                                  : L == 8 ? scl2_kernel<8> : L == 16 ? scl2_kernel<16> : scl2_kernel<32>;
-  kern<<<(unsigned)pl.grid, 32, P.smem_per_warp, st>>>(P);
-  count_launch();
-  POLAR_CHECK_LAUNCH("scl2_kernel");
-  return POLAR_OK;
+  const auto kern = L == 1 ? scl2_kernel<1> : L == 2 ? scl2_kernel<2> : L == 4 ? scl2_kernel<4>
+                    : L == 8 ? scl2_kernel<8> : L == 16 ? scl2_kernel<16> : scl2_kernel<32>;
+  return launch("scl2_kernel", kern, (unsigned)pl.grid, 32, P.smem_per_warp, st, P);
 }
+
+}  // namespace polar

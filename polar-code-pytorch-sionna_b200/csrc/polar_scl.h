@@ -3,16 +3,11 @@
 //
 // polar_scl.cu is compiled twice (min-sum into namespace polar, exact boxplus into namespace polar_bp through
 // polar_bp_wrap.cu).  polar_bp_wrap.cu includes this header before it renames the namespace, so both builds share the
-// types below; its launcher is renamed launch_scl2_boxplus.
+// types below and define the launcher declared here in both namespaces.
 #pragma once
-#include <cuda_runtime.h>
-#include <stddef.h>
-#include <stdint.h>
+#include "polar_launch.h"
 
 namespace polar {
-
-// check-node arithmetic of a list decode; the values are the cn_mode of polar_scl_decode_hybrid
-enum class SclArith { minsum = 0, boxplus = 1, boxplus_pruned = 2 };
 
 struct SclParams {
   const float *logit; const uint32_t *fmask; int n, m; int64_t B;
@@ -43,10 +38,13 @@ __host__ __device__ inline size_t scl2_llr_smem_doubles(int s_glob) { return (si
 // polar_scl_api.cu.  check_scl_shape: n, L and B of any list-decoder call.  scl_plan: the mapping, grid and workspace
 // of a decode of B rows; scl3_rows says whether the rows suit scl3 (16-byte aligned, decoded in order).
 int check_scl_shape(const char *who, int n, int L, int64_t B);
-SclPlan scl_plan(int n, int L, int64_t B, SclArith arith, bool scl3_rows);
+SclPlan scl_plan(int n, int L, int64_t B, Arith arith, bool scl3_rows);
+
+// polar_scl.cu: scl2_kernel<L> over P on pl.grid one-warp CTAs, with the min-sum f here and the exact boxplus f in polar_bp
+int launch_scl2(const SclParams &P, const SclPlan &pl, int L, cudaStream_t st);
 
 }  // namespace polar
 
-// polar_scl.cu: scl2_kernel<L> over P on pl.grid one-warp CTAs, with the min-sum f and with the exact boxplus f
+namespace polar_bp {
 int launch_scl2(const polar::SclParams &P, const polar::SclPlan &pl, int L, cudaStream_t st);
-int launch_scl2_boxplus(const polar::SclParams &P, const polar::SclPlan &pl, int L, cudaStream_t st);
+}

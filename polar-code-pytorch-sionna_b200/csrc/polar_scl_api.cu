@@ -1,14 +1,14 @@
 // polar_scl_api.cu -- the C entry points of the list decoder (include/polar_b200.h, polar_scl_*), for every arithmetic.
 // A call is checked (check_scl_args), planned (scl_plan: which mapping runs, its grid and its workspace) and dispatched
-// to scl3_kernel (polar_scl3.cu, min-sum only) or to scl2_kernel<L> of its arithmetic (polar_scl.cu: launch_scl2, and
-// launch_scl2_boxplus from the same source compiled through polar_bp_wrap.cu).
+// to scl3_kernel (polar_scl3.cu, min-sum only) or to scl2_kernel<L> of its arithmetic (polar_scl.cu: launch_scl2, in
+// namespace polar with min-sum and in namespace polar_bp, compiled through polar_bp_wrap.cu, with exact boxplus).
 //
 // The hybrid SC -> SCL decoder lives here too: CRC-aided selection in the `use_hybrid_sc` mode of the Sionna-style
 // SCL_Dec (my_sn/fec/polar/dec.py:437-470).  It decodes the whole batch with SC, keeps every SC decision whose CRC holds,
 // and list-decodes only the rows whose CRC fails.  At a working Eb/N0 almost every SC decision passes, so the batch
 // costs about one SC decode plus a partial wave of the list kernel instead of a full list decode.  Four stream-ordered
 // operations, no host synchronisation:
-//   1. polar_sc_decode_f32 / polar_sc_decode_boxplus_f32 over all B rows -> packed decisions and u_info
+//   1. the SC decoder of the arithmetic (sc_decode, polar_sc_api.cu) over all B rows -> packed decisions and u_info
 //   2. memset of the failing-row count
 //   3. hybrid_crc_check_kernel: syndrome of each packed row, indices of the failing rows appended to fail_rows[]
 //   4. scl2_kernel<L> of the arithmetic over fail_rows[0 .. count-1], overwriting those rows
@@ -18,6 +18,7 @@
 
 #include "polar_common.cuh"
 #include "polar_internal.h"
+#include "polar_sc.h"
 #include "polar_scl.h"
 
 namespace polar {
@@ -25,7 +26,7 @@ namespace polar {
 static int scl_mode() { return env_int("POLAR_SCL_MODE", 2); }   // 2: scl3 where supported, else scl2 [default]; 1: scl2 always (tests)
 
 int check_scl_shape(const char *who, int n, int L, int64_t B) {
-  if (!is_pow2(n) || n < 2 || n > POLAR_SCL_MAX_N) return set_error(POLAR_EINVAL, "%s: n=%d must be a power of two in [2,%d]", who, n, POLAR_SCL_MAX_N);
+  if (const int rc = check_pow2_n(who, n, 2, POLAR_SCL_MAX_N)) return rc;
   if (!is_pow2(L) || L > POLAR_SCL_MAX_L) return set_error(POLAR_EINVAL, "%s: list_size=%d must be a power of two <= %d", who, L, POLAR_SCL_MAX_L);
   if (B < 0) return set_error(POLAR_EINVAL, "%s: B=%lld < 0", who, (long long)B);
   return POLAR_OK;
@@ -34,7 +35,7 @@ int check_scl_shape(const char *who, int n, int L, int64_t B) {
 // ws_bytes is what the mapping needs at its full grid.  For scl3 it is also at least one scl2 warp per SM: a caller
 // sizes the workspace before it knows whether its rows will be 16-byte aligned, and on misaligned rows scl2 runs with
 // as many warps as the workspace holds (its full-grid appetite is ~1.3 GB at n = 1024, L = 8, not worth reserving).
-SclPlan scl_plan(int n, int L, int64_t B, SclArith arith, bool scl3_rows) {
+SclPlan scl_plan(int n, int L, int64_t B, Arith arith, bool scl3_rows) {
   // scl2_kernel<L>, one warp per CTA: 4 KB of shared memory per warp hold the low LLR stages and, up to n = 128, the
   // partial-sum words; the other stages and words live in the workspace.  32 CTAs per SM fill the register file at 64
   // registers per thread.
@@ -55,7 +56,7 @@ SclPlan scl_plan(int n, int L, int64_t B, SclArith arith, bool scl3_rows) {
   pl.ws_bytes = (size_t)pl.grid * pl.ws_bytes_per_warp;
   pl.scl3 = false;
   Scl3Plan p3;
-  if (scl3_rows && arith == SclArith::minsum && scl_mode() == 2 && scl3_supported(n, L) &&
+  if (scl3_rows && arith == Arith::minsum && scl_mode() == 2 && scl3_supported(n, L) &&
       launch_scl3(nullptr, nullptr, n, L, B, nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, 0, nullptr, nullptr, &p3) == POLAR_OK) {
     const size_t floor2 = std::min(pl.ws_bytes, (size_t)device_sm_count() * pl.ws_bytes_per_warp);
     pl.scl3 = true;
@@ -87,7 +88,7 @@ int check_scl_args(const char *who, int n, int L, int64_t B, const float *logit,
 
 // One list decode on device buffers: every polar_scl_decode* call, and the list stage of the hybrid, which passes the
 // rows to decode (rows[0 .. min(*n_rows, B)-1], written earlier on the stream; only scl2 decodes a row list).
-int scl_decode(SclArith arith, const float *logit, const uint32_t *fmask, int n, int L, int64_t B, uint32_t *best,
+int scl_decode(Arith arith, const float *logit, const uint32_t *fmask, int n, int L, int64_t B, uint32_t *best,
                float *u_info, const int32_t *info_pos, int k, double *pm, uint32_t *list, const uint32_t *crc_rows,
                int crc_len, void *ws, size_t ws_bytes, void *stream, const int32_t *rows = nullptr,
                const int32_t *n_rows = nullptr) {
@@ -115,9 +116,9 @@ int scl_decode(SclArith arith, const float *logit, const uint32_t *fmask, int n,
   P.best = best; P.u_info = u_info; P.info_pos = info_pos; P.k = k;
   P.pm_out = pm; P.list = list; P.crc_rows = crc_rows; P.crc_len = crc_len;
   P.ws = (double *)ws; P.ws_doubles_per_warp = pl.ws_bytes_per_warp / sizeof(double); P.s_glob = pl.s_glob;
-  P.smem_per_warp = pl.smem_per_warp; P.words_global = pl.words_global; P.fast = arith == SclArith::boxplus_pruned;
+  P.smem_per_warp = pl.smem_per_warp; P.words_global = pl.words_global; P.fast = arith == Arith::boxplus_pruned;
   P.rows = rows; P.n_rows = n_rows;
-  return arith == SclArith::minsum ? launch_scl2(P, pl, L, st) : launch_scl2_boxplus(P, pl, L, st);
+  return arith == Arith::minsum ? launch_scl2(P, pl, L, st) : polar_bp::launch_scl2(P, pl, L, st);
 }
 
 constexpr unsigned kFull = 0xFFFFFFFFu;
@@ -131,7 +132,7 @@ inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 //   [scl_off]    scl2_kernel<L> workspace planned for B rows
 struct HybridLayout { size_t count_off, rows_off, scl_off, total; };
 
-HybridLayout hybrid_layout(int n, int L, int64_t B, SclArith arith) {
+HybridLayout hybrid_layout(int n, int L, int64_t B, Arith arith) {
   HybridLayout h;
   h.count_off = align256((size_t)B * POLAR_WORDS(n) * sizeof(uint32_t));
   h.rows_off = h.count_off + 256;
@@ -186,19 +187,19 @@ using namespace polar;
 
 extern "C" size_t polar_scl_workspace_bytes(int n, int L, int64_t B) {
   if (B <= 0 || check_scl_shape("scl", n, L, B) != POLAR_OK) return 0;
-  return scl_plan(n, L, B, SclArith::minsum, true).ws_bytes;
+  return scl_plan(n, L, B, Arith::minsum, true).ws_bytes;
 }
 
 extern "C" size_t polar_scl_boxplus_workspace_bytes(int n, int L, int64_t B) {
   if (B <= 0 || check_scl_shape("scl", n, L, B) != POLAR_OK) return 0;
-  return scl_plan(n, L, B, SclArith::boxplus, true).ws_bytes;
+  return scl_plan(n, L, B, Arith::boxplus, true).ws_bytes;
 }
 
 extern "C" int polar_scl_decode(const float *d_logit, const uint32_t *d_frozen_mask, int n, int L, int64_t B,
                                 uint32_t *d_best_packed, float *d_u_info_f32, const int32_t *d_info_pos, int k,
                                 double *d_pm_sorted, uint32_t *d_list_packed, const uint32_t *d_crc_rows, int crc_len,
                                 void *d_workspace, size_t workspace_bytes, void *stream) {
-  return scl_decode(SclArith::minsum, d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, d_pm_sorted,
+  return scl_decode(Arith::minsum, d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, d_pm_sorted,
                     d_list_packed, d_crc_rows, crc_len, d_workspace, workspace_bytes, stream);
 }
 
@@ -206,7 +207,7 @@ extern "C" int polar_scl_decode_boxplus(const float *d_logit, const uint32_t *d_
                                         uint32_t *d_best_packed, float *d_u_info_f32, const int32_t *d_info_pos, int k,
                                         double *d_pm_sorted, uint32_t *d_list_packed, const uint32_t *d_crc_rows, int crc_len,
                                         void *d_workspace, size_t workspace_bytes, void *stream) {
-  return scl_decode(SclArith::boxplus, d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, d_pm_sorted,
+  return scl_decode(Arith::boxplus, d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, d_pm_sorted,
                     d_list_packed, d_crc_rows, crc_len, d_workspace, workspace_bytes, stream);
 }
 
@@ -215,13 +216,13 @@ extern "C" int polar_scl_decode_boxplus_pruned(const float *d_logit, const uint3
                                                uint32_t *d_best_packed, float *d_u_info_f32, const int32_t *d_info_pos, int k,
                                                double *d_pm_sorted, uint32_t *d_list_packed, const uint32_t *d_crc_rows, int crc_len,
                                                void *d_workspace, size_t workspace_bytes, void *stream) {
-  return scl_decode(SclArith::boxplus_pruned, d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k,
+  return scl_decode(Arith::boxplus_pruned, d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k,
                     d_pm_sorted, d_list_packed, d_crc_rows, crc_len, d_workspace, workspace_bytes, stream);
 }
 
 extern "C" size_t polar_scl_hybrid_workspace_bytes(int n, int L, int64_t B, int cn_mode) {
   if (B <= 0 || B > INT32_MAX || cn_mode < 0 || cn_mode > 2 || check_scl_shape("hybrid", n, L, B) != POLAR_OK) return 0;
-  return hybrid_layout(n, L, B, (SclArith)cn_mode).total;
+  return hybrid_layout(n, L, B, (Arith)cn_mode).total;
 }
 
 extern "C" int polar_scl_decode_hybrid(const float *d_logit, const uint32_t *d_frozen_mask, int n, int L, int64_t B,
@@ -233,7 +234,7 @@ extern "C" int polar_scl_decode_hybrid(const float *d_logit, const uint32_t *d_f
   int rc = check_scl_args("hybrid", n, L, B, d_logit, d_frozen_mask, d_best_packed || d_u_info_f32, d_u_info_f32, d_info_pos, k,
                           d_crc_rows, crc_len, true);
   if (rc != POLAR_OK || B == 0) return rc;
-  const SclArith arith = (SclArith)cn_mode;
+  const Arith arith = (Arith)cn_mode;
   const HybridLayout h = hybrid_layout(n, L, B, arith);
   if (!d_workspace || workspace_bytes < h.total) return set_error(POLAR_ENOMEM, "hybrid: workspace %zu B < required %zu B", d_workspace ? workspace_bytes : (size_t)0, h.total);
   if ((uintptr_t)d_workspace & 255) return set_error(POLAR_EALIGN, "hybrid: workspace must be 256-byte aligned");
@@ -244,20 +245,13 @@ extern "C" int polar_scl_decode_hybrid(const float *d_logit, const uint32_t *d_f
   int32_t *fail_rows = (int32_t *)(ws + h.rows_off);
   cudaStream_t st = (cudaStream_t)stream;
 
-  rc = (arith == SclArith::minsum ? polar_sc_decode_f32 : polar_sc_decode_boxplus_f32)(d_logit, d_frozen_mask, n, B, sc_packed,
-                                                                                        d_u_info_f32, d_info_pos, k, stream);
+  rc = sc_decode(arith, d_logit, d_frozen_mask, n, B, sc_packed, d_u_info_f32, d_info_pos, k, stream);
   if (rc != POLAR_OK) return rc;
   POLAR_CUDA(cudaMemsetAsync(count, 0, sizeof(int32_t), st));
-  {
-    const int rpw = 32 / (POLAR_WORDS(n) < 32 ? POLAR_WORDS(n) : 32);
-    const int64_t warps = (B + rpw - 1) / rpw;
-    int64_t grid = (warps + 7) / 8;
-    const int64_t cap = (int64_t)device_sm_count() * 8;
-    if (grid > cap) grid = cap;
-    hybrid_crc_check_kernel<<<(unsigned)grid, 256, 0, st>>>(sc_packed, n, B, d_crc_rows, count, fail_rows);
-    count_launch();
-    POLAR_CHECK_LAUNCH("hybrid_crc_check_kernel");
-  }
+  const int rpw = 32 / (POLAR_WORDS(n) < 32 ? POLAR_WORDS(n) : 32);   // rows per warp step of the check kernel
+  rc = launch("hybrid_crc_check_kernel", hybrid_crc_check_kernel, grid_for((B + rpw - 1) / rpw, 8, 8), 256, 0, st, sc_packed, n,
+              B, d_crc_rows, count, fail_rows);
+  if (rc != POLAR_OK) return rc;
   return scl_decode(arith, d_logit, d_frozen_mask, n, L, B, d_best_packed, d_u_info_f32, d_info_pos, k, nullptr, nullptr,
                     d_crc_rows, crc_len, ws + h.scl_off, workspace_bytes - h.scl_off, stream, fail_rows, count);
 }
