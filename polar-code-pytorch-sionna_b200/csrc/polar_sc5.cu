@@ -190,28 +190,27 @@ PDEV void tmem_st4(uint32_t taddr, const float4 a) {
                ::"r"(taddr), "r"(f2u(a.x)), "r"(f2u(a.y)), "r"(f2u(a.z)), "r"(f2u(a.w)) : "memory");
 }
 PDEV void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-struct Tm8 { uint32_t r[8]; };
-PDEV void tmem_ld8_issue(uint32_t taddr, Tm8 &v) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(v.r[0]), "=r"(v.r[1]), "=r"(v.r[2]), "=r"(v.r[3]), "=r"(v.r[4]), "=r"(v.r[5]), "=r"(v.r[6]), "=r"(v.r[7])
+struct Tm16 { uint32_t r[16]; };    // 16 columns = the stage-8 pairs of two consecutive codewords
+PDEV void tmem_ld16_issue(uint32_t taddr, Tm16 &v) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+               : "=r"(v.r[0]), "=r"(v.r[1]), "=r"(v.r[2]), "=r"(v.r[3]), "=r"(v.r[4]), "=r"(v.r[5]), "=r"(v.r[6]), "=r"(v.r[7]),
+                 "=r"(v.r[8]), "=r"(v.r[9]), "=r"(v.r[10]), "=r"(v.r[11]), "=r"(v.r[12]), "=r"(v.r[13]), "=r"(v.r[14]), "=r"(v.r[15])
                : "r"(taddr) : "memory");
 }
-PDEV void tmem_ld_wait(Tm8 &a, Tm8 &b) {   // the registers are defined only after the wait; tying them to it keeps every use behind it
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(a.r[0]), "+r"(a.r[1]), "+r"(a.r[2]), "+r"(a.r[3]), "+r"(a.r[4]), "+r"(a.r[5]), "+r"(a.r[6]), "+r"(a.r[7]),
-                 "+r"(b.r[0]), "+r"(b.r[1]), "+r"(b.r[2]), "+r"(b.r[3]), "+r"(b.r[4]), "+r"(b.r[5]), "+r"(b.r[6]), "+r"(b.r[7])
-               :: "memory");
+PDEV void tmem_ld_wait_all() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+PDEV void tmem_tie(Tm16 &v) {      // after tmem_ld_wait_all(): keeps every use of v behind the wait (volatile asm keeps its order)
+  asm volatile(""
+               : "+r"(v.r[0]), "+r"(v.r[1]), "+r"(v.r[2]), "+r"(v.r[3]), "+r"(v.r[4]), "+r"(v.r[5]), "+r"(v.r[6]), "+r"(v.r[7]),
+                 "+r"(v.r[8]), "+r"(v.r[9]), "+r"(v.r[10]), "+r"(v.r[11]), "+r"(v.r[12]), "+r"(v.r[13]), "+r"(v.r[14]), "+r"(v.r[15]));
 }
-PDEV float4 tm_lo(const Tm8 &v) { return make_float4(u2f(v.r[0]), u2f(v.r[1]), u2f(v.r[2]), u2f(v.r[3])); }
-PDEV float4 tm_hi(const Tm8 &v) { return make_float4(u2f(v.r[4]), u2f(v.r[5]), u2f(v.r[6]), u2f(v.r[7])); }
 
 // ---- staging ------------------------------------------------------------------------------------------------------
 // While a warp runs a descent its own stage-7 buffer is dead (it is rewritten by the tensor-memory step that follows), so
 // it serves as kSlots = 4 staging slots of 4 KB: 16 KB of bulk copies in flight per descending warp, no sharing, no
 // atomics.  (A pool of extra slots in the CTA's spare shared memory, shared by the warps, was measured and removed: with
 // 2 or 4 more slots per warp the passes were SLOWER -- the memory system, not the number of requests in flight, bounds
-// them.)  Each slot has its own mbarrier; `par` holds the parity its next completion will have, kept by the warp in a
-// register across descents.
+// them.)  Each slot has its own mbarrier; `par` holds the parity its next completion will have, kept by the warp across
+// descents.
 //
 // Fused descent (file header).  D = stages between the source (stage 8 + D: channel row or scratch node) and the stage-8
 // node that ends in tensor memory; FIRST_G: the first update is g with the partial sums of the left sibling (entering a
@@ -246,6 +245,11 @@ __device__ __noinline__ void descent(const float *__restrict__ src, const int nv
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");            // the stage-7 buffer (generic writes) becomes staging space
   __syncwarp();
   const uint32_t slot_a = smem_u32(Lw);
+  // `par` is a reference into the caller's stack frame (this function is not inlined): read through it, every slot wait
+  // of a step reloads it from local memory, with L1 almost all carved out as shared memory.  The whole-node loops keep a
+  // register copy; the D >= 3 loop (n >= 2048) keeps the reference: its copy spills in the boxplus build at n = 8192.
+  uint32_t par_reg = par;
+  uint32_t &pr = WIDE ? par_reg : par;
 
   // refill slots ring, ring+1 (ring in {0, 2, ..}) with sub-units k, k+1 (all lanes call it)
   auto issue2 = [&](const int k, const int ring) {
@@ -283,7 +287,7 @@ __device__ __noinline__ void descent(const float *__restrict__ src, const int nv
         "@P1 bra SC5_DONE;\n\t"
         "bra SC5_WAIT;\n\t"
         "SC5_DONE:\n\t"
-        "}" ::"r"(bar_a + 8 * s), "r"((par >> s) & 1u), "r"(0x989680u) : "memory");
+        "}" ::"r"(bar_a + 8 * s), "r"((pr >> s) & 1u), "r"(0x989680u) : "memory");
     return Lw + s * kSlotFloats;
   };
 
@@ -335,7 +339,7 @@ __device__ __noinline__ void descent(const float *__restrict__ src, const int nv
       }
       st1 += CW << T1; bp += CW * nws; dp += 2048;
       __syncwarp();                                    // every lane has consumed both slots
-      par ^= 3u << ring;
+      pr ^= 3u << ring;
       if (k + NS < K) issue2(k + NS, ring);
 #pragma unroll
       for (int u = 0; u < CW; ++u) tmem_st8(tm_base + tcol + 8 * u, out[u][0], out[u][1]);
@@ -377,7 +381,7 @@ __device__ __noinline__ void descent(const float *__restrict__ src, const int nv
           asm volatile("discard.global.L2 [%0], 128;" ::"l"(dp + 4 * q * 256 + 128) : "memory");
         }
         __syncwarp();
-        par ^= 3u << ring;
+        pr ^= 3u << ring;
         if (k + NS < K) issue2(k + NS, ring);
         ring = (ring + 2 == NS) ? 0 : ring + 2;
       }
@@ -399,6 +403,7 @@ __device__ __noinline__ void descent(const float *__restrict__ src, const int nv
       st1 += 1 << T1; bp += nws; dp += SRC;
     }
   }
+  if (WIDE) par = par_reg;
   tmem_wait_st();
   __syncwarp();
 }
@@ -407,40 +412,49 @@ __device__ __noinline__ void descent(const float *__restrict__ src, const int nv
 template <bool IS_G>
 PDEV void step_tmem(float *L, const uint32_t *beta, const int stride, const int nws, const int lane, const uint32_t tm_base,
                     const int left_word) {
-  // 128 outputs per codeword = 32 float4; round k = codeword k, lane = float4 column.  tcgen05.wait::ld waits for every
-  // load issued before it, so the loads of group g+1 are issued right AFTER the wait for group g and fly while group g
-  // is computed (two register sets of 4 x 8).
+  // 128 outputs per codeword = 32 float4; codeword k, lane = float4 column.  Two register sets of G = 4 codewords (two
+  // 32x32b.x16 loads each): tcgen05.wait::ld waits for every load issued before it, so the loads of the next set are
+  // issued right AFTER the wait for this one and fly while its codewords are computed.  The g pass reads the partial-sum
+  // bits of a set together with its loads -- read per codeword, each read queued behind the previous codeword's store and
+  // the whole g chain waited on it.  (Sets of 8: the pass is as short, the kernel 1.4 % slower -- 200 more instructions.)
+  constexpr int G = 4;
   const int j = lane << 2;
   const uint32_t *bp = beta + left_word + (j >> 5);
   const int sh = j & 31;
   float *dst = L + j;
-  Tm8 a0, a1, a2, a3, b0, b1, b2, b3;
-  auto issue4 = [&](const int k0, Tm8 &v0, Tm8 &v1, Tm8 &v2, Tm8 &v3) {
-    tmem_ld8_issue(tm_base + 8 * k0, v0);
-    tmem_ld8_issue(tm_base + 8 * (k0 + 1), v1);
-    tmem_ld8_issue(tm_base + 8 * (k0 + 2), v2);
-    tmem_ld8_issue(tm_base + 8 * (k0 + 3), v3);
-  };
-  auto compute4 = [&](const int k0, const Tm8 &v0, const Tm8 &v1, const Tm8 &v2, const Tm8 &v3) {
+  Tm16 a[G / 2], b[G / 2];
+  uint32_t ba[G], bb[G];
+  auto issue = [&](const int k0, Tm16 (&v)[G / 2], uint32_t (&bits)[G]) {
 #pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      const Tm8 &v = r == 0 ? v0 : r == 1 ? v1 : r == 2 ? v2 : v3;
-      const float4 a = tm_lo(v), b = tm_hi(v);
-      float4 o;
-      if (IS_G) o = g4(a, b, bp[(k0 + r) * nws] >> sh);
-      else o = f4(a, b);
-      sts4(dst + (k0 + r) * stride, o);
+    for (int q = 0; q < G / 2; ++q) tmem_ld16_issue(tm_base + 8 * (k0 + 2 * q), v[q]);
+    if (IS_G) {
+#pragma unroll
+      for (int r = 0; r < G; ++r) bits[r] = bp[(k0 + r) * nws] >> sh;
     }
   };
-  issue4(0, a0, a1, a2, a3);
+  auto wait = [&](Tm16 (&v)[G / 2]) {
+    tmem_ld_wait_all();
+#pragma unroll
+    for (int q = 0; q < G / 2; ++q) tmem_tie(v[q]);
+  };
+  auto compute = [&](const int k0, const Tm16 (&v)[G / 2], const uint32_t (&bits)[G]) {
+#pragma unroll
+    for (int r = 0; r < G; ++r) {
+      const uint32_t *w = v[r >> 1].r + 8 * (r & 1);
+      const float4 x = make_float4(u2f(w[0]), u2f(w[1]), u2f(w[2]), u2f(w[3]));
+      const float4 y = make_float4(u2f(w[4]), u2f(w[5]), u2f(w[6]), u2f(w[7]));
+      sts4(dst + (k0 + r) * stride, IS_G ? g4(x, y, bits[r]) : f4(x, y));
+    }
+  };
+  issue(0, a, ba);
 #pragma unroll 1
-  for (int k0 = 0; k0 < 32; k0 += 8) {
-    tmem_ld_wait(a0, a1); tmem_ld_wait(a2, a3);
-    issue4(k0 + 4, b0, b1, b2, b3);
-    compute4(k0, a0, a1, a2, a3);
-    tmem_ld_wait(b0, b1); tmem_ld_wait(b2, b3);
-    if (k0 + 8 < 32) issue4(k0 + 8, a0, a1, a2, a3);
-    compute4(k0 + 4, b0, b1, b2, b3);
+  for (int k0 = 0; k0 < 32; k0 += 2 * G) {
+    wait(a);
+    issue(k0 + G, b, bb);
+    compute(k0, a, ba);
+    wait(b);
+    if (k0 + 2 * G < 32) issue(k0 + 2 * G, a, ba);
+    compute(k0 + G, b, bb);
   }
 }
 
